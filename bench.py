@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the COMET tracking hot path on B200 (contract: see the task statement / DESIGN.md section 6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch Q] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch Q] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], "batched inference, seqlen=16, synthetic sequences on 1xB200"): one *step*
 is one pass of the hot path over a batch of Q synthetic 16-frame sequences per GPU.  Per sequence that is
@@ -40,6 +40,7 @@ COARSE = dict(S=16, N=512, C=128, H=64, W=64, L=5, r=4, iters=4, fine=False)
 FINE = dict(S=16, P=512, C=32, H=31, W=31, L=3, r=3, iters=6, fine=True)
 METRIC = "sequences/sec (seqlen=16)"
 UNIT = "sequences/s"
+DUMP_BYTES = 63 * 10 ** 6      # data of all --dump-outputs arrays together: under 64 MB with the .npy headers
 
 
 def peaks():
@@ -155,6 +156,24 @@ class HotPath:
                 tk.tokens(x["coords"][i], x["feats"][i], out=out)
                 self._mark(name + "_tokens")
         return self.tok_c, self.tok_f
+
+
+def sample_outputs(outputs, budget=DUMP_BYTES):
+    """Host float32 copies of `outputs` (name -> tensor), DUMP_BYTES in all.  A tensor larger than its share of the
+    budget is cut to a fixed, seeded sample of rows (leading axes flattened, last axis whole, rows in order), so two
+    runs with the same arguments keep the same elements."""
+    import numpy as np
+    import torch
+
+    share = budget // len(outputs)
+    out = {}
+    for name, t in outputs.items():
+        if t.numel() * 4 > share:
+            rows = t.reshape(-1, t.shape[-1])
+            keep = np.sort(np.random.default_rng(0).choice(rows.shape[0], share // (rows.shape[1] * 4), replace=False))
+            t = rows[torch.as_tensor(keep, device=rows.device)]
+        out[name] = t.float().cpu().numpy()
+    return out
 
 
 def fine_lines_per_query(coords, layout):
@@ -425,7 +444,13 @@ def main():
                          "refine_track: the 31x31 up-sampling is evaluated inside the lookup); cl = materialised 31x31 "
                          "features as a channels-last view; nchw = contiguous (B,S,C,H,W) as the reference's own "
                          "refine_track would hand over")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the tokens the last timed step computed (rank 0) as "
+                         "DIR/coarse_tokens.npy and DIR/fine_tokens.npy, float32; beyond 64 MB in all, a fixed seeded "
+                         "sample of token rows is written")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -511,6 +536,13 @@ def main():
     launches = cb._lib.lib.comet_launch_count() - launches0  # counted by the library itself, one per kernel launch
     clocks = sampler.stop() if sampler else None
     value = Q * world / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # the variants below reuse hp's output buffers: save the timed step's tokens now
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in sample_outputs({"coarse_tokens": hp.tok_c, "fine_tokens": hp.tok_f}).items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     kern = {k: {"launch_groups": len(v), "ms_avg": sum(v) / len(v), "ms_per_step": sum(v) / args.steps}
             for k, v in per.items()}

@@ -13,6 +13,7 @@ What is stored (weights are NOT stored: ``cases.seeded_state_dict`` rebuilds the
   float64 (``pred64_i``), visibility, a slice of the track features.  The float64 run is the yard-stick that turns
   the "any two fp32 implementations drift" statement of DESIGN.md section 3 into a measured bar:
   a conforming fp32 implementation must satisfy |impl - ref64| <= 3 |ref32 - ref64| per iteration.
+  The query features and the track-feature slice are stored in ``tracker_full_feats.npz``.
 * ``refine_full.npz``   ``refine_track`` (31x31 patches of 512x512 images -> ShallowEncoder -> fine tracker hidden 256 /
   depth 4 / 6 iterations (abl_ours.yaml:419-428) -> compute_score_fn) fed with the reference's own float32 coarse prediction: refined tracks
   and score in float32 and float64, and the inverted score of E2Epose2.py:232-236.
@@ -114,10 +115,10 @@ def run_coarse(torch, btp):
         d = (a.double() - b).abs().max() / b.abs().max()
         print(f"  iteration {i}: |ref32 - ref64| / max|ref64| = {float(d):.3e}")
     out["vis32"], out["vis64"] = vis32.numpy(), vis64.numpy()
-    out["query_feat32"] = qf32.numpy()
-    out["track_feats32_slice"] = tf32[:, :, ::37].numpy()
-    out["track_feats64_slice"] = tf64[:, :, ::37].numpy()
     mg.save("tracker_full", **out)
+    # the features go to a file of their own: together with the tracks they exceed 1 MB
+    mg.save("tracker_full_feats", digest=out["digest"], query_feat32=qf32.numpy(),
+            track_feats32_slice=tf32[:, :, ::37].numpy(), track_feats64_slice=tf64[:, :, ::37].numpy())
     return p32[-1].numpy(), p64[-1].numpy()
 
 

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -65,6 +66,19 @@ def test_synthetic_inputs_layouts():
     finally:
         bench.FINE.clear(); bench.FINE.update(saved[0])
         bench.COARSE.clear(); bench.COARSE.update(saved[1])
+
+
+def test_dumped_outputs_are_a_fixed_sample_within_64_mb():
+    rows = 4 * 512 * 16
+    coarse = torch.arange(rows, dtype=torch.float32)[:, None].repeat(1, 664).reshape(4, 512, 16, 664)   # row i holds i
+    fine = torch.randn(4 * 512, 1, 16, 216)
+    a = bench.sample_outputs({"coarse_tokens": coarse, "fine_tokens": fine})
+    b = bench.sample_outputs({"coarse_tokens": coarse, "fine_tokens": fine})
+    assert sum(v.nbytes for v in a.values()) <= 64 * 10 ** 6
+    assert a["fine_tokens"].dtype == np.float32 and np.array_equal(a["fine_tokens"], fine.numpy())   # fits: whole
+    got = a["coarse_tokens"]
+    assert got.shape[1] == 664 and 0 < got.shape[0] < rows and np.array_equal(got, b["coarse_tokens"])
+    assert (got == got[:, :1]).all() and (np.diff(got[:, 0]) > 0).all()     # whole rows, distinct, in order
 
 
 def test_reference_arm_json_line():

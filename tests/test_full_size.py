@@ -139,7 +139,7 @@ def no_tf32():
 @pytest.mark.gpu
 def test_full_coarse_tracker_against_fp64_reference(golden, no_tf32):
     """hidden 384, depth 6, S=16, N=512, 4 iterations (abl_ours.yaml:99, 399-412) through the drop-in predictor."""
-    g = golden("tracker_full")
+    g, gf = golden("tracker_full"), golden("tracker_full_feats")
     preds, vis, feats, qfeat, _ = _run_coarse(_coarse_model())
     rows = []
     for i in range(cases.FULL_COARSE_ITERS):
@@ -150,10 +150,10 @@ def test_full_coarse_tracker_against_fp64_reference(golden, no_tf32):
     _record("coarse_tracker_full", rows)
     for r in rows:
         assert r["impl_vs_ref64"] <= r["bar"], rows
-    assert rel_to_max(qfeat.cpu().numpy(), g["query_feat32"]) < 1e-5
+    assert rel_to_max(qfeat.cpu().numpy(), gf["query_feat32"]) < 1e-5
     assert rel_to_max(vis.cpu().numpy(), g["vis64"]) <= bar(g["vis32"], g["vis64"])
-    assert rel_to_max(feats[:, :, ::37].cpu().numpy(), g["track_feats64_slice"]) <= \
-        bar(g["track_feats32_slice"], g["track_feats64_slice"])
+    assert rel_to_max(feats[:, :, ::37].cpu().numpy(), gf["track_feats64_slice"]) <= \
+        bar(gf["track_feats32_slice"], gf["track_feats64_slice"])
 
 
 @pytest.mark.gpu

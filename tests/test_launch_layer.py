@@ -53,8 +53,11 @@ def _worker(rank, world, port, n_items, out_dir):
     dist.destroy_process_group()
 
 
-def test_two_rank_gloo_shard_and_gather(tmp_path):
+def test_two_rank_gloo_shard_and_gather(tmp_path, monkeypatch):
     world, n_items = 2, 7
+    # a CPU run whatever the machine has: with GPUs visible, init_distributed binds rank r to cuda:r, which a machine
+    # with fewer GPUs than ranks does not have
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     mp.spawn(_worker, args=(world, _free_port(), n_items, str(tmp_path)), nprocs=world, join=True)
     assert (tmp_path / "ok").exists()
 
