@@ -34,6 +34,6 @@ from .track_tokens import TrackTokenizer, sampled_pos_emb, transformer_dim  # no
 from .update_former import EfficientUpdateFormer  # noqa: F401
 from .base_track_predictor import BaseTrackerPredictor  # noqa: F401
 from .refine_track import ShallowEncoder, compute_score_fn, extract_patches, inverted_score, refine_track  # noqa: F401
-from .track_predictor import BasicEncoder, TrackerPredictor  # noqa: F401
+from .track_predictor import BasicEncoder, TrackerPredictor, split_batch  # noqa: F401
 
 __version__ = "0.1.0"

@@ -47,7 +47,19 @@ class BaseTrackerPredictor(nn.Module):
             self.vis_predictor = nn.Sequential(nn.Linear(latent_dim, 1))
 
     def forward(self, query_points, fmaps=None, iters=4, return_feat=False, down_ratio=1, is_train=False,
-                track_feats=None, TRACKorPOSE=True, ind=0):
+                track_feats=None, TRACKorPOSE=True, ind=0, num_tracks=None):
+        """``num_tracks`` (B ints or a 1-D tensor, ``TRACKorPOSE=False`` only): ``query_points`` (B, N_max, 2) is a padded
+        batch of sequences with different track counts.  Sequence b's tracks get what a call on that sequence alone
+        computes (up to rounding); every output entry of a padded track (n >= num_tracks[b]) is 0."""
+        counts = None
+        if num_tracks is not None:
+            assert not TRACKorPOSE, "num_tracks is served with TRACKorPOSE=False only"
+            from .utils import check_num_tracks
+
+            counts = check_num_tracks(num_tracks, query_points.shape[0], query_points.shape[1])
+            real = torch.arange(query_points.shape[1], device=query_points.device)[None, :] < torch.tensor(
+                counts, device=query_points.device)[:, None]                                  # (B, N)
+            query_points = query_points * real[:, :, None]          # padded queries start at 0 and never move
         if TRACKorPOSE:
             B, S, N, D = query_points.shape
         else:
@@ -75,14 +87,17 @@ class BaseTrackerPredictor(nn.Module):
         else:
             fcorr_fn = CorrBlock(fmaps, num_levels=self.corr_levels, radius=self.corr_radius)
         # sampled_pos_emb depends on coords[:, 0] only, which the loop pins -> computed once, not per iteration
-        tokenizer = TrackTokenizer(fcorr_fn, coords[:, 0], self.transformer_dim)
+        tokenizer = TrackTokenizer(fcorr_fn, coords[:, 0], self.transformer_dim, num_tracks=counts)
 
         coord_preds = []
         for _ in range(iters):
             coords = coords.detach()
             x = tokenizer.tokens(coords, track_feats)  # (B, N, S, transformer_dim), one fused kernel
 
-            delta = self.updateformer(x).reshape(B * N, S, self.latent_dim + 2)
+            if counts is None:
+                delta = self.updateformer(x).reshape(B * N, S, self.latent_dim + 2)
+            else:
+                delta = self.updateformer(x, num_tracks=counts).reshape(B * N, S, self.latent_dim + 2)   # 0 when padded
             delta_coords_ = delta[:, :, :2]
             delta_feats_ = delta[:, :, 2:].reshape(B * N * S, self.latent_dim)
 
@@ -104,6 +119,13 @@ class BaseTrackerPredictor(nn.Module):
         conf_e = None
         if self.cfg.track_conf:
             conf_e = torch.sigmoid(self.conf_predictor(track_feats.reshape(B * S * N, self.latent_dim)).reshape(B, S, N))
+        if counts is not None:
+            pad_s = ~real[:, None, :]                                                         # (B, 1, N)
+            coord_preds = [c.masked_fill(pad_s[..., None], 0.0) for c in coord_preds]
+            vis_e = None if vis_e is None else vis_e.masked_fill(pad_s, 0.0)
+            conf_e = None if conf_e is None else conf_e.masked_fill(pad_s, 0.0)
+            track_feats = track_feats.masked_fill(pad_s[..., None], 0.0)
+            query_track_feat = query_track_feat.masked_fill(~real[..., None], 0.0)
         if return_feat:
             return coord_preds, vis_e, track_feats, query_track_feat, conf_e
         return coord_preds, vis_e, conf_e

@@ -19,6 +19,7 @@ struct LookupParams {
   float* out;
   long long o_sb, o_ss, o_sn;
   const float* pos;  // TOKENS: (B,N,D_tok)
+  const int* ntr;    // TOKENS: (B,) query count of each sequence (rows n >= ntr[b] are written as zeros), or null
   int D_tok;
   int B, S, N, C, L, r;
   int pad_border, bf16;

@@ -284,11 +284,13 @@ __device__ __forceinline__ void zero_border(float* b0, int tid) {
 struct Params {
   const float* src;        // images (B,S,3,H,W) or a patch tensor
   const int* topleft;      // (B,S,N,2) (x, y) corners, or null: `src` holds the patches themselves
+  const int* seq_of_track; // packed tracks, or null: topleft is (N,S,2) and track n reads the frames of sequence seq_of_track[n]
   const float* packed;
   float* out;              // (P, 16, 16, 32) channel-last
   long long P;             // number of patches
   long long sn, sc, sy, sx;  // element strides of the patch tensor (topleft == null) / of the image (sc, sy, sx)
   int S, N, H, W;
+  int nseq;                // packed tracks: number of sequences in `src`
   float eps;
 };
 
@@ -303,8 +305,12 @@ __device__ __forceinline__ void prefetch_pixels(const Params& p, long long pair,
       const int s = (int)(pi % p.S);
       const long long bn = pi / p.S;
       const int n = (int)(bn % p.N);
-      const long long b = bn / p.N;
+      long long b = bn / p.N;
       const int* tl = p.topleft + ((b * p.S + s) * p.N + n) * 2;
+      if (p.seq_of_track) {
+        b = min(max(__ldg(p.seq_of_track + n), 0), p.nseq - 1);
+        tl = p.topleft + ((long long)n * p.S + s) * 2;
+      }
       const int x0 = min(max(__ldg(tl), 0), p.W - PSZ), y0 = min(max(__ldg(tl + 1), 0), p.H - PSZ);
       base[g] = p.src + (b * p.S + s) * 3 * p.sc + (long long)y0 * p.sy + (long long)x0 * p.sx;
     } else {
@@ -598,5 +604,20 @@ extern "C" int comet_shallow_encoder_from_images_f32(const float* images, const 
   p.src = images; p.topleft = topleft; p.packed = packed; p.out = out; p.P = P;
   p.sn = 0; p.sc = (long long)H * W; p.sy = W; p.sx = 1;
   p.S = S; p.N = N; p.H = H; p.W = W; p.eps = eps;
+  return launch_shallow_encoder(p, stream);
+}
+
+extern "C" int comet_shallow_encoder_from_images_ragged_f32(const float* images, const int* topleft, const int* seq_of_track,
+                                                            const float* packed, float* out, int P, int B, int S, int H, int W,
+                                                            float eps, comet_stream_t stream) {
+  COMET_REQUIRE(P >= 0 && B >= 1 && S >= 0 && H >= senc::PSZ && W >= senc::PSZ, "bad shape");
+  if ((long long)P * S == 0) return COMET_OK;
+  COMET_REQUIRE(images && topleft && seq_of_track && packed && out, "null pointer");
+  COMET_REQUIRE(((uintptr_t)packed % 16) == 0, "packed parameters must be 16-byte aligned");
+  senc::Params p{};
+  p.src = images; p.topleft = topleft; p.seq_of_track = seq_of_track; p.packed = packed; p.out = out;
+  p.P = (long long)P * S;
+  p.sn = 0; p.sc = (long long)H * W; p.sy = W; p.sx = 1;
+  p.S = S; p.N = P; p.H = H; p.W = W; p.nseq = B; p.eps = eps;
   return launch_shallow_encoder(p, stream);
 }

@@ -167,14 +167,51 @@ struct AttnParams {
   int B, H, Lq, Lk, dh;
   float scale;
   int vec_out;   // output planes can be written four values (8 bytes) at a time
+  // Variable lengths (comet_attention_varlen_planes_f32), null otherwise: item b's queries / outputs start at row q_off[b]
+  // and its keys / values at row k_off[b] (the *_sb strides are then row pitches), with q_len[b] / k_len[b] positions.
+  // Lq / Lk hold the largest lengths.  A launch serves only the items whose attn_path() is `path`.
+  const int* q_off; const int* q_len; const int* k_off; const int* k_len;
+  int path, group, mma_opt, mma_align;
 };
+
+// Kernel family of an attention problem: one definition for the host dispatch of comet_attention_planes_f32 and for the
+// per-item choice of the varlen launches, so that an item of a varlen call gets exactly the arithmetic a single call of
+// the same shape gets.  `B` is the number of problems of that single call (it sizes the grid of the key-split kernel).
+enum { AP_SMALL_MMA, AP_SMALL, AP_ROWS_MMA, AP_ROWS, AP_KSPLIT, AP_TILED, AP_COUNT };
+constexpr int ATR_KMAX = 64;
+__host__ __device__ __forceinline__ int attn_path(int np, int Lq, int Lk, int dh, long long B, int H, int mma_opt,
+                                                  int mma_align) {
+  if (np == 1 && Lq <= 16 && Lk <= 32 && (dh == 32 || dh == 48) && (mma_opt & 2) && mma_align) return AP_SMALL_MMA;
+  if (Lq <= 32 && Lk <= 32) return AP_SMALL;
+  if (np == 1 && Lq >= 64 && (dh == 32 || dh == 48 || dh == 64) && (mma_opt & 1) && mma_align) return AP_ROWS_MMA;
+  if (Lk <= ATR_KMAX && Lq >= 64) return AP_ROWS;
+  if (Lk > ATR_KMAX && B * H * ((Lq + 63) / 64) <= 148LL * 4) return AP_KSPLIT;
+  return AP_TILED;
+}
+
+// Rows and lengths of problem b.  Varlen: false when this launch does not serve the item, or the query chunk starting at
+// q0 is past its queries (block-uniform: b and q0 are).
+struct AttnItem { long long qb, kb, vb, ob; int Lq, Lk; };
+template <bool VARLEN>
+__device__ __forceinline__ bool attn_item(const AttnParams& p, int b, int q0, AttnItem& it) {
+  if (!VARLEN) {
+    it.qb = b * p.q_sb; it.kb = b * p.k_sb; it.vb = b * p.v_sb; it.ob = b * p.o_sb; it.Lq = p.Lq; it.Lk = p.Lk;
+    return true;
+  }
+  it.Lq = __ldg(p.q_len + b); it.Lk = __ldg(p.k_len + b);
+  if (q0 >= it.Lq || it.Lk < 1 || attn_path(p.np, it.Lq, it.Lk, p.dh, p.group, p.H, p.mma_opt, p.mma_align) != p.path)
+    return false;
+  const long long qo = __ldg(p.q_off + b), ko = __ldg(p.k_off + b);
+  it.qb = qo * p.q_sb; it.kb = ko * p.k_sb; it.vb = ko * p.v_sb; it.ob = qo * p.o_sb;
+  return true;
+}
 // One CTA per (batch item, head, chunk of ATT_QB queries): the query chunk and one tile of ATT_KT keys / values are staged
 // in shared memory (coalesced 128-bit loads, rows padded by 4 floats so that lanes <-> keys read conflict-free
 // LDS.128), every warp walks its queries over the tile with an online softmax (running max / sum / output, rescaled per
 // tile), so K and V are read from L2 once per CTA instead of once per query (the first version of this kernel did the
 // latter and was L2-bound: 215 us per launch on the 64 x 512 space attention, 4.5 of the 8 ms of a coarse forward).
 constexpr int ATT_QB = 64, ATT_KT = 64, ATT_WARPS = 8;
-template <int DH4>   // dh / 4 (dh <= 4 * DH4)
+template <int DH4, bool VARLEN>   // dh / 4 (dh <= 4 * DH4)
 __global__ void __launch_bounds__(ATT_WARPS * 32) attention_kernel(const AttnParams p) {
   constexpr int DH = 4 * DH4, KLD = DH + 4;
   constexpr int QPW = ATT_QB / ATT_WARPS;   // queries per warp
@@ -190,10 +227,12 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) attention_kernel(const AttnPar
     const int qc = (int)(blk % qchunks);
     const int h = (int)((blk / qchunks) % p.H);
     const int b = (int)(blk / ((long long)qchunks * p.H));
-    const int q0 = qc * ATT_QB, nq = min(ATT_QB, p.Lq - q0);
-    const float* qp = p.q + b * p.q_sb + h * p.dh;
-    const float* kp = p.k + b * p.k_sb + h * p.dh;
-    const float* vp = p.v + b * p.v_sb + h * p.dh;
+    AttnItem it;
+    if (!attn_item<VARLEN>(p, b, qc * ATT_QB, it)) continue;
+    const int q0 = qc * ATT_QB, nq = min(ATT_QB, it.Lq - q0);
+    const float* qp = p.q + it.qb + h * p.dh;
+    const float* kp = p.k + it.kb + h * p.dh;
+    const float* vp = p.v + it.vb + h * p.dh;
     const int dh4 = p.dh >> 2;
     __syncthreads();                       // previous chunk fully consumed
     for (int e = threadIdx.x; e < nq * DH4; e += blockDim.x) {
@@ -211,8 +250,8 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) attention_kernel(const AttnPar
     // scheduler instruction-level parallelism (one query at a time: 132 us on the 64 x 512 space attention, ncu r02).
     const int nmine = nq > warp ? (nq - warp + ATT_WARPS - 1) / ATT_WARPS : 0;     // warp-uniform
 
-    for (int k0 = 0; k0 < p.Lk; k0 += ATT_KT) {
-      const int nk = min(ATT_KT, p.Lk - k0);
+    for (int k0 = 0; k0 < it.Lk; k0 += ATT_KT) {
+      const int nk = min(ATT_KT, it.Lk - k0);
       __syncthreads();                     // Q staged / previous tile consumed
       for (int e = threadIdx.x; e < ATT_KT * DH4; e += blockDim.x) {
         const int r = e / DH4, t = e - r * DH4;
@@ -291,7 +330,7 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) attention_kernel(const AttnPar
       const int qi = u * ATT_WARPS + warp;
       if (qi >= nq) break;
       const float inv = 1.f / l[u];
-      const long long base = b * p.o_sb + (long long)(q0 + qi) * p.o_si + h * p.dh;
+      const long long base = it.ob + (long long)(q0 + qi) * p.o_si + h * p.dh;
       if (lane < p.dh) store_planes(p.out, p.o_plane_stride, base + lane, acc0[u] * inv, p.np);
       if (lane + 32 < p.dh) store_planes(p.out, p.o_plane_stride, base + lane + 32, acc1[u] * inv, p.np);
     }
@@ -422,8 +461,8 @@ __global__ void __launch_bounds__(ATS_WARPS * 32) attention_small_kernel(const A
 // attention_small_kernel -- no cross-lane reductions, K / V rows are broadcast reads.  (The tiled kernel needs ~500
 // instructions per query here, half of them warp reductions and probability traffic: 85 us per launch for the 512 x 64
 // point -> virtual attention; this formulation needs ~250.)
-constexpr int ATR_WARPS = 4, ATR_KMAX = 64;
-template <int DH4>
+constexpr int ATR_WARPS = 4;
+template <int DH4, bool VARLEN>
 __global__ void __launch_bounds__(ATR_WARPS * 32) attention_rows_kernel(const AttnParams p) {
   constexpr int DH = 4 * DH4, OLD = DH + 4;
   extern __shared__ __align__(16) float atr_smem[];
@@ -439,11 +478,13 @@ __global__ void __launch_bounds__(ATR_WARPS * 32) attention_rows_kernel(const At
     const int qc = (int)(blk % qchunks);
     const int h = (int)((blk / qchunks) % p.H);
     const int b = (int)(blk / ((long long)qchunks * p.H));
-    const float* qp = p.q + b * p.q_sb + h * p.dh;
-    const float* kp = p.k + b * p.k_sb + h * p.dh;
-    const float* vp = p.v + b * p.v_sb + h * p.dh;
+    AttnItem it;
+    if (!attn_item<VARLEN>(p, b, qc * (ATR_WARPS * 32), it)) continue;
+    const float* qp = p.q + it.qb + h * p.dh;
+    const float* kp = p.k + it.kb + h * p.dh;
+    const float* vp = p.v + it.vb + h * p.dh;
     __syncthreads();                            // previous chunk's K / V fully consumed
-    for (int e = threadIdx.x; e < p.Lk * DH4; e += blockDim.x) {
+    for (int e = threadIdx.x; e < it.Lk * DH4; e += blockDim.x) {
       const int r = e / DH4, t = e - r * DH4;
       float4 kk = make_float4(0.f, 0.f, 0.f, 0.f), vv = kk;
       if (t < dh4) {
@@ -454,7 +495,7 @@ __global__ void __launch_bounds__(ATR_WARPS * 32) attention_rows_kernel(const At
       reinterpret_cast<float4*>(Vs)[e] = vv;
     }
     const int qi = qc * (ATR_WARPS * 32) + warp * 32 + lane;
-    const bool active = qi < p.Lq;
+    const bool active = qi < it.Lq;
     float4 q4[DH4];
 #pragma unroll
     for (int t = 0; t < DH4; ++t) {
@@ -464,7 +505,7 @@ __global__ void __launch_bounds__(ATR_WARPS * 32) attention_rows_kernel(const At
     }
     __syncthreads();
     float mx = -INFINITY;
-    for (int j = 0; j < p.Lk; ++j) {
+    for (int j = 0; j < it.Lk; ++j) {
       const float4* kr = reinterpret_cast<const float4*>(Ks + j * DH);
       float sx = 0.f, sy = 0.f, sz = 0.f, sw = 0.f;      // four independent chains: one serial chain of dh FMAs is latency-bound
 #pragma unroll
@@ -480,7 +521,7 @@ __global__ void __launch_bounds__(ATR_WARPS * 32) attention_rows_kernel(const At
 #pragma unroll
     for (int t = 0; t < DH4; ++t) acc[t] = make_float4(0.f, 0.f, 0.f, 0.f);
     float sum = 0.f;
-    for (int j = 0; j < p.Lk; ++j) {
+    for (int j = 0; j < it.Lk; ++j) {
       const float pj = expf(Ss[j * 33 + lane] - mx);
       sum += pj;
       const float4* vr = reinterpret_cast<const float4*>(Vs + j * DH);
@@ -497,17 +538,17 @@ __global__ void __launch_bounds__(ATR_WARPS * 32) attention_rows_kernel(const At
       *reinterpret_cast<float4*>(Os + lane * OLD + 4 * t) = make_float4(acc[t].x * inv, acc[t].y * inv, acc[t].z * inv, acc[t].w * inv);
     __syncwarp();
     const int q0w = qc * (ATR_WARPS * 32) + warp * 32;
-    const int nqw = min(32, p.Lq - q0w);
+    const int nqw = min(32, it.Lq - q0w);
     if (p.vec_out) {
       for (int e = lane; e < nqw * dh4; e += 32) {
         const int i = e / dh4, t = e - i * dh4;
-        store_planes4(p.out, p.o_plane_stride, b * p.o_sb + (long long)(q0w + i) * p.o_si + h * p.dh + 4 * t,
+        store_planes4(p.out, p.o_plane_stride, it.ob + (long long)(q0w + i) * p.o_si + h * p.dh + 4 * t,
                       *reinterpret_cast<const float4*>(Os + i * OLD + 4 * t), p.np);
       }
     } else
     for (int e = lane; e < nqw * p.dh; e += 32) {
       const int i = e / p.dh, d = e - i * p.dh;
-      store_planes(p.out, p.o_plane_stride, b * p.o_sb + (long long)(q0w + i) * p.o_si + h * p.dh + d, Os[i * OLD + d], p.np);
+      store_planes(p.out, p.o_plane_stride, it.ob + (long long)(q0w + i) * p.o_si + h * p.dh + d, Os[i * OLD + d], p.np);
     }
     __syncwarp();
   }
@@ -530,22 +571,24 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
   const __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
   return *reinterpret_cast<const uint32_t*>(&v);
 }
-template <int DH>   // head dimension, a multiple of 16
+template <int DH, bool VARLEN>   // head dimension, a multiple of 16
 __global__ void __launch_bounds__(ATM_WARPS * 32) attention_rows_mma_kernel(const AttnParams p) {
   constexpr int KLD = DH + 8, VLD = 64 + 8, KS = DH / 16, DT = DH / 8;
   __shared__ __align__(16) __nv_bfloat16 Ks[64 * KLD];    // [key][dh]
   __shared__ __align__(16) __nv_bfloat16 Vt[DH * VLD];    // [dim][key]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
   const int qchunks = (p.Lq + ATM_WARPS * 16 - 1) / (ATM_WARPS * 16);
-  const int ktiles = (p.Lk + 63) / 64;          // more than 64 keys: tiles of 64 with the online-softmax rescale
   const long long nblocks = (long long)p.B * p.H * qchunks;
   for (long long blk = blockIdx.x; blk < nblocks; blk += gridDim.x) {
     const int qc = (int)(blk % qchunks);
     const int h = (int)((blk / qchunks) % p.H);
     const int b = (int)(blk / ((long long)qchunks * p.H));
-    const float* qp = p.q + b * p.q_sb + h * DH;
-    const float* kp = p.k + b * p.k_sb + h * DH;
-    const float* vp = p.v + b * p.v_sb + h * DH;
+    AttnItem it;
+    if (!attn_item<VARLEN>(p, b, qc * (ATM_WARPS * 16), it)) continue;
+    const int ktiles = (it.Lk + 63) / 64;        // more than 64 keys: tiles of 64 with the online-softmax rescale
+    const float* qp = p.q + it.qb + h * DH;
+    const float* kp = p.k + it.kb + h * DH;
+    const float* vp = p.v + it.vb + h * DH;
     // this warp's 16 queries as A fragments (rows g and g + 8; MHA scales q before the product)
     const int q0 = qc * (ATM_WARPS * 16) + warp * 16;
     const int r0 = q0 + g, r1 = q0 + g + 8;
@@ -553,11 +596,11 @@ __global__ void __launch_bounds__(ATM_WARPS * 32) attention_rows_mma_kernel(cons
 #pragma unroll
     for (int ks = 0; ks < KS; ++ks) {
       float2 x00 = make_float2(0.f, 0.f), x01 = x00, x10 = x00, x11 = x00;
-      if (r0 < p.Lq) {
+      if (r0 < it.Lq) {
         x00 = __ldg(reinterpret_cast<const float2*>(qp + (long long)r0 * p.q_si + ks * 16 + 2 * t));
         x01 = __ldg(reinterpret_cast<const float2*>(qp + (long long)r0 * p.q_si + ks * 16 + 2 * t + 8));
       }
-      if (r1 < p.Lq) {
+      if (r1 < it.Lq) {
         x10 = __ldg(reinterpret_cast<const float2*>(qp + (long long)r1 * p.q_si + ks * 16 + 2 * t));
         x11 = __ldg(reinterpret_cast<const float2*>(qp + (long long)r1 * p.q_si + ks * 16 + 2 * t + 8));
       }
@@ -577,7 +620,7 @@ __global__ void __launch_bounds__(ATM_WARPS * 32) attention_rows_mma_kernel(cons
       for (int e = threadIdx.x; e < 64 * (DH / 4); e += blockDim.x) {
         const int r = e / (DH / 4), c4 = e - r * (DH / 4);
         float4 kk = make_float4(0.f, 0.f, 0.f, 0.f), vv = kk;
-        if (key0 + r < p.Lk) {
+        if (key0 + r < it.Lk) {
           kk = __ldg(reinterpret_cast<const float4*>(kp + (long long)(key0 + r) * p.k_si) + c4);
           vv = __ldg(reinterpret_cast<const float4*>(vp + (long long)(key0 + r) * p.v_si) + c4);
         }
@@ -588,7 +631,7 @@ __global__ void __launch_bounds__(ATM_WARPS * 32) attention_rows_mma_kernel(cons
         Vt[(4 * c4 + 3) * VLD + r] = __float2bfloat16_rn(vv.w);
       }
       __syncthreads();
-      if (q0 >= p.Lq) continue;                 // warp-uniform: this warp only helps with the staging
+      if (q0 >= it.Lq) continue;                 // warp-uniform: this warp only helps with the staging
       // S = q k^T: 8 key tiles of 8
       float sacc[8][4];
 #pragma unroll
@@ -605,8 +648,8 @@ __global__ void __launch_bounds__(ATM_WARPS * 32) attention_rows_mma_kernel(cons
 #pragma unroll
       for (int nt = 0; nt < 8; ++nt) {
         const int key = key0 + nt * 8 + 2 * t;
-        if (key >= p.Lk) { sacc[nt][0] = -INFINITY; sacc[nt][2] = -INFINITY; }
-        if (key + 1 >= p.Lk) { sacc[nt][1] = -INFINITY; sacc[nt][3] = -INFINITY; }
+        if (key >= it.Lk) { sacc[nt][0] = -INFINITY; sacc[nt][2] = -INFINITY; }
+        if (key + 1 >= it.Lk) { sacc[nt][1] = -INFINITY; sacc[nt][3] = -INFINITY; }
         t0 = fmaxf(t0, fmaxf(sacc[nt][0], sacc[nt][1]));
         t1 = fmaxf(t1, fmaxf(sacc[nt][2], sacc[nt][3]));
       }
@@ -643,14 +686,14 @@ __global__ void __launch_bounds__(ATM_WARPS * 32) attention_rows_mma_kernel(cons
         }
       }
     }
-    if (q0 < p.Lq) {
+    if (q0 < it.Lq) {
       const float i0 = 1.f / l0, i1 = 1.f / l1;
-      __nv_bfloat16* o0 = p.out + b * p.o_sb + (long long)r0 * p.o_si + h * DH + 2 * t;
-      __nv_bfloat16* o1 = p.out + b * p.o_sb + (long long)r1 * p.o_si + h * DH + 2 * t;
+      __nv_bfloat16* o0 = p.out + it.ob + (long long)r0 * p.o_si + h * DH + 2 * t;
+      __nv_bfloat16* o1 = p.out + it.ob + (long long)r1 * p.o_si + h * DH + 2 * t;
 #pragma unroll
       for (int dt = 0; dt < DT; ++dt) {
-        if (r0 < p.Lq) *reinterpret_cast<uint32_t*>(o0 + dt * 8) = pack_bf16(oacc[dt][0] * i0, oacc[dt][1] * i0);
-        if (r1 < p.Lq) *reinterpret_cast<uint32_t*>(o1 + dt * 8) = pack_bf16(oacc[dt][2] * i1, oacc[dt][3] * i1);
+        if (r0 < it.Lq) *reinterpret_cast<uint32_t*>(o0 + dt * 8) = pack_bf16(oacc[dt][0] * i0, oacc[dt][1] * i0);
+        if (r1 < it.Lq) *reinterpret_cast<uint32_t*>(o1 + dt * 8) = pack_bf16(oacc[dt][2] * i1, oacc[dt][3] * i1);
       }
     }
   }
@@ -773,7 +816,7 @@ __global__ void __launch_bounds__(ATSM_WARPS * 32) attention_small_mma_kernel(co
 // results (running max, sum, output row) of a query are merged through shared memory at the end.  (The tiled kernel gives
 // this shape 128 CTAs of dependent warp reductions: 108 us per launch at N = 512.)
 constexpr int AKS_SPLITS = 4, AKS_KT = 64;
-template <int DH4>
+template <int DH4, bool VARLEN>
 __global__ void __launch_bounds__(256) attention_ksplit_kernel(const AttnParams p) {
   constexpr int DH = 4 * DH4, MP = DH + 8;       // merge row pitch: DH outputs, max, sum; a multiple of 4 floats (float4 rows)
   extern __shared__ __align__(16) float aks_smem[];
@@ -785,17 +828,19 @@ __global__ void __launch_bounds__(256) attention_ksplit_kernel(const AttnParams 
   float* Mg = aks_smem;                                            // merge area (reuses the K / V tiles): [split][64][MP]
   const int dh4 = p.dh >> 2;
   const int qchunks = (p.Lq + 63) / 64;
-  const int per_split = (((p.Lk + AKS_SPLITS - 1) / AKS_SPLITS) + AKS_KT - 1) / AKS_KT * AKS_KT;   // keys per split, tile multiple
   const long long nblocks = (long long)p.B * p.H * qchunks;
   for (long long blk = blockIdx.x; blk < nblocks; blk += gridDim.x) {
     const int qc = (int)(blk % qchunks);
     const int h = (int)((blk / qchunks) % p.H);
     const int b = (int)(blk / ((long long)qchunks * p.H));
-    const float* qp = p.q + b * p.q_sb + h * p.dh;
-    const float* kp = p.k + b * p.k_sb + h * p.dh;
-    const float* vp = p.v + b * p.v_sb + h * p.dh;
+    AttnItem it;
+    if (!attn_item<VARLEN>(p, b, qc * 64, it)) continue;
+    const int per_split = (((it.Lk + AKS_SPLITS - 1) / AKS_SPLITS) + AKS_KT - 1) / AKS_KT * AKS_KT;   // keys per split, tile multiple
+    const float* qp = p.q + it.qb + h * p.dh;
+    const float* kp = p.k + it.kb + h * p.dh;
+    const float* vp = p.v + it.vb + h * p.dh;
     const int qi = qc * 64 + grp * 32 + lane;
-    const bool active = qi < p.Lq;
+    const bool active = qi < it.Lq;
     float4 q4[DH4];
 #pragma unroll
     for (int t = 0; t < DH4; ++t) {
@@ -814,7 +859,7 @@ __global__ void __launch_bounds__(256) attention_ksplit_kernel(const AttnParams 
         const int sp = e / (AKS_KT * DH4), r = (e / DH4) % AKS_KT, t = e % DH4;
         const int key = sp * per_split + t0 + r;
         float4 kk = make_float4(0.f, 0.f, 0.f, 0.f), vv = kk;
-        if (key < p.Lk && key < (sp + 1) * per_split && t < dh4) {
+        if (key < it.Lk && key < (sp + 1) * per_split && t < dh4) {
           kk = __ldg(reinterpret_cast<const float4*>(kp + (long long)key * p.k_si) + t);
           vv = __ldg(reinterpret_cast<const float4*>(vp + (long long)key * p.v_si) + t);
         }
@@ -823,7 +868,7 @@ __global__ void __launch_bounds__(256) attention_ksplit_kernel(const AttnParams 
         reinterpret_cast<float4*>(dstk + AKS_KT * DH)[r * DH4 + t] = vv;
       }
       __syncthreads();
-      const int nk = max(0, min(AKS_KT, min(p.Lk, (split + 1) * per_split) - (split * per_split + t0)));   // warp-uniform
+      const int nk = max(0, min(AKS_KT, min(it.Lk, (split + 1) * per_split) - (split * per_split + t0)));   // warp-uniform
       if (nk > 0) {
         float mx = mrun;
         for (int j = 0; j < nk; ++j) {
@@ -892,17 +937,17 @@ __global__ void __launch_bounds__(256) attention_ksplit_kernel(const AttnParams 
         *reinterpret_cast<float4*>(Os + lane * MP + 4 * t) = make_float4(acc[t].x * inv, acc[t].y * inv, acc[t].z * inv, acc[t].w * inv);
       __syncwarp();
       const int q0w = qc * 64 + grp * 32;
-      const int nqw = min(32, p.Lq - q0w);
+      const int nqw = min(32, it.Lq - q0w);
       if (p.vec_out) {
         for (int e = lane; e < nqw * (p.dh >> 2); e += 32) {
           const int i = e / (p.dh >> 2), t = e - i * (p.dh >> 2);
-          store_planes4(p.out, p.o_plane_stride, b * p.o_sb + (long long)(q0w + i) * p.o_si + h * p.dh + 4 * t,
+          store_planes4(p.out, p.o_plane_stride, it.ob + (long long)(q0w + i) * p.o_si + h * p.dh + 4 * t,
                         *reinterpret_cast<const float4*>(Os + i * MP + 4 * t), p.np);
         }
       } else
       for (int e = lane; e < nqw * p.dh; e += 32) {
         const int i = e / p.dh, d = e - i * p.dh;
-        store_planes(p.out, p.o_plane_stride, b * p.o_sb + (long long)(q0w + i) * p.o_si + h * p.dh + d, Os[i * MP + d], p.np);
+        store_planes(p.out, p.o_plane_stride, it.ob + (long long)(q0w + i) * p.o_si + h * p.dh + d, Os[i * MP + d], p.np);
       }
     }
   }
@@ -959,6 +1004,102 @@ extern "C" int comet_layernorm_planes_f32(const float* x, long long x_ld, const 
   return launch_status("layernorm_planes_kernel");
 }
 
+// One launch of kernel family `path` over p.B problems (grid sized from the largest query length p.Lq).
+template <bool VARLEN>
+static int launch_attention(int path, const AttnParams& p, cudaStream_t stream) {
+  const long long B = p.B;
+  const int H = p.H, Lq = p.Lq, dh = p.dh;
+  if (path == AP_SMALL_MMA) {
+    long long nb = (B * H + ATSM_WARPS - 1) / ATSM_WARPS;
+    if (nb > 148LL * 16) nb = 148LL * 16;
+    if (dh == 32) attention_small_mma_kernel<32><<<(unsigned)nb, ATSM_WARPS * 32, 0, stream>>>(p);
+    else attention_small_mma_kernel<48><<<(unsigned)nb, ATSM_WARPS * 32, 0, stream>>>(p);
+    return launch_status("attention_small_mma_kernel");
+  }
+  if (path == AP_SMALL) {
+    long long nb = (B * H + ATS_WARPS - 1) / ATS_WARPS;
+    if (nb > 148LL * 16) nb = 148LL * 16;
+#define COMET_ATS_LAUNCH(D4)                                                                                       \
+  do {                                                                                                             \
+    const int smem = ATS_WARPS * (32 * 4 * D4 + 32 * (4 * D4 + 4) + 32 * 33) * (int)sizeof(float);                 \
+    if (smem > 48 * 1024)                                                                                          \
+      COMET_CUDA(cudaFuncSetAttribute(attention_small_kernel<D4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
+    attention_small_kernel<D4><<<(unsigned)nb, ATS_WARPS * 32, smem, stream>>>(p);                                 \
+  } while (0)
+    if (dh <= 4) COMET_ATS_LAUNCH(1);
+    else if (dh <= 16) COMET_ATS_LAUNCH(4);
+    else if (dh <= 32) COMET_ATS_LAUNCH(8);
+    else if (dh <= 48) COMET_ATS_LAUNCH(12);
+    else COMET_ATS_LAUNCH(16);
+#undef COMET_ATS_LAUNCH
+    return launch_status("attention_small_kernel");
+  }
+  if (path == AP_ROWS_MMA) {
+    long long nb = B * H * ((Lq + ATM_WARPS * 16 - 1) / (ATM_WARPS * 16));
+    if (nb > 148LL * 16) nb = 148LL * 16;
+    if (dh == 32) attention_rows_mma_kernel<32, VARLEN><<<(unsigned)nb, ATM_WARPS * 32, 0, stream>>>(p);
+    else if (dh == 48) attention_rows_mma_kernel<48, VARLEN><<<(unsigned)nb, ATM_WARPS * 32, 0, stream>>>(p);
+    else attention_rows_mma_kernel<64, VARLEN><<<(unsigned)nb, ATM_WARPS * 32, 0, stream>>>(p);
+    return launch_status("attention_rows_mma_kernel");
+  }
+  if (path == AP_ROWS) {
+    long long nb = B * H * ((Lq + ATR_WARPS * 32 - 1) / (ATR_WARPS * 32));
+    if (nb > 148LL * 16) nb = 148LL * 16;
+#define COMET_ATR_LAUNCH(D4)                                                                                       \
+  do {                                                                                                             \
+    const int smem = (2 * ATR_KMAX * 4 * D4 + ATR_WARPS * (ATR_KMAX * 33 + 32 * (4 * D4 + 4))) * (int)sizeof(float); \
+    if (smem > 48 * 1024)                                                                                          \
+      COMET_CUDA(cudaFuncSetAttribute(attention_rows_kernel<D4, VARLEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
+    attention_rows_kernel<D4, VARLEN><<<(unsigned)nb, ATR_WARPS * 32, smem, stream>>>(p);                                  \
+  } while (0)
+    if (dh <= 4) COMET_ATR_LAUNCH(1);
+    else if (dh <= 16) COMET_ATR_LAUNCH(4);
+    else if (dh <= 32) COMET_ATR_LAUNCH(8);
+    else if (dh <= 48) COMET_ATR_LAUNCH(12);
+    else COMET_ATR_LAUNCH(16);
+#undef COMET_ATR_LAUNCH
+    return launch_status("attention_rows_kernel");
+  }
+  if (path == AP_KSPLIT) {
+    long long nb = B * H * ((Lq + 63) / 64);
+    if (nb > 148LL * 16) nb = 148LL * 16;   // (a single call takes this path only at <= 148 * 4 CTAs)
+#define COMET_AKS_LAUNCH(D4)                                                                                       \
+  do {                                                                                                             \
+    const int smem = (AKS_SPLITS * 2 * AKS_KT * 4 * D4 + 8 * AKS_KT * 33) * (int)sizeof(float);                    \
+    if (smem > 48 * 1024)                                                                                          \
+      COMET_CUDA(cudaFuncSetAttribute(attention_ksplit_kernel<D4, VARLEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
+    attention_ksplit_kernel<D4, VARLEN><<<(unsigned)nb, 256, smem, stream>>>(p);                                           \
+  } while (0)
+    if (dh <= 4) COMET_AKS_LAUNCH(1);
+    else if (dh <= 16) COMET_AKS_LAUNCH(4);
+    else if (dh <= 32) COMET_AKS_LAUNCH(8);
+    else if (dh <= 48) COMET_AKS_LAUNCH(12);
+    else COMET_AKS_LAUNCH(16);
+#undef COMET_AKS_LAUNCH
+    return launch_status("attention_ksplit_kernel");
+  }
+  long long blocks = B * H * ((Lq + ATT_QB - 1) / ATT_QB);
+  if (blocks > 148LL * 16) blocks = 148LL * 16;
+#define COMET_ATTN_LAUNCH(D4)                                                                                       \
+  do {                                                                                                              \
+    const int smem = (ATT_QB * 4 * D4 + ATT_KT * (4 * D4 + 4) + ATT_KT * 4 * D4 + ATT_QB * ATT_KT) * (int)sizeof(float); \
+    if (smem > 48 * 1024)                                                                                           \
+      COMET_CUDA(cudaFuncSetAttribute(attention_kernel<D4, VARLEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));    \
+    attention_kernel<D4, VARLEN><<<(unsigned)blocks, ATT_WARPS * 32, smem, stream>>>(p);                                    \
+  } while (0)
+  if (dh <= 4) COMET_ATTN_LAUNCH(1);
+  else if (dh <= 16) COMET_ATTN_LAUNCH(4);
+  else if (dh <= 32) COMET_ATTN_LAUNCH(8);
+  else if (dh <= 48) COMET_ATTN_LAUNCH(12);
+  else COMET_ATTN_LAUNCH(16);
+#undef COMET_ATTN_LAUNCH
+  return launch_status("attention_kernel");
+}
+
+static int mma_alignment(long long q_sb, long long q_si, long long o_sb, long long o_si, const void* out_planes) {
+  return (o_sb % 2 == 0 && o_si % 2 == 0 && ((uintptr_t)out_planes % 4) == 0 && q_si % 2 == 0 && q_sb % 2 == 0) ? 1 : 0;
+}
+
 extern "C" int comet_attention_planes_f32(const float* q, long long q_sb, long long q_si, const float* k, long long k_sb,
                                           long long k_si, const float* v, long long v_sb, long long v_si, void* out_planes,
                                           long long o_plane_stride, long long o_sb, long long o_si, int np, int B, int H,
@@ -975,92 +1116,52 @@ extern "C" int comet_attention_planes_f32(const float* q, long long q_sb, long l
   AttnParams p{q, q_sb, q_si, k, k_sb, k_si, v, v_sb, v_si, reinterpret_cast<__nv_bfloat16*>(out_planes),
                o_plane_stride, o_sb, o_si, np, B, H, Lq, Lk, dh, 1.0f / sqrtf((float)dh),
                (o_sb % 4 == 0 && o_si % 4 == 0 && o_plane_stride % 4 == 0 && ((uintptr_t)out_planes % 8) == 0) ? 1 : 0};
-  if (np == 1 && Lq <= 16 && Lk <= 32 && (dh == 32 || dh == 48) && (option(COMET_OPT_ATTN_MMA) & 2) && o_sb % 2 == 0 &&
-      o_si % 2 == 0 && ((uintptr_t)out_planes % 4) == 0 && q_si % 2 == 0 && q_sb % 2 == 0) {
-    long long nb = ((long long)B * H + ATSM_WARPS - 1) / ATSM_WARPS;
-    if (nb > 148LL * 16) nb = 148LL * 16;
-    if (dh == 32) attention_small_mma_kernel<32><<<(unsigned)nb, ATSM_WARPS * 32, 0, (cudaStream_t)stream>>>(p);
-    else attention_small_mma_kernel<48><<<(unsigned)nb, ATSM_WARPS * 32, 0, (cudaStream_t)stream>>>(p);
-    return launch_status("attention_small_mma_kernel");
+  const int path = attn_path(np, Lq, Lk, dh, B, H, option(COMET_OPT_ATTN_MMA),
+                             mma_alignment(q_sb, q_si, o_sb, o_si, out_planes));
+  return launch_attention<false>(path, p, (cudaStream_t)stream);
+}
+
+extern "C" int comet_attention_varlen_planes_f32(const float* q, long long q_ld, long long q_step, const float* k,
+                                                 long long k_ld, long long k_step, const float* v, void* out_planes,
+                                                 long long o_plane_stride, long long o_ld, int np, int items, int H, int dh,
+                                                 const int* q_off, const int* q_len, const int* k_off, const int* k_len,
+                                                 int min_lq, int max_lq, int min_lk, int max_lk, int group,
+                                                 comet_stream_t stream) {
+  COMET_REQUIRE(items >= 0 && H >= 1 && min_lq >= 1 && max_lq >= min_lq && min_lk >= 1 && max_lk >= min_lk && group >= 1 &&
+                    dh >= 4 && dh <= 64 && dh % 4 == 0,
+                "bad varlen attention shape (items=%d H=%d Lq in [%d, %d] Lk in [%d, %d] group=%d dh=%d)", items, H, min_lq,
+                max_lq, min_lk, max_lk, group, dh);
+  COMET_REQUIRE(np == 1 || np == 3, "np must be 1 or 3");
+  if ((long long)items * max_lq == 0) return COMET_OK;
+  COMET_REQUIRE(q && k && v && out_planes && q_off && q_len && k_off && k_len, "null pointer");
+  COMET_REQUIRE(((uintptr_t)q % 16) == 0 && ((uintptr_t)k % 16) == 0 && ((uintptr_t)v % 16) == 0 && q_ld % 4 == 0 &&
+                    k_ld % 4 == 0, "q / k / v rows must be 16-byte aligned");
+  AttnParams p{q, q_ld, q_step * q_ld, k, k_ld, k_step * k_ld, v, k_ld, k_step * k_ld,
+               reinterpret_cast<__nv_bfloat16*>(out_planes), o_plane_stride, o_ld, q_step * o_ld, np, items, H, max_lq,
+               max_lk, dh, 1.0f / sqrtf((float)dh),
+               (o_ld % 4 == 0 && (q_step * o_ld) % 4 == 0 && o_plane_stride % 4 == 0 && ((uintptr_t)out_planes % 8) == 0) ? 1 : 0};
+  p.q_off = q_off; p.q_len = q_len; p.k_off = k_off; p.k_len = k_len;
+  p.group = group;
+  p.mma_opt = option(COMET_OPT_ATTN_MMA);
+  p.mma_align = mma_alignment(q_ld, q_step * q_ld, o_ld, q_step * o_ld, out_planes);
+  // The lengths live on the device: launch every family that some length pair of the given ranges selects (the path
+  // depends on a length only through the thresholds 16 / 32 / 64 and the number of 64-query chunks, so every length up
+  // to 65 and then every 64th is enough); each CTA serves the items of its own family.
+  auto next = [](int x, int hi) { return x < 65 ? x + 1 : x < hi ? (x + 64 < hi ? x + 64 : hi) : hi + 1; };
+  bool used[AP_COUNT] = {};
+  for (int lq = min_lq; lq <= max_lq; lq = next(lq, max_lq))
+    for (int lk = min_lk; lk <= max_lk; lk = next(lk, max_lk))
+      used[attn_path(np, lq, lk, dh, group, H, p.mma_opt, p.mma_align)] = true;
+  COMET_REQUIRE(!used[AP_SMALL] && !used[AP_SMALL_MMA],
+                "varlen attention serves items with more than 32 queries or more than 32 keys (Lq in [%d, %d], Lk in [%d, %d])",
+                min_lq, max_lq, min_lk, max_lk);
+  for (int path = 0; path < AP_COUNT; ++path) {
+    if (!used[path]) continue;
+    p.path = path;
+    const int rc = launch_attention<true>(path, p, (cudaStream_t)stream);
+    if (rc != COMET_OK) return rc;
   }
-  if (Lq <= 32 && Lk <= 32) {
-    long long nb = ((long long)B * H + ATS_WARPS - 1) / ATS_WARPS;
-    if (nb > 148LL * 16) nb = 148LL * 16;
-#define COMET_ATS_LAUNCH(D4)                                                                                       \
-  do {                                                                                                             \
-    const int smem = ATS_WARPS * (32 * 4 * D4 + 32 * (4 * D4 + 4) + 32 * 33) * (int)sizeof(float);                 \
-    if (smem > 48 * 1024)                                                                                          \
-      COMET_CUDA(cudaFuncSetAttribute(attention_small_kernel<D4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-    attention_small_kernel<D4><<<(unsigned)nb, ATS_WARPS * 32, smem, (cudaStream_t)stream>>>(p);                   \
-  } while (0)
-    if (dh <= 4) COMET_ATS_LAUNCH(1);
-    else if (dh <= 16) COMET_ATS_LAUNCH(4);
-    else if (dh <= 32) COMET_ATS_LAUNCH(8);
-    else if (dh <= 48) COMET_ATS_LAUNCH(12);
-    else COMET_ATS_LAUNCH(16);
-#undef COMET_ATS_LAUNCH
-    return launch_status("attention_small_kernel");
-  }
-  if (np == 1 && Lq >= 64 && (dh == 32 || dh == 48 || dh == 64) && (option(COMET_OPT_ATTN_MMA) & 1) &&
-      o_sb % 2 == 0 && o_si % 2 == 0 && ((uintptr_t)out_planes % 4) == 0 && q_si % 2 == 0 && q_sb % 2 == 0) {
-    long long nb = (long long)B * H * ((Lq + ATM_WARPS * 16 - 1) / (ATM_WARPS * 16));
-    if (nb > 148LL * 16) nb = 148LL * 16;
-    if (dh == 32) attention_rows_mma_kernel<32><<<(unsigned)nb, ATM_WARPS * 32, 0, (cudaStream_t)stream>>>(p);
-    else if (dh == 48) attention_rows_mma_kernel<48><<<(unsigned)nb, ATM_WARPS * 32, 0, (cudaStream_t)stream>>>(p);
-    else attention_rows_mma_kernel<64><<<(unsigned)nb, ATM_WARPS * 32, 0, (cudaStream_t)stream>>>(p);
-    return launch_status("attention_rows_mma_kernel");
-  }
-  if (Lk <= ATR_KMAX && Lq >= 64) {
-    long long nb = (long long)B * H * ((Lq + ATR_WARPS * 32 - 1) / (ATR_WARPS * 32));
-    if (nb > 148LL * 16) nb = 148LL * 16;
-#define COMET_ATR_LAUNCH(D4)                                                                                       \
-  do {                                                                                                             \
-    const int smem = (2 * ATR_KMAX * 4 * D4 + ATR_WARPS * (ATR_KMAX * 33 + 32 * (4 * D4 + 4))) * (int)sizeof(float); \
-    if (smem > 48 * 1024)                                                                                          \
-      COMET_CUDA(cudaFuncSetAttribute(attention_rows_kernel<D4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-    attention_rows_kernel<D4><<<(unsigned)nb, ATR_WARPS * 32, smem, (cudaStream_t)stream>>>(p);                    \
-  } while (0)
-    if (dh <= 4) COMET_ATR_LAUNCH(1);
-    else if (dh <= 16) COMET_ATR_LAUNCH(4);
-    else if (dh <= 32) COMET_ATR_LAUNCH(8);
-    else if (dh <= 48) COMET_ATR_LAUNCH(12);
-    else COMET_ATR_LAUNCH(16);
-#undef COMET_ATR_LAUNCH
-    return launch_status("attention_rows_kernel");
-  }
-  if (Lk > ATR_KMAX && (long long)B * H * ((Lq + 63) / 64) <= 148LL * 4) {
-    long long nb = (long long)B * H * ((Lq + 63) / 64);
-#define COMET_AKS_LAUNCH(D4)                                                                                       \
-  do {                                                                                                             \
-    const int smem = (AKS_SPLITS * 2 * AKS_KT * 4 * D4 + 8 * AKS_KT * 33) * (int)sizeof(float);                    \
-    if (smem > 48 * 1024)                                                                                          \
-      COMET_CUDA(cudaFuncSetAttribute(attention_ksplit_kernel<D4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-    attention_ksplit_kernel<D4><<<(unsigned)nb, 256, smem, (cudaStream_t)stream>>>(p);                             \
-  } while (0)
-    if (dh <= 4) COMET_AKS_LAUNCH(1);
-    else if (dh <= 16) COMET_AKS_LAUNCH(4);
-    else if (dh <= 32) COMET_AKS_LAUNCH(8);
-    else if (dh <= 48) COMET_AKS_LAUNCH(12);
-    else COMET_AKS_LAUNCH(16);
-#undef COMET_AKS_LAUNCH
-    return launch_status("attention_ksplit_kernel");
-  }
-  long long blocks = (long long)B * H * ((Lq + ATT_QB - 1) / ATT_QB);
-  if (blocks > 148LL * 16) blocks = 148LL * 16;
-#define COMET_ATTN_LAUNCH(D4)                                                                                       \
-  do {                                                                                                              \
-    const int smem = (ATT_QB * 4 * D4 + ATT_KT * (4 * D4 + 4) + ATT_KT * 4 * D4 + ATT_QB * ATT_KT) * (int)sizeof(float); \
-    if (smem > 48 * 1024)                                                                                           \
-      COMET_CUDA(cudaFuncSetAttribute(attention_kernel<D4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));    \
-    attention_kernel<D4><<<(unsigned)blocks, ATT_WARPS * 32, smem, (cudaStream_t)stream>>>(p);                      \
-  } while (0)
-  if (dh <= 4) COMET_ATTN_LAUNCH(1);
-  else if (dh <= 16) COMET_ATTN_LAUNCH(4);
-  else if (dh <= 32) COMET_ATTN_LAUNCH(8);
-  else if (dh <= 48) COMET_ATTN_LAUNCH(12);
-  else COMET_ATTN_LAUNCH(16);
-#undef COMET_ATTN_LAUNCH
-  return launch_status("attention_kernel");
+  return COMET_OK;
 }
 
 extern "C" int comet_add_planes_f32(const float* a, const float* b, void* planes, long long plane_stride, int np, long long n,

@@ -97,6 +97,25 @@ def run_sharded(items: Sequence[Any], fn: Callable[[Any], Any], rank: Optional[i
     return {i: fn(items[i]) for i in shard_indices(len(items), rank, world)}
 
 
+def run_sharded_batched(items: Sequence[Any], fn: Callable[[List[Any]], Sequence[Any]], batch_size: int,
+                        rank: Optional[int] = None, world: Optional[int] = None) -> Dict[int, Any]:
+    """``run_sharded`` for a batched ``fn``: this rank's round-robin shard is cut, in order, into batches of at most
+    ``batch_size`` items; ``fn(list of items)`` returns one result per item.  Returns {global index: result}, the same
+    mapping ``run_sharded`` returns, so ``gather_results`` applies unchanged."""
+    assert batch_size >= 1
+    env = dist_env()
+    rank = env["RANK"] if rank is None else rank
+    world = env["WORLD_SIZE"] if world is None else world
+    mine = shard_indices(len(items), rank, world)
+    out: Dict[int, Any] = {}
+    for k in range(0, len(mine), batch_size):
+        idx = mine[k:k + batch_size]
+        res = list(fn([items[i] for i in idx]))
+        assert len(res) == len(idx), f"batched fn returned {len(res)} results for {len(idx)} items"
+        out.update(zip(idx, res))
+    return out
+
+
 def gather_results(local: Dict[int, Any], n_items: int) -> Optional[List[Any]]:
     """End-of-run gather of per-sequence results (small objects: metrics, poses) to rank 0, in global order.
     This is the only collective of the inference path."""

@@ -171,6 +171,26 @@ class ShallowEncoder(nn.Module):
                 float(self.norm1.eps), stream_ptr(images.device)))
         return self._fused_result(out, (31 // self.stride, 31 // self.stride), defer_upsample)
 
+    def encode_packed_patches_of(self, images: torch.Tensor, topleft: torch.Tensor, seq_of_track: torch.Tensor,
+                                 defer_upsample: bool = True):
+        """``encode_patches_of`` for P tracks packed from the sequences of ``images`` (B,S,3,H,W): ``topleft`` (P,S,2)
+        corners, ``seq_of_track`` (P,) the sequence of each track.  Maps in (track, frame) order, each one bit-identical
+        to ``encode_patches_of`` on the same patch."""
+        from . import _lib
+        from ._dev import stream_ptr
+
+        B, S, _, H, W = images.shape
+        P = topleft.shape[0]
+        img = images.contiguous()
+        tl32 = topleft.to(torch.int32).contiguous()
+        seq32 = seq_of_track.to(device=images.device, dtype=torch.int32).contiguous()
+        out = torch.empty((P * S, 16, 16, 32), dtype=torch.float32, device=images.device)
+        with torch.cuda.device(images.device):
+            _lib.check(_lib.lib.comet_shallow_encoder_from_images_ragged_f32(
+                img.data_ptr(), tl32.data_ptr(), seq32.data_ptr(), self.packed_parameters().data_ptr(), out.data_ptr(), P, B,
+                S, H, W, float(self.norm1.eps), stream_ptr(images.device)))
+        return self._fused_result(out, (31 // self.stride, 31 // self.stride), defer_upsample)
+
     def forward(self, x, defer_upsample: bool = False):
         """``defer_upsample=True`` returns the map *before* the last resize together with the size that resize would
         produce -- ``(x_half, (Ho, Wo))`` -- for callers that consume the up-sampling lazily (:class:`Upsampled2x`)."""
@@ -230,9 +250,19 @@ def extract_patches(images: torch.Tensor, topleft: torch.Tensor, psize: int) -> 
     return patches.reshape(B * N * S, psize, psize, C).permute(0, 3, 1, 2)  # NCHW shape, NHWC memory
 
 
-def refine_track(images, fine_fnet, fine_tracker, coarse_pred, pradius=15, sradius=2, compute_score=False):
+def refine_track(images, fine_fnet, fine_tracker, coarse_pred, pradius=15, sradius=2, compute_score=False,
+                 num_tracks=None):
     """refine_track.py:26-171.  ``images`` (B,S,3,H,W); ``coarse_pred`` (B,S,N,2) pixels ->
-    (refined_tracks (B,S,N,2), score (B,S,N) | None)."""
+    (refined_tracks (B,S,N,2), score (B,S,N) | None).
+
+    ``num_tracks`` (B ints or a 1-D tensor): ``coarse_pred`` is a padded batch; sequence b's tracks get what the call on
+    that sequence alone returns (including the score quirk as it behaves for one sequence: every window of sequence b
+    is cut from the frame-0 map of its own first track), entries of padded tracks are 0."""
+    if num_tracks is not None:
+        from .utils import check_num_tracks
+
+        counts = check_num_tracks(num_tracks, coarse_pred.shape[0], coarse_pred.shape[2])
+        return _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, sradius, compute_score, counts)
     B, S, N, _ = coarse_pred.shape
     _, _, _, H, W = images.shape
     psize = pradius * 2 + 1
@@ -299,6 +329,118 @@ def refine_track(images, fine_fnet, fine_tracker, coarse_pred, pradius=15, sradi
     if compute_score:
         score = compute_score_fn(query_point_feat, patch_feat, fine_pred_track, sradius, psize, B, N, S, C_out)
     return refined_tracks, score
+
+
+def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, sradius, compute_score, counts):
+    """The fine tracker works per track, so the real tracks of all sequences run as ONE packed batch of P = sum(counts)
+    tracks, without per-sequence padding: the fused encoder reads each track's patches from its own sequence's frames.  Configurations
+    without the fused encoder run the per-sequence definition."""
+    from .base_track_predictor import BaseTrackerPredictor
+
+    B, S, N, _ = coarse_pred.shape
+    _, _, _, H, W = images.shape
+    psize = pradius * 2 + 1
+    dev = coarse_pred.device
+    fused = (USE_LIBRARY_KERNELS and DEFER_UPSAMPLE and isinstance(fine_fnet, ShallowEncoder) and images.is_cuda
+             and isinstance(fine_tracker, BaseTrackerPredictor) and not torch.is_grad_enabled() and images.shape[2] == 3
+             and psize == 31 and fine_fnet._fused_ok(images, psize, psize))
+    if not fused:
+        refined = coarse_pred.new_zeros(coarse_pred.shape)
+        score = coarse_pred.new_zeros((B, S, N)) if compute_score else None
+        for b, n in enumerate(counts):
+            r, sc = refine_track(images[b:b + 1], fine_fnet, fine_tracker, coarse_pred[b:b + 1, :, :n], pradius, sradius,
+                                 compute_score)
+            refined[b, :, :n] = r[0]
+            if compute_score:
+                score[b, :, :n] = sc[0]
+        return refined, score
+
+    # The packed count is rounded up to one of four buckets per octave, so that the fine transformer's captured graphs
+    # (keyed by shape) serve a dataset's changing counts; the padding tracks read sequence 0 at corner 0 and are dropped.
+    P = sum(counts)
+    quantum = 1 << max(P.bit_length() - 3, 0)
+    P_cap = (P + quantum - 1) // quantum * quantum
+    seq_host = [b for b, n in enumerate(counts) for _ in range(n)]
+    seq_real = torch.tensor(seq_host, device=dev)                          # (P,) sequence of each packed track
+    loc = torch.tensor([j for n in counts for j in range(n)], device=dev)  # (P,) its index inside the sequence
+    first = torch.tensor([sum(counts[:b]) for b in range(B)], device=dev)  # (B,) packed index of each first track
+    seq = torch.cat([seq_real, seq_real.new_zeros(P_cap - P)])
+    coarse = torch.cat([coarse_pred[seq_real, :, loc], coarse_pred.new_zeros((P_cap - P, S, 2))])   # (P_cap, S, 2)
+    query_points = coarse[:, 0]
+    track_int = coarse.floor().int()
+    track_frac = coarse - track_int
+    topleft_raw = track_int - pradius
+    topleft = torch.stack([topleft_raw[..., 0].clamp(0, W - psize), topleft_raw[..., 1].clamp(0, H - psize)], dim=-1)
+
+    half, size = fine_fnet.encode_packed_patches_of(images, topleft, seq, defer_upsample=True)
+    Hs, Ws = half.shape[-2:]
+    C_out = half.shape[1]
+    half = half.contiguous(memory_format=torch.channels_last)
+    patch_feat = None
+    if size == (2 * Hs - 1, 2 * Ws - 1) and size == (psize, psize):
+        src = half.permute(0, 2, 3, 1).reshape(P_cap, S, Hs, Ws, C_out).permute(0, 1, 4, 2, 3)
+        up = Upsampled2x(src)
+        if up2_supported(up, fine_tracker.corr_levels, fine_tracker.corr_radius, "zeros") and not fine_tracker.efficient_corr:
+            patch_feat = up
+    if patch_feat is None:
+        patch_feat = _resize(half, size).reshape(P_cap, S, C_out, psize, psize)
+
+    patch_query_points = (track_frac[:, 0] + pradius).reshape(P_cap, 2).unsqueeze(1)
+    fine_lists, _, _, query_point_feat, _ = fine_tracker(
+        query_points=patch_query_points, fmaps=patch_feat, iters=6, return_feat=True, TRACKorPOSE=False)
+    fine_pred_track = fine_lists[-1][:P].clone()                           # (P, S, 1, 2), relative to the patch corner
+    refined_p = fine_lists[-1][:P].squeeze(-2) + topleft_raw[:P]           # (P, S, 2)
+    refined_p[:, 0] = query_points[:P]
+    refined = coarse_pred.new_zeros(coarse_pred.shape)
+    refined[seq_real, :, loc] = refined_p
+
+    score = None
+    if compute_score:
+        score = _score_ragged(query_point_feat[:P].reshape(P, C_out), patch_feat, fine_pred_track, sradius, psize, counts,
+                              first, B, N, S, C_out)
+    return refined, score
+
+
+def _score_ragged(query_point_feat, patch_feat, fine_pred_track, sradius, psize, counts, first, B, N, S, C_out):
+    """``compute_score_fn`` of every sequence of a packed batch at once, each as the single-sequence call computes it:
+    its windows cut from the frame-0 map of its first track, at the corners of its own k-th track in (n, s) order re-read
+    as (s, n).  -> (B, S, N), zeros for padded tracks."""
+    dev = fine_pred_track.device
+    ssize = sradius * 2 + 1
+    cnt = torch.tensor(counts, device=dev)
+    corner = (fine_pred_track.floor().int() - sradius).clamp(0, psize - ssize).squeeze(2)   # (P, S, 2) = (x, y)
+    bb = torch.arange(B, device=dev)[:, None, None].expand(B, S - 1, N)
+    sp = torch.arange(1, S, device=dev)[None, :, None].expand(B, S - 1, N)
+    nn_ = torch.arange(N, device=dev)[None, None, :].expand(B, S - 1, N)
+    nb = cnt[bb]
+    real = nn_ < nb
+    k = sp * nb + nn_                                   # position (s, n) of sequence b reads window k of its (n, s) list
+    src_track = torch.where(real, first[bb] + k // S, first[bb])
+    src_frame = torch.where(real, k % S, torch.zeros_like(k))
+    b_r, src_track, src_frame = bb[real], src_track[real], src_frame[real]
+    q = query_point_feat[first[b_r] + nn_[real]]       # (M, C)
+    cx = corner[src_track, src_frame, 0].long()
+    cy = corner[src_track, src_frame, 1].long()
+    ar = torch.arange(ssize, device=dev)
+    rows = (cy[:, None] + ar)[:, :, None]
+    cols = (cx[:, None] + ar)[:, None, :]
+    if isinstance(patch_feat, Upsampled2x):
+        small = patch_feat.materialize(first * S)                                         # (B, C, p, p)
+    else:
+        small = patch_feat[first, 0]
+    win = small[b_r[:, None, None], :, rows, cols]                                        # (M, ss, ss, C)
+    win = win.permute(0, 3, 1, 2).reshape(-1, C_out, ssize * ssize)
+    sim = torch.einsum("mc,mcr->mr", q, win)
+    heat = torch.softmax(sim * (1.0 / C_out ** 0.5), dim=1)
+    lin = torch.linspace(-1.0, 1.0, ssize, device=heat.device, dtype=heat.dtype)
+    grid = torch.stack([lin.repeat(ssize), lin.repeat_interleave(ssize)], -1)
+    mean = heat @ grid
+    var = heat @ (grid ** 2) - mean ** 2
+    std = torch.sqrt(torch.clamp(var, min=1e-10)).sum(-1)
+    score = std.new_zeros((B, S, N))
+    score[:, 1:][real] = std
+    score[:, 0] = (torch.arange(N, device=dev)[None, :] < cnt[:, None]).to(score.dtype)
+    return score
 
 
 def inverted_score(track_score: torch.Tensor, eps: float = 1e-6) -> torch.Tensor:

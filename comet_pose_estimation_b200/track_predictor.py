@@ -22,6 +22,7 @@ import torch.nn.functional as F
 
 from .base_track_predictor import BaseTrackerPredictor
 from .refine_track import ShallowEncoder, _inorm, _ResidualBlock, _resize, inverted_score, refine_track
+from .utils import check_num_tracks
 
 
 class BasicEncoder(nn.Module):
@@ -90,6 +91,11 @@ class TrackerPredictor(nn.Module):
         B, S, C, H, W = images.shape
         if not training:
             assert B == 1, "now we only support processing one scene during inference"
+        return self._encode_frames(images)
+
+    def _encode_frames(self, images):
+        """(B,S,3,H,W) -> (B,S,128,h,w): one encoder call over all B*S frames."""
+        B, S, C, H, W = images.shape
         x = images.reshape(B * S, C, H, W)
         if self.coarse_down_ratio > 1:
             # F.interpolate(scale_factor=1/down_ratio, bilinear, align_corners=True): output size floor(H / down_ratio)
@@ -121,3 +127,58 @@ class TrackerPredictor(nn.Module):
             out["refine_pred_track"] = coarse
             out["pred_score"] = torch.ones_like(vis)
         return out
+
+    @torch.no_grad()
+    def track_batch(self, images, query_points, num_tracks=None, coarse_iters=4, fine_tracking=True):
+        """``track`` for B sequences in one call: images (B,S,3,H,W) (same S and image size for all), ``query_points``
+        a list of B tensors (N_b, 2) or a padded (B, N_max, 2) tensor with ``num_tracks`` (B,) (None: every sequence
+        has N_max tracks).  Returns ``track``'s dict with padded tensors (entries of tracks n >= N_b are 0) plus
+        ``num_tracks`` (B,) int64; ``split_batch`` cuts it into per-sequence dicts.  Sequence b gets what ``track``
+        returns for it alone (up to the rounding of the iterated loop)."""
+        B = images.shape[0]
+        if isinstance(query_points, (list, tuple)):
+            assert len(query_points) == B, f"{len(query_points)} query tensors for {B} sequences"
+            lens = [int(q.shape[0]) for q in query_points]
+            assert num_tracks is None or check_num_tracks(num_tracks, B, max(lens)) == lens, \
+                "num_tracks disagrees with the query lists"
+            padded = query_points[0].new_zeros((B, max(lens), 2))
+            for b, q in enumerate(query_points):
+                padded[b, :q.shape[0]] = q
+            query_points = padded
+            num_tracks = lens
+        assert query_points.dim() == 3 and query_points.shape[0] == B and query_points.shape[2] == 2
+        N = query_points.shape[1]
+        counts = check_num_tracks([N] * B if num_tracks is None else num_tracks, B, N)
+        fmaps = self._encode_frames(images)
+        coarse_list, vis, track_feats, query_feat, conf = self.coarse_predictor(
+            query_points=query_points, fmaps=fmaps, iters=coarse_iters, down_ratio=self.coarse_down_ratio, is_train=False,
+            return_feat=True, TRACKorPOSE=False, num_tracks=counts)
+        coarse = coarse_list[-1]
+        out = {"coarse_pred_track_list": coarse_list, "coarse_pred_track": coarse, "vis": vis, "conf": conf}
+        if fine_tracking:
+            refined, score = refine_track(images, self.fine_fnet, self.fine_predictor, coarse, compute_score=True,
+                                          num_tracks=counts)
+            real = (torch.arange(N, device=coarse.device)[None, :] < torch.tensor(counts, device=coarse.device)[:, None])
+            out["refine_pred_track"] = refined
+            out["track_score"] = score
+            out["pred_score"] = inverted_score(score) * real[:, None, :]
+        else:
+            out["refine_pred_track"] = coarse
+            real = (torch.arange(N, device=coarse.device)[None, :] < torch.tensor(counts, device=coarse.device)[:, None])
+            out["pred_score"] = torch.ones_like(vis) * real[:, None, :]
+        out["num_tracks"] = torch.tensor(counts, dtype=torch.int64)
+        return out
+
+
+def split_batch(out):
+    """``track_batch``'s padded dict -> list of per-sequence dicts with exactly ``track``'s keys and shapes."""
+    counts = [int(n) for n in out["num_tracks"]]
+
+    def cut(v, b, n):
+        if v is None:
+            return None
+        if isinstance(v, list):
+            return [cut(x, b, n) for x in v]
+        return v[b:b + 1, :, :n]
+
+    return [{k: cut(v, b, n) for k, v in out.items() if k != "num_tracks"} for b, n in enumerate(counts)]

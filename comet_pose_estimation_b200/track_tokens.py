@@ -83,7 +83,9 @@ class TrackTokenizer:
 
     def __init__(self, corr: Union[CorrBlock, EfficientCorrBlock, torch.Tensor], coords0: torch.Tensor,
                  tdim: int, num_levels: Optional[int] = None, radius: Optional[int] = None,
-                 padding_mode: Optional[str] = None):
+                 padding_mode: Optional[str] = None, num_tracks=None):
+        """``num_tracks`` (B ints or a 1-D tensor): the queries form a padded batch; queries n >= num_tracks[b] are
+        padding, their token rows are zeros and cost no correlation work."""
         if isinstance(corr, (torch.Tensor, Upsampled2x)):
             assert num_levels is not None and radius is not None
             self.radius = radius
@@ -97,6 +99,12 @@ class TrackTokenizer:
         self.tdim = tdim
         p = self._pyr
         self.pos = sampled_pos_emb(coords0, tdim, p.H, p.W)
+        self.num_tracks = None
+        if num_tracks is not None:
+            from .utils import check_num_tracks
+
+            counts = check_num_tracks(num_tracks, coords0.shape[0], coords0.shape[1])
+            self.num_tracks = torch.tensor(counts, dtype=torch.int32).to(coords0.device)
 
     def tokens(self, coords: torch.Tensor, track_feats: torch.Tensor, out: Optional[torch.Tensor] = None):
         """coords (B,S,N,2), track_feats (B,S,N,latent) (any outer strides) -> (B,N,S,D_tok) float32."""
@@ -115,19 +123,23 @@ class TrackTokenizer:
         else:
             assert out.shape == (B, N, S, self.tdim) and out.is_contiguous() and out.dtype == torch.float32
         with torch.cuda.device(c.device):
+            nt = self.num_tracks
             if B * S * N and _use_tc(p, t, self.radius, self.padding_mode):
-                _lib.check(lib.comet_tc_track_tokens_f32(
-                    p.split.data_ptr(), t.data_ptr(), t.stride(0), t.stride(1), t.stride(2),
-                    c.data_ptr(), c.stride(0), c.stride(1), c.stride(2),
-                    self.pos.data_ptr(), out.data_ptr(),
-                    B, S, N, p.C, p.H, p.W, p.num_levels, self.radius, pad_mode(self.padding_mode), prec_mode(),
-                    self.tdim, _tc_workspace(p, N).data_ptr(), stream_ptr(c.device)))
+                head = (p.split.data_ptr(), t.data_ptr(), t.stride(0), t.stride(1), t.stride(2),
+                        c.data_ptr(), c.stride(0), c.stride(1), c.stride(2), self.pos.data_ptr(), out.data_ptr())
+                tail = (B, S, N, p.C, p.H, p.W, p.num_levels, self.radius, pad_mode(self.padding_mode), prec_mode(),
+                        self.tdim, _tc_workspace(p, N).data_ptr(), stream_ptr(c.device))
+                if nt is None:
+                    _lib.check(lib.comet_tc_track_tokens_f32(*head, *tail))
+                else:
+                    _lib.check(lib.comet_tc_track_tokens_ragged_f32(*head, nt.data_ptr(), *tail))
                 return out
-            _lib.check(lib.comet_track_tokens_f32(
-                p.fmaps0.data_ptr(), p.pyr.data_ptr(),
-                t.data_ptr(), t.stride(0), t.stride(1), t.stride(2),
-                c.data_ptr(), c.stride(0), c.stride(1), c.stride(2),
-                self.pos.data_ptr(), out.data_ptr(),
-                B, S, N, p.C, p.H, p.W, p.num_levels, self.radius, pad_mode(self.padding_mode), prec_mode(),
-                p.layout, self.tdim, stream_ptr(c.device)))
+            head = (p.fmaps0.data_ptr(), p.pyr.data_ptr(), t.data_ptr(), t.stride(0), t.stride(1), t.stride(2),
+                    c.data_ptr(), c.stride(0), c.stride(1), c.stride(2), self.pos.data_ptr(), out.data_ptr())
+            tail = (B, S, N, p.C, p.H, p.W, p.num_levels, self.radius, pad_mode(self.padding_mode), prec_mode(),
+                    p.layout, self.tdim, stream_ptr(c.device))
+            if nt is None:
+                _lib.check(lib.comet_track_tokens_f32(*head, *tail))
+            else:
+                _lib.check(lib.comet_track_tokens_ragged_f32(*head, nt.data_ptr(), *tail))
         return out

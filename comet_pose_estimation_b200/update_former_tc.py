@@ -137,6 +137,21 @@ class _Run:
                                                   self.stream))
         return op
 
+    def attention_varlen(self, q, k, v, H: int, dh: int, step: int, items, q_off, q_len, k_off, k_len, lq, lk, group: int,
+                         rows_out: int, D: int, zero: bool = False):
+        """Every item of ``items`` in one call: item i's position j is row ``q_off[i] + j * step`` of q / of the output
+        and row ``k_off[i] + j * step`` of k / v (int32 device arrays); ``lq`` / ``lk`` bound the lengths.  ``zero``: the
+        output rows no item writes (padded queries) are zeros instead of unset."""
+        op = self.new_planes(rows_out, D)
+        if zero:
+            op.zero_()
+        assert k.stride(0) == v.stride(0)
+        _lib.check(lib.comet_attention_varlen_planes_f32(
+            q.data_ptr(), q.stride(0), step, k.data_ptr(), k.stride(0), step, v.data_ptr(), op.data_ptr(), op.stride(0),
+            op.stride(1), self.np, items, H, dh, q_off.data_ptr(), q_len.data_ptr(), k_off.data_ptr(), k_len.data_ptr(),
+            lq[0], lq[1], lk[0], lk[1], group, self.stream))
+        return op
+
     def mlp_tail(self, y: torch.Tensor, blk, out: torch.Tensor):
         """out = y + fc2(GELU(fc1(norm2(y))))   (modules.py:119-154; norm2 without affine)."""
         _, ynp = self.layernorm(y, blk.norm2, want_f32=False)
@@ -173,6 +188,31 @@ class _Run:
         self.mlp_tail(y, blk, out=x)
 
 
+    def self_block_varlen(self, x: torch.Tensor, blk, H: int, step: int, lay, group: int):
+        """``self_block`` on the virtual-track rows of every sequence at once (one attention problem per (sequence, frame))."""
+        rows, D = x.shape
+        xn, xnp = self.layernorm(x, blk.norm1, want_f32=True)
+        qkv, _ = self.linear(xnp, blk.attn.in_proj_weight, blk.attn.in_proj_bias)
+        ctx = self.attention_varlen(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], H, D // H, step, lay.items, lay.vir_off,
+                                    lay.vir_len, lay.vir_off, lay.vir_len, (lay.V, lay.V), (lay.V, lay.V), group, rows, D)
+        y, _ = self.linear(ctx, blk.attn.out_proj.weight, blk.attn.out_proj.bias, resid=xn)
+        self.mlp_tail(y, blk, out=x)
+
+    def cross_block_varlen(self, x: torch.Tensor, ctxt: torch.Tensor, blk, H: int, step: int, items: int, q_off, q_len, k_off,
+                           k_len, lq, lk, group: int):
+        """``cross_block`` of every sequence at once: item i attends from its rows of ``x`` to its rows of ``ctxt``."""
+        rows, D = x.shape
+        xn, xnp = self.layernorm(x, blk.norm1, want_f32=True)
+        _, cnp = self.layernorm(ctxt, blk.norm_context, want_f32=False)
+        a = blk.cross_attn
+        q, _ = self.linear(xnp, a.in_proj_weight, a.in_proj_bias, 0, D)
+        kv, _ = self.linear(cnp, a.in_proj_weight, a.in_proj_bias, D, 3 * D)
+        ctx = self.attention_varlen(q, kv[:, :D], kv[:, D:], H, D // H, step, items, q_off, q_len, k_off, k_len, lq, lk,
+                                    group, rows, D, zero=lq[0] != lq[1])
+        y, _ = self.linear(ctx, a.out_proj.weight, a.out_proj.bias, resid=xn)
+        self.mlp_tail(y, blk, out=x)
+
+
 # One forward is ~180 kernel launches (coarse tracker) whose device time is a few milliseconds at most: issued one by one
 # from Python the host is the bottleneck, so the launch sequence of a (shape, precision) is captured once into a CUDA
 # graph and replayed (workspaces live in the graph's private pool).  False = eager launches (A/B timing, debugging).
@@ -181,22 +221,36 @@ _MAX_GRAPHS = 4
 
 
 class _Captured:
-    def __init__(self, m, x: torch.Tensor, np_: int):
+    """``counts`` given: the ragged forward, captured for the capacity of ``x`` (B, N_cap, T, Din); the track counts are
+    read from a device buffer, so one graph serves every set of counts up to N_cap."""
+
+    def __init__(self, m, x: torch.Tensor, np_: int, counts: torch.Tensor = None):
         self.x = torch.empty_like(x)
         self.x.copy_(x)
+        self.counts = None if counts is None else counts.clone()
+        run = (lambda: forward_eager(m, self.x, np_)) if counts is None else (
+            lambda: forward_ragged_eager(m, self.x, np_, self.counts))
         side = torch.cuda.Stream(device=x.device)
         side.wait_stream(torch.cuda.current_stream(x.device))
         with torch.cuda.stream(side):                      # warm-up: weight planes, kernel attributes, allocator
-            forward_eager(m, self.x, np_)
+            run()
         torch.cuda.current_stream(x.device).wait_stream(side)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
-            self.out = forward_eager(m, self.x, np_)
+            self.out = run()
 
-    def __call__(self, x: torch.Tensor) -> torch.Tensor:
-        self.x.copy_(x, non_blocking=True)
+    def __call__(self, x: torch.Tensor, counts: torch.Tensor = None) -> torch.Tensor:
+        if counts is None:
+            self.x.copy_(x, non_blocking=True)
+        else:
+            n = x.shape[1]
+            self.x[:, :n].copy_(x, non_blocking=True)
+            self.x[:, n:].zero_()
+            self.counts.copy_(counts, non_blocking=True)
         self.graph.replay()
-        return self.out.clone()
+        if counts is None:
+            return self.out.clone()
+        return self.out[:, :x.shape[1]].clone()
 
 
 def _weights_tag(m) -> tuple:
@@ -217,7 +271,98 @@ def forward(m, x: torch.Tensor, np_: int) -> torch.Tensor:
             m._tc_graphs.pop(next(iter(m._tc_graphs)))
         with torch.cuda.device(x.device):
             g = m._tc_graphs[key] = _Captured(m, x.contiguous(), np_)
+        m._tc_captures = getattr(m, "_tc_captures", 0) + 1
     return g(x)
+
+
+# Track capacity of a ragged graph: N_max rounded up to this, so that a dataset's changing counts reuse a few graphs.
+RAGGED_TRACK_QUANTUM = 64
+
+
+def ragged_supported(m) -> bool:
+    """The varlen space attention serves problems with more than 32 queries or keys: true for >= 33 virtual tracks."""
+    return not m.add_space_attn or m.num_virtual_tracks > 32
+
+
+def forward_ragged(m, x: torch.Tensor, np_: int, counts: torch.Tensor) -> torch.Tensor:
+    """``EfficientUpdateFormer.forward`` of B sequences at once: tokens ``x`` (B, N_max, T, input_dim), ``counts`` (B,)
+    int32 on the device (1 <= counts[b] <= N_max).  Sequence b's rows n < counts[b] get what the forward of that
+    sequence alone gives; its rows n >= counts[b] are zeros."""
+    B, N, T, Din = x.shape
+    ncap = (N + RAGGED_TRACK_QUANTUM - 1) // RAGGED_TRACK_QUANTUM * RAGGED_TRACK_QUANTUM
+    if not USE_CUDA_GRAPH or torch.cuda.is_current_stream_capturing():
+        xp = x.new_zeros((B, ncap, T, Din))
+        xp[:, :N] = x
+        return forward_ragged_eager(m, xp, np_, counts)[:, :N]
+    if not hasattr(m, "_tc_graphs"):
+        m._tc_graphs = {}
+    key = ("ragged", B, ncap, T, Din, np_, str(x.device), _weights_tag(m))
+    g = m._tc_graphs.get(key)
+    if g is None:
+        while len(m._tc_graphs) >= _MAX_GRAPHS:
+            m._tc_graphs.pop(next(iter(m._tc_graphs)))
+        xp = x.new_zeros((B, ncap, T, Din))
+        xp[:, :N] = x
+        with torch.cuda.device(x.device):
+            g = m._tc_graphs[key] = _Captured(m, xp, np_, counts)
+        m._tc_captures = getattr(m, "_tc_captures", 0) + 1
+    return g(x, counts)
+
+
+class _RaggedLayout:
+    """Device index arrays of the space attention over B sequences: item i = (sequence b, frame t) = b * T + t.  Point
+    rows are (b, n, t) -> (b * N_cap + n) * T + t, virtual rows (b, v, t) -> (b * V + v) * T + t of their own block."""
+
+    def __init__(self, counts: torch.Tensor, B: int, ncap: int, V: int, T: int):
+        dev = counts.device
+        b = torch.arange(B, device=dev, dtype=torch.int32).repeat_interleave(T)
+        t = torch.arange(T, device=dev, dtype=torch.int32).repeat(B)
+        self.items, self.V, self.ncap = B * T, V, ncap
+        self.pts_off = (b * (ncap * T) + t).contiguous()
+        self.vir_off = (b * (V * T) + t).contiguous()
+        self.pts_len = counts.to(torch.int32).repeat_interleave(T).contiguous()
+        self.vir_len = torch.full((B * T,), V, dtype=torch.int32, device=dev)
+
+
+def forward_ragged_eager(m, x: torch.Tensor, np_: int, counts: torch.Tensor) -> torch.Tensor:
+    """Ragged forward for x (B, N_cap, T, input_dim).  Tokens are laid out as all sequences' point rows followed by all
+    sequences' virtual rows, so every LayerNorm and GEMM of a block is one launch over all sequences and the space
+    attention is one varlen launch per kernel family.  Padded point rows are never keys or queries of the space
+    attention; they only pass through row-wise work (and the time attention, per track) and stay finite."""
+    B, Nc, T, Din = x.shape
+    D, H, V = m.hidden_size, m.num_heads, (m.num_virtual_tracks if m.add_space_attn else 0)
+    if not hasattr(m, "_tc_weights"):
+        m._tc_weights = _Weights()
+    with torch.cuda.device(x.device):
+        run = _Run(m._tc_weights, np_, x.device)
+        x = x.contiguous()
+        P = B * Nc * T
+        xp = run.split(x.view(P, Din))
+        skip, _ = run.linear(xp, m.input_transform.weight, m.input_transform.bias)          # (B*Nc*T, D)
+        flat = torch.empty((P + B * V * T, D), dtype=torch.float32, device=x.device)
+        flat[:P] = skip
+        pts, vir = flat[:P], flat[P:]
+        if V:
+            vir.view(B, V, T, D)[:] = m.virual_tracks                                        # (1, V, 1, D) broadcast
+            lay = _RaggedLayout(counts, B, Nc, V, T)
+        every = len(m.time_blocks) // len(m.space_virtual_blocks) if V else 0
+        j = 0
+        for i, tb in enumerate(m.time_blocks):
+            run.self_block(flat, tb, B * (Nc + V), T, T, 1, H)                               # time attention per track
+            if V and i % every == 0:
+                run.cross_block_varlen(vir, pts, m.space_virtual2point_blocks[j], H, T, lay.items, lay.vir_off, lay.vir_len,
+                                       lay.pts_off, lay.pts_len, (V, V), (1, Nc), T)
+                run.self_block_varlen(vir, m.space_virtual_blocks[j], H, T, lay, T)
+                run.cross_block_varlen(pts, vir, m.space_point2virtual_blocks[j], H, T, lay.items, lay.pts_off, lay.pts_len,
+                                       lay.vir_off, lay.vir_len, (1, Nc), (V, V), T)
+                j += 1
+        sp = run.new_planes(P, D)
+        _lib.check(lib.comet_add_planes_f32(pts.data_ptr(), skip.data_ptr(), sp.data_ptr(), sp.stride(0), np_, P * D,
+                                            run.stream))
+        out, _ = run.linear(sp, m.flow_head.weight, m.flow_head.bias)
+        out = out.view(B, Nc, T, -1)
+        real = torch.arange(Nc, device=x.device)[None, :] < counts[:, None]
+        return out.masked_fill_(~real[:, :, None, None], 0.0)
 
 
 def forward_eager(m, x: torch.Tensor, np_: int) -> torch.Tensor:

@@ -203,3 +203,16 @@ def instance_norm(x: torch.Tensor, relu: bool = False, eps: float = 1e-5) -> tor
                                                _lib.FMAPS_CHANNEL_LAST if cl else _lib.FMAPS_NCHW, int(relu), float(eps),
                                                stream_ptr(x.device)))
     return out if in_dtype == torch.float32 else out.to(in_dtype)
+
+
+def check_num_tracks(num_tracks, B: int, N_max: int) -> list:
+    """Per-sequence track counts of a padded batch (a sequence of ints or a 1-D tensor) -> list of B Python ints, each in
+    [1, N_max].  Anything else raises AssertionError."""
+    if isinstance(num_tracks, torch.Tensor):
+        assert num_tracks.dim() == 1, f"num_tracks must be 1-D, got shape {tuple(num_tracks.shape)}"
+        vals = [int(v) for v in num_tracks.tolist()]
+    else:
+        vals = [int(v) for v in num_tracks]
+    assert len(vals) == B, f"num_tracks has {len(vals)} entries for a batch of {B} sequences"
+    assert all(1 <= v <= N_max for v in vals), f"num_tracks {vals} outside [1, {N_max}]"
+    return vals

@@ -147,6 +147,15 @@ int comet_track_tokens_f32(const float* fmaps, const float* pyr, const float* tr
                            long long c_sn, const float* pos_emb, float* tokens, int B, int S, int N, int C, int H,
                            int W, int L, int r, int pad_mode, int prec_mode, int pyr_layout, int D_tok,
                            comet_stream_t stream);
+/* The same for a batch of sequences with different track counts: num_tracks (B,) int32 in DEVICE memory, 1 <= num_tracks[b]
+ * <= N.  Queries n >= num_tracks[b] are padding: their token rows are written as zeros and nothing else is computed for
+ * them; every other row equals comet_track_tokens_f32 on sequence b alone with N = num_tracks[b].  Not served for
+ * COMET_PYR_UP2_SOURCE or C == 32 (COMET_ERR_UNSUPPORTED / COMET_ERR_INVALID). */
+int comet_track_tokens_ragged_f32(const float* fmaps, const float* pyr, const float* track_feats, long long t_sb,
+                                  long long t_ss, long long t_sn, const float* coords, long long c_sb, long long c_ss,
+                                  long long c_sn, const float* pos_emb, float* tokens, const int* num_tracks, int B, int S,
+                                  int N, int C, int H, int W, int L, int r, int pad_mode, int prec_mode, int pyr_layout,
+                                  int D_tok, comet_stream_t stream);
 
 /* sampled_pos_emb = sample_features4d(get_2d_sincos_pos_embed(D,(H,W)), coords[:,0])
  * (base_track_predictor.py:200-208; utils.py:724-755, :942-974): the float64 table is evaluated on the fly at
@@ -219,6 +228,12 @@ int comet_shallow_encoder_f32(const float* patches, long long sn, long long sc, 
                               const float* packed, float* out, long long P, float eps, comet_stream_t stream);
 int comet_shallow_encoder_from_images_f32(const float* images, const int* topleft, const float* packed, float* out,
                                           int B, int S, int N, int H, int W, float eps, comet_stream_t stream);
+/* The same for P tracks packed from several sequences of images (B,S,3,H,W): topleft (P,S,2) int32 corners, seq_of_track
+ * (P,) int32 the sequence of each track (device memory).  out (P*S, 16, 16, 32) in (track, frame) order; each map is
+ * bit-identical to comet_shallow_encoder_from_images_f32 on the same patch. */
+int comet_shallow_encoder_from_images_ragged_f32(const float* images, const int* topleft, const int* seq_of_track,
+                                                 const float* packed, float* out, int P, int B, int S, int H, int W,
+                                                 float eps, comet_stream_t stream);
 
 /* ---- sin/cos encodings: comet/models/utils.py:37-101, :724-832 ----------- */
 /* get_2d_embedding(xy, C, cat_coords): xy (M,2) contiguous -> out (M, 2*C [+2 in front if cat_coords]). */
@@ -251,6 +266,14 @@ int comet_tc_track_tokens_f32(const void* split, const float* track_feats, long 
                               long long t_sn, const float* coords, long long c_sb, long long c_ss, long long c_sn,
                               const float* pos_emb, float* tokens, int B, int S, int N, int C, int H, int W, int L,
                               int r, int pad_mode, int prec_mode, int D_tok, void* workspace, comet_stream_t stream);
+/* comet_tc_track_tokens_f32 for a batch of sequences with different track counts (num_tracks (B,) int32, device memory;
+ * see comet_track_tokens_ragged_f32).  Padded queries are left out of the sort: they occupy no tile slot, and a tile
+ * that holds none of them is an empty one-row job.  Real rows are bit-identical to the single-sequence call. */
+int comet_tc_track_tokens_ragged_f32(const void* split, const float* track_feats, long long t_sb, long long t_ss,
+                                     long long t_sn, const float* coords, long long c_sb, long long c_ss, long long c_sn,
+                                     const float* pos_emb, float* tokens, const int* num_tracks, int B, int S, int N, int C,
+                                     int H, int W, int L, int r, int pad_mode, int prec_mode, int D_tok, void* workspace,
+                                     comet_stream_t stream);
 /* vols: HOST array of L device pointers, level l = (B*S, N, H_l*W_l) float32. */
 int comet_tc_corr_volume_f32(const void* split, const float* targets, long long t_sb, long long t_ss, long long t_sn,
                              float* const* vols, int B, int S, int N, int C, int H, int W, int L, int prec_mode,
@@ -286,6 +309,17 @@ int comet_attention_planes_f32(const float* q, long long q_sb, long long q_si, c
                                const float* v, long long v_sb, long long v_si, void* out_planes, long long o_plane_stride,
                                long long o_sb, long long o_si, int np, int B, int H, int Lq, int Lk, int dh,
                                comet_stream_t stream);
+/* Many attention problems of different lengths in one call (all sequences of a space block): item i's query position j
+ * (and output row) is row q_off[i] + j*q_step of q (row pitch q_ld) / of the output planes (row pitch o_ld), its key /
+ * value position j is row k_off[i] + j*k_step of k and v (row pitch k_ld), with q_len[i] / k_len[i] positions.  The four
+ * int32 arrays live in DEVICE memory; every length must lie in [min_lq, max_lq] / [min_lk, max_lk].  Item i gets exactly
+ * the arithmetic comet_attention_planes_f32 uses for (Lq, Lk, dh, np) with B = group problems of that shape (same kernel
+ * family, same key split).  Items with at most 32 queries AND at most 32 keys are not served. */
+int comet_attention_varlen_planes_f32(const float* q, long long q_ld, long long q_step, const float* k, long long k_ld,
+                                      long long k_step, const float* v, void* out_planes, long long o_plane_stride,
+                                      long long o_ld, int np, int items, int H, int dh, const int* q_off, const int* q_len,
+                                      const int* k_off, const int* k_len, int min_lq, int max_lq, int min_lk, int max_lk,
+                                      int group, comet_stream_t stream);
 /* planes of a + b (contiguous float32 vectors of n elements): `tokens + init_tokens` before the flow head (blocks.py:344). */
 int comet_add_planes_f32(const float* a, const float* b, void* planes, long long plane_stride, int np, long long n,
                          comet_stream_t stream);
