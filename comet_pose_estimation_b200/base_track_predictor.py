@@ -47,11 +47,20 @@ class BaseTrackerPredictor(nn.Module):
             self.vis_predictor = nn.Sequential(nn.Linear(latent_dim, 1))
 
     def forward(self, query_points, fmaps=None, iters=4, return_feat=False, down_ratio=1, is_train=False,
-                track_feats=None, TRACKorPOSE=True, ind=0, num_tracks=None):
+                track_feats=None, TRACKorPOSE=True, ind=0, num_tracks=None, num_frames=None):
         """``num_tracks`` (B ints or a 1-D tensor, ``TRACKorPOSE=False`` only): ``query_points`` (B, N_max, 2) is a padded
         batch of sequences with different track counts.  Sequence b's tracks get what a call on that sequence alone
-        computes (up to rounding); every output entry of a padded track (n >= num_tracks[b]) is 0."""
-        counts = None
+        computes (up to rounding); every output entry of a padded track (n >= num_tracks[b]) is 0.  ``num_frames``
+        (likewise): sequence b has the first ``num_frames[b]`` of the S frames of ``fmaps``; every output entry of a padded
+        frame is 0, and the tracks of padded frames start at 0 and receive zero updates."""
+        counts = frames = None
+        if num_frames is not None:
+            assert not TRACKorPOSE, "num_frames is served with TRACKorPOSE=False only"
+            from .utils import check_num_tracks
+
+            frames = check_num_tracks(num_frames, fmaps.shape[0], fmaps.shape[1])
+            live = torch.arange(fmaps.shape[1], device=query_points.device)[None, :] < torch.tensor(
+                frames, device=query_points.device)[:, None]                                  # (B, S)
         if num_tracks is not None:
             assert not TRACKorPOSE, "num_tracks is served with TRACKorPOSE=False only"
             from .utils import check_num_tracks
@@ -73,6 +82,8 @@ class BaseTrackerPredictor(nn.Module):
             coords = query_points.clone()
         else:
             coords = query_points.clone().reshape(B, 1, N, 2).repeat(1, S, 1, 1)
+        if frames is not None:
+            coords = coords * live[:, :, None, None]
 
         if isinstance(fmaps, Upsampled2x):
             # bilinear sample (border) of the 2x-1 up-sampling at p == bilinear sample of its source at p / 2
@@ -87,17 +98,19 @@ class BaseTrackerPredictor(nn.Module):
         else:
             fcorr_fn = CorrBlock(fmaps, num_levels=self.corr_levels, radius=self.corr_radius)
         # sampled_pos_emb depends on coords[:, 0] only, which the loop pins -> computed once, not per iteration
-        tokenizer = TrackTokenizer(fcorr_fn, coords[:, 0], self.transformer_dim, num_tracks=counts)
+        tokenizer = TrackTokenizer(fcorr_fn, coords[:, 0], self.transformer_dim, num_tracks=counts, num_frames=frames)
 
         coord_preds = []
         for _ in range(iters):
             coords = coords.detach()
             x = tokenizer.tokens(coords, track_feats)  # (B, N, S, transformer_dim), one fused kernel
 
-            if counts is None:
+            if counts is None and frames is None:
                 delta = self.updateformer(x).reshape(B * N, S, self.latent_dim + 2)
-            else:
+            elif frames is None:
                 delta = self.updateformer(x, num_tracks=counts).reshape(B * N, S, self.latent_dim + 2)   # 0 when padded
+            else:
+                delta = self.updateformer(x, num_tracks=counts, num_frames=frames).reshape(B * N, S, self.latent_dim + 2)
             delta_coords_ = delta[:, :, :2]
             delta_feats_ = delta[:, :, 2:].reshape(B * N * S, self.latent_dim)
 
@@ -119,8 +132,10 @@ class BaseTrackerPredictor(nn.Module):
         conf_e = None
         if self.cfg.track_conf:
             conf_e = torch.sigmoid(self.conf_predictor(track_feats.reshape(B * S * N, self.latent_dim)).reshape(B, S, N))
-        if counts is not None:
-            pad_s = ~real[:, None, :]                                                         # (B, 1, N)
+        if counts is not None or frames is not None:
+            if counts is None:
+                real = torch.ones((B, N), dtype=torch.bool, device=coords.device)
+            pad_s = ~real[:, None, :] if frames is None else ~(real[:, None, :] & live[:, :, None])  # (B, 1 or S, N)
             coord_preds = [c.masked_fill(pad_s[..., None], 0.0) for c in coord_preds]
             vis_e = None if vis_e is None else vis_e.masked_fill(pad_s, 0.0)
             conf_e = None if conf_e is None else conf_e.masked_fill(pad_s, 0.0)

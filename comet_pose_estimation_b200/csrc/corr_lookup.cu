@@ -44,7 +44,7 @@ __global__ void __launch_bounds__(256) corr_lookup_kernel(const LookupParams p) 
   const int s = (int)((q / p.N) % p.S);
   const int b = (int)(q / ((long long)p.N * p.S));
   const long long bs = (long long)b * p.S + s;
-  if (TOKENS && p.ntr && n >= __ldg(p.ntr + b)) {   // padded query: zero row
+  if (TOKENS && ((p.ntr && n >= __ldg(p.ntr + b)) || (p.nfr && s >= __ldg(p.nfr + b)))) {   // padded query / frame: zero row
     float* zp = p.out + (((long long)b * p.N + n) * p.S + s) * p.D_tok;
     for (int d = lane; d < p.D_tok; d += 32) zp[d] = 0.f;
     return;
@@ -598,7 +598,9 @@ static int launch_lookup(const LookupParams& p, cudaStream_t stream) {
   if (blocks > 0x7fffffffLL) return fail(COMET_ERR_UNSUPPORTED, "too many queries for one launch");
   if (p.C == 32 && p.r >= 1 && p.r <= 3 && p.t_level_stride == 0 && ((uintptr_t)p.pyr % 16) == 0 &&
       (!p.cl0 || ((uintptr_t)p.fmaps % 16) == 0)) {
-    if (p.ntr) return fail(COMET_ERR_UNSUPPORTED, "per-sequence query counts are served by the generic lookup kernel (C != 32)");
+    if (p.ntr || p.nfr)
+      return fail(COMET_ERR_UNSUPPORTED, "per-sequence query / frame counts are served by the generic lookup kernel (C != 32) "
+                                         "and, frame counts, by COMET_PYR_UP2_SOURCE");
     const bool use_tma = option(COMET_OPT_TMA_LOOKUP) && device_sm_count_if_sm100() > 0 && tensor_map_encoder() != nullptr;
     if (use_tma && p.cl0 && p.L <= 3 && total < (1LL << 40)) {
       TmaMaps maps;
@@ -702,8 +704,9 @@ extern "C" int comet_corr_lookup_f32(const float* fmaps, const float* pyr, const
 
 static int track_tokens(const float* fmaps, const float* pyr, const float* track_feats, long long t_sb, long long t_ss,
                         long long t_sn, const float* coords, long long c_sb, long long c_ss, long long c_sn,
-                        const float* pos_emb, float* tokens, const int* num_tracks, int B, int S, int N, int C, int H, int W,
-                        int L, int r, int pad_mode, int prec_mode, int pyr_layout, int D_tok, comet_stream_t stream) {
+                        const float* pos_emb, float* tokens, const int* num_tracks, const int* num_frames, int B, int S, int N,
+                        int C, int H, int W, int L, int r, int pad_mode, int prec_mode, int pyr_layout, int D_tok,
+                        comet_stream_t stream) {
   LookupParams p{};
   int rc = fill_params(p, fmaps, pyr, track_feats, t_sb, t_ss, t_sn, 0, coords, c_sb, c_ss, c_sn, B, S, N, C, H, W,
                        L, r, pad_mode, prec_mode, pyr_layout);
@@ -712,7 +715,7 @@ static int track_tokens(const float* fmaps, const float* pyr, const float* track
   COMET_REQUIRE(C % 4 == 0, "latent_dim must be a multiple of 4 for the flow embedding (got %d)", C);
   COMET_REQUIRE(D_tok >= need, "D_tok=%d smaller than the %d token channels", D_tok, need);
   COMET_REQUIRE((long long)B * S * N == 0 || (tokens && pos_emb), "null tokens / pos_emb pointer");
-  p.out = tokens; p.pos = pos_emb; p.D_tok = D_tok; p.ntr = num_tracks;
+  p.out = tokens; p.pos = pos_emb; p.D_tok = D_tok; p.ntr = num_tracks; p.nfr = num_frames;
   if (pyr_layout == COMET_PYR_UP2_SOURCE) {
     COMET_REQUIRE(!num_tracks, "per-sequence query counts are not served by COMET_PYR_UP2_SOURCE");
     rc = up2_supported(C, H, W, L, r, pad_mode);
@@ -727,8 +730,8 @@ extern "C" int comet_track_tokens_f32(const float* fmaps, const float* pyr, cons
                                       long long c_ss, long long c_sn, const float* pos_emb, float* tokens, int B,
                                       int S, int N, int C, int H, int W, int L, int r, int pad_mode, int prec_mode,
                                       int pyr_layout, int D_tok, comet_stream_t stream) {
-  return track_tokens(fmaps, pyr, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, nullptr, B, S,
-                      N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok, stream);
+  return track_tokens(fmaps, pyr, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, nullptr, nullptr, B,
+                      S, N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok, stream);
 }
 
 extern "C" int comet_track_tokens_ragged_f32(const float* fmaps, const float* pyr, const float* track_feats, long long t_sb,
@@ -737,6 +740,16 @@ extern "C" int comet_track_tokens_ragged_f32(const float* fmaps, const float* py
                                              const int* num_tracks, int B, int S, int N, int C, int H, int W, int L, int r,
                                              int pad_mode, int prec_mode, int pyr_layout, int D_tok, comet_stream_t stream) {
   COMET_REQUIRE((long long)B * S * N == 0 || num_tracks, "null num_tracks");
-  return track_tokens(fmaps, pyr, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks, B,
-                      S, N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok, stream);
+  return track_tokens(fmaps, pyr, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks, nullptr,
+                      B, S, N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok, stream);
+}
+
+extern "C" int comet_track_tokens_varlen_f32(const float* fmaps, const float* pyr, const float* track_feats, long long t_sb,
+                                             long long t_ss, long long t_sn, const float* coords, long long c_sb,
+                                             long long c_ss, long long c_sn, const float* pos_emb, float* tokens,
+                                             const int* num_tracks, const int* num_frames, int B, int S, int N, int C, int H,
+                                             int W, int L, int r, int pad_mode, int prec_mode, int pyr_layout, int D_tok,
+                                             comet_stream_t stream) {
+  return track_tokens(fmaps, pyr, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks,
+                      num_frames, B, S, N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok, stream);
 }

@@ -96,6 +96,12 @@ __global__ void __launch_bounds__(UP2_WARPS * 32, 1) corr_lookup_c32_up2_kernel(
     const int s = (int)((q / p.N) % p.S);
     const int b = (int)(q / ((long long)p.N * p.S));
     const int bs = b * p.S + s;
+    if (TOKENS && p.nfr && s >= __ldg(p.nfr + b)) {   // padded frame: zero row, no map is read
+      float* zp = p.out + (((long long)b * p.N + n) * p.S + s) * p.D_tok;
+      for (int d = lane; d < p.D_tok; d += 32) zp[d] = 0.f;
+      fetch(q + nwarps, cx, cy, cx0, cy0, tl);
+      continue;
+    }
     AxisWindow ax[3], ay[3];
 #pragma unroll
     for (int l = 0; l < 3; ++l) {

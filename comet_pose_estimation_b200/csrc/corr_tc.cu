@@ -138,6 +138,7 @@ struct Params {
   int vec4;                                           // tokens: rows of out / pos are 16-byte aligned (float4 token_misc path)
   int red;                                            // tokens: windows are ADDED to the rows (MODE_REDUCE); tc_pre_kernel writes pos_emb there
   const int* ntr;                                     // tokens: (B,) query count of each sequence (queries n >= ntr[b] are padding), or null
+  const int* nfr;                                     // tokens: (B,) frame count of each sequence (frames s >= nfr[b] are padding), or null
   float* vol[5]; int volume_mode;                      // volume mode: per-level (BS,N,H_l,W_l)
   int B, S, N, L, r, npass, bf16;
   int BS, mtiles, npad, nsplit, npyr, nchunk, njobs;
@@ -378,7 +379,8 @@ __device__ __forceinline__ void plan_frame(const Params& p, int* __restrict__ pe
   int* myperm = perm + (long long)bs * p.npad;
   int4* myslots = const_cast<int4*>(p.slots) + (long long)bs * p.npad;
   const bool track = p.mtiles <= PLAN_MAX_MT;  // else: sorted, but every job covers the full maps
-  const int Nb = p.ntr ? min(max(__ldg(p.ntr + b), 0), p.N) : p.N;   // padded queries are not sorted: no tile, no job work
+  int Nb = p.ntr ? min(max(__ldg(p.ntr + b), 0), p.N) : p.N;   // padded queries are not sorted: no tile, no job work
+  if (p.nfr && s >= __ldg(p.nfr + b)) Nb = 0;                   // padded frame: every tile of it is an empty job
 
   for (int i = threadIdx.x; i < PLAN_BINS; i += blockDim.x) hist[i] = 0;
   if (track)
@@ -489,7 +491,7 @@ __device__ __forceinline__ void token_misc_rows(const Params& p, long long warp_
     const int s = (int)(row % p.S);
     const long long bn = row / p.S;
     const int n = (int)(bn % p.N), b = (int)(bn / p.N);
-    if (p.ntr && n >= __ldg(p.ntr + b)) {          // padded query: zero row
+    if ((p.ntr && n >= __ldg(p.ntr + b)) || (p.nfr && s >= __ldg(p.nfr + b))) {   // padded query / frame: zero row
       for (int c = lane; c < p.D_tok; c += 32) p.out[row * p.D_tok + c] = 0.f;
       continue;
     }
@@ -596,9 +598,10 @@ __device__ __forceinline__ void token_misc_rows_v4(const Params& p, long long wa
       __syncwarp();                                 // the feature row was copied by all 32 lanes
     }
     float* o = p.out + (long long)row * p.D_tok;
-    if (p.ntr) {
+    if (p.ntr || p.nfr) {
       const int bn = row / p.S, b_ = bn / p.N;
-      if (bn - b_ * p.N >= __ldg(p.ntr + b_)) {     // padded query: zero row (its loads above were in bounds and unused)
+      if ((p.ntr && bn - b_ * p.N >= __ldg(p.ntr + b_)) || (p.nfr && row - bn * p.S >= __ldg(p.nfr + b_))) {
+        // padded query / frame: zero row (its loads above were in bounds and unused)
         for (int k = lane; k < nv; k += 32) reinterpret_cast<float4*>(o)[k] = make_float4(0.f, 0.f, 0.f, 0.f);
         if (p.red) {                                // keep the bulk-group count of the store pipeline in step
           asm volatile("cp.async.bulk.commit_group;" ::: "memory");
@@ -1641,7 +1644,8 @@ extern "C" int comet_tc_corr_lookup_f32(const void* split, const float* targets,
 
 static int tc_track_tokens(const void* split, const float* track_feats, long long t_sb, long long t_ss, long long t_sn,
                            const float* coords, long long c_sb, long long c_ss, long long c_sn, const float* pos_emb,
-                           float* tokens, const int* num_tracks, int B, int S, int N, int C, int H, int W, int L, int r,
+                           float* tokens, const int* num_tracks, const int* num_frames, int B, int S, int N, int C, int H,
+                           int W, int L, int r,
                            int pad_mode, int prec_mode, int D_tok, void* workspace, comet_stream_t stream) {
   tc::Params p{};
   int rc = tc_common(p, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, B, S, N, C, H, W, L, r, pad_mode,
@@ -1651,7 +1655,7 @@ static int tc_track_tokens(const void* split, const float* track_feats, long lon
   COMET_REQUIRE(D_tok >= need, "D_tok=%d smaller than the %d token channels", D_tok, need);
   if ((long long)B * S * N == 0) return COMET_OK;
   COMET_REQUIRE(split && track_feats && coords && pos_emb && tokens, "null pointer");
-  p.out = tokens; p.pos = pos_emb; p.D_tok = D_tok; p.tokens = 1; p.ntr = num_tracks;
+  p.out = tokens; p.pos = pos_emb; p.D_tok = D_tok; p.tokens = 1; p.ntr = num_tracks; p.nfr = num_frames;
   return tc::launch(p, split, workspace, (cudaStream_t)stream);
 }
 
@@ -1660,8 +1664,8 @@ extern "C" int comet_tc_track_tokens_f32(const void* split, const float* track_f
                                          long long c_sn, const float* pos_emb, float* tokens, int B, int S, int N,
                                          int C, int H, int W, int L, int r, int pad_mode, int prec_mode, int D_tok,
                                          void* workspace, comet_stream_t stream) {
-  return tc_track_tokens(split, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, nullptr, B, S, N,
-                         C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace, stream);
+  return tc_track_tokens(split, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, nullptr, nullptr, B,
+                         S, N, C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace, stream);
 }
 
 extern "C" int comet_tc_track_tokens_ragged_f32(const void* split, const float* track_feats, long long t_sb, long long t_ss,
@@ -1670,8 +1674,18 @@ extern "C" int comet_tc_track_tokens_ragged_f32(const void* split, const float* 
                                                 int B, int S, int N, int C, int H, int W, int L, int r, int pad_mode,
                                                 int prec_mode, int D_tok, void* workspace, comet_stream_t stream) {
   COMET_REQUIRE((long long)B * S * N == 0 || num_tracks, "null num_tracks");
-  return tc_track_tokens(split, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks, B, S,
-                         N, C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace, stream);
+  return tc_track_tokens(split, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks, nullptr,
+                         B, S, N, C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace, stream);
+}
+
+extern "C" int comet_tc_track_tokens_varlen_f32(const void* split, const float* track_feats, long long t_sb, long long t_ss,
+                                                long long t_sn, const float* coords, long long c_sb, long long c_ss,
+                                                long long c_sn, const float* pos_emb, float* tokens, const int* num_tracks,
+                                                const int* num_frames, int B, int S, int N, int C, int H, int W, int L, int r,
+                                                int pad_mode, int prec_mode, int D_tok, void* workspace,
+                                                comet_stream_t stream) {
+  return tc_track_tokens(split, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks,
+                         num_frames, B, S, N, C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace, stream);
 }
 
 extern "C" int comet_tc_corr_volume_f32(const void* split, const float* targets, long long t_sb, long long t_ss,

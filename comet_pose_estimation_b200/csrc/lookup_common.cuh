@@ -20,6 +20,7 @@ struct LookupParams {
   long long o_sb, o_ss, o_sn;
   const float* pos;  // TOKENS: (B,N,D_tok)
   const int* ntr;    // TOKENS: (B,) query count of each sequence (rows n >= ntr[b] are written as zeros), or null
+  const int* nfr;    // TOKENS: (B,) frame count of each sequence (rows s >= nfr[b] are written as zeros), or null
   int D_tok;
   int B, S, N, C, L, r;
   int pad_border, bf16;

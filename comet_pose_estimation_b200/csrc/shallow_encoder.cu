@@ -291,8 +291,18 @@ struct Params {
   long long sn, sc, sy, sx;  // element strides of the patch tensor (topleft == null) / of the image (sc, sy, sx)
   int S, N, H, W;
   int nseq;                // packed tracks: number of sequences in `src`
+  const int* num_frames;   // packed tracks, nullable: sequence b has num_frames[b] real frames; the patches of the others
+                           // are not read and their maps are written as zeros
   float eps;
 };
+
+// Packed tracks with frame counts: patch pi lies in a frame past its sequence's count.
+__device__ __forceinline__ bool padded_patch(const Params& p, long long pi) {
+  if (!p.num_frames) return false;
+  const int s = (int)(pi % p.S);
+  const int b = min(max(__ldg(p.seq_of_track + pi / p.S), 0), p.nseq - 1);
+  return s >= __ldg(p.num_frames + b);
+}
 
 // pixels of patch pair `pair` -> registers: thread <-> cells tid + 256 k of the 2 x 31 x 31 cells, 3 channels each
 __device__ __forceinline__ void prefetch_pixels(const Params& p, long long pair, int tid, float (&pre)[24]) {
@@ -301,7 +311,9 @@ __device__ __forceinline__ void prefetch_pixels(const Params& p, long long pair,
   for (int g = 0; g < G; ++g) {
     long long pi = pair * G + g;
     if (pi >= p.P) pi = p.P - 1;   // odd patch count: the last pair encodes the last patch twice and stores it once
-    if (p.topleft) {
+    if (padded_patch(p, pi)) {
+      base[g] = nullptr;           // encodes a zero patch; its output is written as zeros
+    } else if (p.topleft) {
       const int s = (int)(pi % p.S);
       const long long bn = pi / p.S;
       const int n = (int)(bn % p.N);
@@ -322,10 +334,15 @@ __device__ __forceinline__ void prefetch_pixels(const Params& p, long long pair,
     const int cell = tid + k * THREADS;
     if (cell < G * PSZ * PSZ) {
       const int g = cell >= PSZ * PSZ ? 1 : 0, r = cell - g * (PSZ * PSZ), y = r / PSZ, x = r - y * PSZ;
-      const float* b = (g == 0 ? base[0] : base[1]) + y * p.sy + x * p.sx;
-      pre[3 * k] = __ldg(b);
-      pre[3 * k + 1] = __ldg(b + p.sc);
-      pre[3 * k + 2] = __ldg(b + 2 * p.sc);
+      const float* b = g == 0 ? base[0] : base[1];
+      if (b) {
+        b += y * p.sy + x * p.sx;
+        pre[3 * k] = __ldg(b);
+        pre[3 * k + 1] = __ldg(b + p.sc);
+        pre[3 * k + 2] = __ldg(b + 2 * p.sc);
+      } else {
+        pre[3 * k] = pre[3 * k + 1] = pre[3 * k + 2] = 0.f;
+      }
     }
   }
 }
@@ -504,9 +521,15 @@ __global__ void __launch_bounds__(THREADS, 1) shallow_encoder_kernel(const Param
       const long long pi = pair * G + g;
       if (pi >= p.P) continue;
       const float* row = smem + g * PATCH_FLOATS + OFF_XP + ((oy + 1) * XP_W + 1 + pw) * CS;
+      float* o = p.out + (pi * 256 + oy * 16 + pw) * C + 4 * cw;
+      if (padded_patch(p, pi)) {
+#pragma unroll
+        for (int jj = 0; jj < 8; ++jj)
+          *reinterpret_cast<float4*>(o + ((jj >> 2) * 16 + (jj & 3) * 4) * C) = make_float4(0.f, 0.f, 0.f, 0.f);
+        continue;
+      }
       fill32(acw, bias4[L_CONV2 * 8 + cw]);
       conv32<16, 1, XP_W, CS, 1, 8, 8>(row, ws + WS_CONV2, cw, 0, acw);
-      float* o = p.out + (pi * 256 + oy * 16 + pw) * C + 4 * cw;
 #pragma unroll
       for (int jj = 0; jj < 8; ++jj) {
         const float4 x = *reinterpret_cast<const float4*>(row + ((jj >> 2) * XP_W + (jj & 3) * 4) * CS + 4 * cw);
@@ -607,17 +630,24 @@ extern "C" int comet_shallow_encoder_from_images_f32(const float* images, const 
   return launch_shallow_encoder(p, stream);
 }
 
-extern "C" int comet_shallow_encoder_from_images_ragged_f32(const float* images, const int* topleft, const int* seq_of_track,
-                                                            const float* packed, float* out, int P, int B, int S, int H, int W,
-                                                            float eps, comet_stream_t stream) {
+extern "C" int comet_shallow_encoder_from_images_varlen_f32(const float* images, const int* topleft, const int* seq_of_track,
+                                                            const int* num_frames, const float* packed, float* out, int P, int B,
+                                                            int S, int H, int W, float eps, comet_stream_t stream) {
   COMET_REQUIRE(P >= 0 && B >= 1 && S >= 0 && H >= senc::PSZ && W >= senc::PSZ, "bad shape");
   if ((long long)P * S == 0) return COMET_OK;
   COMET_REQUIRE(images && topleft && seq_of_track && packed && out, "null pointer");
   COMET_REQUIRE(((uintptr_t)packed % 16) == 0, "packed parameters must be 16-byte aligned");
   senc::Params p{};
-  p.src = images; p.topleft = topleft; p.seq_of_track = seq_of_track; p.packed = packed; p.out = out;
+  p.src = images; p.topleft = topleft; p.seq_of_track = seq_of_track; p.num_frames = num_frames; p.packed = packed; p.out = out;
   p.P = (long long)P * S;
   p.sn = 0; p.sc = (long long)H * W; p.sy = W; p.sx = 1;
   p.S = S; p.N = P; p.H = H; p.W = W; p.nseq = B; p.eps = eps;
   return launch_shallow_encoder(p, stream);
+}
+
+extern "C" int comet_shallow_encoder_from_images_ragged_f32(const float* images, const int* topleft, const int* seq_of_track,
+                                                            const float* packed, float* out, int P, int B, int S, int H, int W,
+                                                            float eps, comet_stream_t stream) {
+  return comet_shallow_encoder_from_images_varlen_f32(images, topleft, seq_of_track, nullptr, packed, out, P, B, S, H, W, eps,
+                                                      stream);
 }

@@ -170,8 +170,10 @@ struct AttnParams {
   // Variable lengths (comet_attention_varlen_planes_f32), null otherwise: item b's queries / outputs start at row q_off[b]
   // and its keys / values at row k_off[b] (the *_sb strides are then row pitches), with q_len[b] / k_len[b] positions.
   // Lq / Lk hold the largest lengths.  A launch serves only the items whose attn_path() is `path`.
+  // `groups` (varlen, nullable): item b's problem count for attn_path() is groups[b] instead of `group`.
   const int* q_off; const int* q_len; const int* k_off; const int* k_len;
   int path, group, mma_opt, mma_align;
+  const int* groups;
 };
 
 // Kernel family of an attention problem: one definition for the host dispatch of comet_attention_planes_f32 and for the
@@ -199,8 +201,9 @@ __device__ __forceinline__ bool attn_item(const AttnParams& p, int b, int q0, At
     return true;
   }
   it.Lq = __ldg(p.q_len + b); it.Lk = __ldg(p.k_len + b);
-  if (q0 >= it.Lq || it.Lk < 1 || attn_path(p.np, it.Lq, it.Lk, p.dh, p.group, p.H, p.mma_opt, p.mma_align) != p.path)
-    return false;
+  if (q0 >= it.Lq || it.Lk < 1) return false;
+  const int group = p.groups ? __ldg(p.groups + b) : p.group;
+  if (attn_path(p.np, it.Lq, it.Lk, p.dh, group, p.H, p.mma_opt, p.mma_align) != p.path) return false;
   const long long qo = __ldg(p.q_off + b), ko = __ldg(p.k_off + b);
   it.qb = qo * p.q_sb; it.kb = ko * p.k_sb; it.vb = ko * p.v_sb; it.ob = qo * p.o_sb;
   return true;
@@ -343,7 +346,7 @@ __global__ void __launch_bounds__(ATT_WARPS * 32) attention_kernel(const AttnPar
 // output row; outputs go back through shared memory so that the plane stores are coalesced.  (The tiled kernel above
 // spends a CTA with two block-wide barriers per (batch, head) on 16 x 16 scores: 113 us per launch for 4608 of them.)
 constexpr int ATS_WARPS = 4;
-template <int DH4>
+template <int DH4, bool VARLEN>
 __global__ void __launch_bounds__(ATS_WARPS * 32) attention_small_kernel(const AttnParams p) {
   constexpr int DH = 4 * DH4;
   extern __shared__ __align__(16) float ats_smem[];
@@ -357,11 +360,14 @@ __global__ void __launch_bounds__(ATS_WARPS * 32) attention_small_kernel(const A
   for (long long w = (long long)blockIdx.x * ATS_WARPS + warp; w < total; w += (long long)gridDim.x * ATS_WARPS) {
     const int h = (int)(w % p.H);
     const int b = (int)(w / p.H);
-    const float* qp = p.q + b * p.q_sb + h * p.dh;
-    const float* kp = p.k + b * p.k_sb + h * p.dh;
-    const float* vp = p.v + b * p.v_sb + h * p.dh;
+    AttnItem it;
+    if (!attn_item<VARLEN>(p, b, 0, it)) continue;     // (warp-uniform)
+    const int Lq = it.Lq, Lk = it.Lk;
+    const float* qp = p.q + it.qb + h * p.dh;
+    const float* kp = p.k + it.kb + h * p.dh;
+    const float* vp = p.v + it.vb + h * p.dh;
     __syncwarp();
-    for (int e = lane; e < p.Lk * DH4; e += 32) {
+    for (int e = lane; e < Lk * DH4; e += 32) {
       const int r = e / DH4, t = e - r * DH4;
       float4 kk = make_float4(0.f, 0.f, 0.f, 0.f), vv = kk;
       if (t < dh4) {
@@ -375,11 +381,11 @@ __global__ void __launch_bounds__(ATS_WARPS * 32) attention_small_kernel(const A
     // At most 16 queries (the T = 16 time attention): both half-warps take the same queries and split the KEYS -- lanes
     // 0-15 the first half, lanes 16-31 the second -- and merge their running (max, sum, output row) with the online-softmax
     // rescale through 16-lane shuffles; otherwise half of the warp would idle through the whole (batch item, head).
-    const bool split = p.Lq <= 16;
+    const bool split = Lq <= 16;
     const int qrow = split ? (lane & 15) : lane;
-    const int khalf = (p.Lk + 1) >> 1;
-    const int j0 = split ? (lane >> 4) * khalf : 0, jn = split ? khalf : p.Lk;
-    const bool active = qrow < p.Lq;
+    const int khalf = (Lk + 1) >> 1;
+    const int j0 = split ? (lane >> 4) * khalf : 0, jn = split ? khalf : Lk;
+    const bool active = qrow < Lq;
 #pragma unroll
     for (int t = 0; t < DH4; ++t) {
       q4[t] = (active && t < dh4) ? __ldg(reinterpret_cast<const float4*>(qp + (long long)qrow * p.q_si) + t)
@@ -390,7 +396,7 @@ __global__ void __launch_bounds__(ATS_WARPS * 32) attention_small_kernel(const A
     float mx = -INFINITY;
     for (int jj = 0; jj < jn; ++jj) {
       const int j = j0 + jj;
-      if (j >= p.Lk) break;              // (odd Lk: the second half is one key shorter)
+      if (j >= Lk) break;                // (odd Lk: the second half is one key shorter)
       const float4* kr = reinterpret_cast<const float4*>(Ks + j * DH);
       float sx = 0.f, sy = 0.f, sz = 0.f, sw = 0.f;      // four independent chains: one serial chain of dh FMAs is latency-bound
 #pragma unroll
@@ -408,7 +414,7 @@ __global__ void __launch_bounds__(ATS_WARPS * 32) attention_small_kernel(const A
     float sum = 0.f;
     for (int jj = 0; jj < jn; ++jj) {
       const int j = j0 + jj;
-      if (j >= p.Lk) break;
+      if (j >= Lk) break;
       const float pj = expf(Ss[j * 33 + lane] - mx);
       sum += pj;
       const float4* vr = reinterpret_cast<const float4*>(Vs + j * DH);
@@ -443,15 +449,15 @@ __global__ void __launch_bounds__(ATS_WARPS * 32) attention_small_kernel(const A
     }
     __syncwarp();
     if (p.vec_out) {
-      for (int e = lane; e < p.Lq * dh4; e += 32) {
+      for (int e = lane; e < Lq * dh4; e += 32) {
         const int i = e / dh4, t = e - i * dh4;
-        store_planes4(p.out, p.o_plane_stride, b * p.o_sb + (long long)i * p.o_si + h * p.dh + 4 * t,
+        store_planes4(p.out, p.o_plane_stride, it.ob + (long long)i * p.o_si + h * p.dh + 4 * t,
                       *reinterpret_cast<const float4*>(Os + i * OLD + 4 * t), p.np);
       }
     } else
-    for (int e = lane; e < p.Lq * p.dh; e += 32) {
+    for (int e = lane; e < Lq * p.dh; e += 32) {
       const int i = e / p.dh, d = e - i * p.dh;
-      store_planes(p.out, p.o_plane_stride, b * p.o_sb + (long long)i * p.o_si + h * p.dh + d, Os[i * OLD + d], p.np);
+      store_planes(p.out, p.o_plane_stride, it.ob + (long long)i * p.o_si + h * p.dh + d, Os[i * OLD + d], p.np);
     }
   }
 }
@@ -704,7 +710,7 @@ __global__ void __launch_bounds__(ATM_WARPS * 32) attention_rows_mma_kernel(cons
 // 12 + 12 MMAs instead of ~2000 FMA-pipe instructions.  K / V of the (batch, head) sit in the warp's own shared-memory
 // slice (bf16; V transposed); no block-wide barrier.
 constexpr int ATSM_WARPS = 4;
-template <int DH>
+template <int DH, bool VARLEN>
 __global__ void __launch_bounds__(ATSM_WARPS * 32) attention_small_mma_kernel(const AttnParams p) {
   constexpr int KLD = DH + 8, VLD = 32 + 8, KS = DH / 16, DT = DH / 8;
   __shared__ __align__(16) __nv_bfloat16 Ks_all[ATSM_WARPS][32 * KLD];    // [key][dh]
@@ -715,15 +721,18 @@ __global__ void __launch_bounds__(ATSM_WARPS * 32) attention_small_mma_kernel(co
   const long long total = (long long)p.B * p.H;
   for (long long w = (long long)blockIdx.x * ATSM_WARPS + warp; w < total; w += (long long)gridDim.x * ATSM_WARPS) {
     const int h = (int)(w % p.H);
-    const long long b = w / p.H;
-    const float* qp = p.q + b * p.q_sb + h * DH;
-    const float* kp = p.k + b * p.k_sb + h * DH;
-    const float* vp = p.v + b * p.v_sb + h * DH;
+    const int b = (int)(w / p.H);
+    AttnItem it;
+    if (!attn_item<VARLEN>(p, b, 0, it)) continue;     // (warp-uniform)
+    const int Lq = it.Lq, Lk = it.Lk;
+    const float* qp = p.q + it.qb + h * DH;
+    const float* kp = p.k + it.kb + h * DH;
+    const float* vp = p.v + it.vb + h * DH;
     __syncwarp();                               // the previous (batch, head) is fully consumed
     for (int e = lane; e < 32 * (DH / 4); e += 32) {
       const int r = e / (DH / 4), c4 = e - r * (DH / 4);
       float4 kk = make_float4(0.f, 0.f, 0.f, 0.f), vv = kk;
-      if (r < p.Lk) {
+      if (r < Lk) {
         kk = __ldg(reinterpret_cast<const float4*>(kp + (long long)r * p.k_si) + c4);
         vv = __ldg(reinterpret_cast<const float4*>(vp + (long long)r * p.v_si) + c4);
       }
@@ -738,11 +747,11 @@ __global__ void __launch_bounds__(ATSM_WARPS * 32) attention_small_mma_kernel(co
 #pragma unroll
     for (int ks = 0; ks < KS; ++ks) {
       float2 x00 = make_float2(0.f, 0.f), x01 = x00, x10 = x00, x11 = x00;
-      if (r0 < p.Lq) {
+      if (r0 < Lq) {
         x00 = __ldg(reinterpret_cast<const float2*>(qp + (long long)r0 * p.q_si + ks * 16 + 2 * t));
         x01 = __ldg(reinterpret_cast<const float2*>(qp + (long long)r0 * p.q_si + ks * 16 + 2 * t + 8));
       }
-      if (r1 < p.Lq) {
+      if (r1 < Lq) {
         x10 = __ldg(reinterpret_cast<const float2*>(qp + (long long)r1 * p.q_si + ks * 16 + 2 * t));
         x11 = __ldg(reinterpret_cast<const float2*>(qp + (long long)r1 * p.q_si + ks * 16 + 2 * t + 8));
       }
@@ -766,8 +775,8 @@ __global__ void __launch_bounds__(ATSM_WARPS * 32) attention_small_mma_kernel(co
 #pragma unroll
     for (int nt = 0; nt < 4; ++nt) {
       const int key = nt * 8 + 2 * t;
-      if (key >= p.Lk) { sacc[nt][0] = -INFINITY; sacc[nt][2] = -INFINITY; }
-      if (key + 1 >= p.Lk) { sacc[nt][1] = -INFINITY; sacc[nt][3] = -INFINITY; }
+      if (key >= Lk) { sacc[nt][0] = -INFINITY; sacc[nt][2] = -INFINITY; }
+      if (key + 1 >= Lk) { sacc[nt][1] = -INFINITY; sacc[nt][3] = -INFINITY; }
       m0 = fmaxf(m0, fmaxf(sacc[nt][0], sacc[nt][1]));
       m1 = fmaxf(m1, fmaxf(sacc[nt][2], sacc[nt][3]));
     }
@@ -800,12 +809,12 @@ __global__ void __launch_bounds__(ATSM_WARPS * 32) attention_small_mma_kernel(co
       }
     }
     const float i0 = 1.f / s0, i1 = 1.f / s1;
-    __nv_bfloat16* o0 = p.out + b * p.o_sb + (long long)r0 * p.o_si + h * DH + 2 * t;
-    __nv_bfloat16* o1 = p.out + b * p.o_sb + (long long)r1 * p.o_si + h * DH + 2 * t;
+    __nv_bfloat16* o0 = p.out + it.ob + (long long)r0 * p.o_si + h * DH + 2 * t;
+    __nv_bfloat16* o1 = p.out + it.ob + (long long)r1 * p.o_si + h * DH + 2 * t;
 #pragma unroll
     for (int dt = 0; dt < DT; ++dt) {
-      if (r0 < p.Lq) *reinterpret_cast<uint32_t*>(o0 + dt * 8) = pack_bf16(oacc[dt][0] * i0, oacc[dt][1] * i0);
-      if (r1 < p.Lq) *reinterpret_cast<uint32_t*>(o1 + dt * 8) = pack_bf16(oacc[dt][2] * i1, oacc[dt][3] * i1);
+      if (r0 < Lq) *reinterpret_cast<uint32_t*>(o0 + dt * 8) = pack_bf16(oacc[dt][0] * i0, oacc[dt][1] * i0);
+      if (r1 < Lq) *reinterpret_cast<uint32_t*>(o1 + dt * 8) = pack_bf16(oacc[dt][2] * i1, oacc[dt][3] * i1);
     }
   }
 }
@@ -1012,8 +1021,8 @@ static int launch_attention(int path, const AttnParams& p, cudaStream_t stream) 
   if (path == AP_SMALL_MMA) {
     long long nb = (B * H + ATSM_WARPS - 1) / ATSM_WARPS;
     if (nb > 148LL * 16) nb = 148LL * 16;
-    if (dh == 32) attention_small_mma_kernel<32><<<(unsigned)nb, ATSM_WARPS * 32, 0, stream>>>(p);
-    else attention_small_mma_kernel<48><<<(unsigned)nb, ATSM_WARPS * 32, 0, stream>>>(p);
+    if (dh == 32) attention_small_mma_kernel<32, VARLEN><<<(unsigned)nb, ATSM_WARPS * 32, 0, stream>>>(p);
+    else attention_small_mma_kernel<48, VARLEN><<<(unsigned)nb, ATSM_WARPS * 32, 0, stream>>>(p);
     return launch_status("attention_small_mma_kernel");
   }
   if (path == AP_SMALL) {
@@ -1023,8 +1032,8 @@ static int launch_attention(int path, const AttnParams& p, cudaStream_t stream) 
   do {                                                                                                             \
     const int smem = ATS_WARPS * (32 * 4 * D4 + 32 * (4 * D4 + 4) + 32 * 33) * (int)sizeof(float);                 \
     if (smem > 48 * 1024)                                                                                          \
-      COMET_CUDA(cudaFuncSetAttribute(attention_small_kernel<D4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-    attention_small_kernel<D4><<<(unsigned)nb, ATS_WARPS * 32, smem, stream>>>(p);                                 \
+      COMET_CUDA(cudaFuncSetAttribute(attention_small_kernel<D4, VARLEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
+    attention_small_kernel<D4, VARLEN><<<(unsigned)nb, ATS_WARPS * 32, smem, stream>>>(p);                                 \
   } while (0)
     if (dh <= 4) COMET_ATS_LAUNCH(1);
     else if (dh <= 16) COMET_ATS_LAUNCH(4);
@@ -1121,18 +1130,20 @@ extern "C" int comet_attention_planes_f32(const float* q, long long q_sb, long l
   return launch_attention<false>(path, p, (cudaStream_t)stream);
 }
 
-extern "C" int comet_attention_varlen_planes_f32(const float* q, long long q_ld, long long q_step, const float* k,
-                                                 long long k_ld, long long k_step, const float* v, void* out_planes,
-                                                 long long o_plane_stride, long long o_ld, int np, int items, int H, int dh,
-                                                 const int* q_off, const int* q_len, const int* k_off, const int* k_len,
-                                                 int min_lq, int max_lq, int min_lk, int max_lk, int group,
-                                                 comet_stream_t stream) {
-  COMET_REQUIRE(items >= 0 && H >= 1 && min_lq >= 1 && max_lq >= min_lq && min_lk >= 1 && max_lk >= min_lk && group >= 1 &&
-                    dh >= 4 && dh <= 64 && dh % 4 == 0,
-                "bad varlen attention shape (items=%d H=%d Lq in [%d, %d] Lk in [%d, %d] group=%d dh=%d)", items, H, min_lq,
-                max_lq, min_lk, max_lk, group, dh);
+extern "C" int comet_attention_varlen_grouped_planes_f32(const float* q, long long q_ld, long long q_step, const float* k,
+                                                         long long k_ld, long long k_step, const float* v, void* out_planes,
+                                                         long long o_plane_stride, long long o_ld, int np, int items, int H,
+                                                         int dh, const int* q_off, const int* q_len, const int* k_off,
+                                                         const int* k_len, int min_lq, int max_lq, int min_lk, int max_lk,
+                                                         const int* groups, int min_group, int max_group,
+                                                         comet_stream_t stream) {
+  COMET_REQUIRE(items >= 0 && H >= 1 && min_lq >= 0 && max_lq >= min_lq && min_lk >= 0 && max_lk >= min_lk &&
+                    min_group >= 1 && max_group >= min_group && (groups || min_group == max_group) && dh >= 4 && dh <= 64 &&
+                    dh % 4 == 0,
+                "bad varlen attention shape (items=%d H=%d Lq in [%d, %d] Lk in [%d, %d] group in [%d, %d] dh=%d)", items, H,
+                min_lq, max_lq, min_lk, max_lk, min_group, max_group, dh);
   COMET_REQUIRE(np == 1 || np == 3, "np must be 1 or 3");
-  if ((long long)items * max_lq == 0) return COMET_OK;
+  if ((long long)items * max_lq * max_lk == 0) return COMET_OK;
   COMET_REQUIRE(q && k && v && out_planes && q_off && q_len && k_off && k_len, "null pointer");
   COMET_REQUIRE(((uintptr_t)q % 16) == 0 && ((uintptr_t)k % 16) == 0 && ((uintptr_t)v % 16) == 0 && q_ld % 4 == 0 &&
                     k_ld % 4 == 0, "q / k / v rows must be 16-byte aligned");
@@ -1141,20 +1152,19 @@ extern "C" int comet_attention_varlen_planes_f32(const float* q, long long q_ld,
                max_lk, dh, 1.0f / sqrtf((float)dh),
                (o_ld % 4 == 0 && (q_step * o_ld) % 4 == 0 && o_plane_stride % 4 == 0 && ((uintptr_t)out_planes % 8) == 0) ? 1 : 0};
   p.q_off = q_off; p.q_len = q_len; p.k_off = k_off; p.k_len = k_len;
-  p.group = group;
+  p.group = max_group;
+  p.groups = groups;
   p.mma_opt = option(COMET_OPT_ATTN_MMA);
   p.mma_align = mma_alignment(q_ld, q_step * q_ld, o_ld, q_step * o_ld, out_planes);
-  // The lengths live on the device: launch every family that some length pair of the given ranges selects (the path
-  // depends on a length only through the thresholds 16 / 32 / 64 and the number of 64-query chunks, so every length up
-  // to 65 and then every 64th is enough); each CTA serves the items of its own family.
+  // The lengths live on the device: launch every family that some (length pair, group) of the given ranges selects (the
+  // path depends on a length only through the thresholds 16 / 32 / 64 and the number of 64-query chunks, so every length
+  // up to 65 and then every 64th is enough; on the group only through one upper bound, so both ends are enough).  Items
+  // of length 0 select no family; each CTA serves the items of its own family.
   auto next = [](int x, int hi) { return x < 65 ? x + 1 : x < hi ? (x + 64 < hi ? x + 64 : hi) : hi + 1; };
   bool used[AP_COUNT] = {};
-  for (int lq = min_lq; lq <= max_lq; lq = next(lq, max_lq))
-    for (int lk = min_lk; lk <= max_lk; lk = next(lk, max_lk))
-      used[attn_path(np, lq, lk, dh, group, H, p.mma_opt, p.mma_align)] = true;
-  COMET_REQUIRE(!used[AP_SMALL] && !used[AP_SMALL_MMA],
-                "varlen attention serves items with more than 32 queries or more than 32 keys (Lq in [%d, %d], Lk in [%d, %d])",
-                min_lq, max_lq, min_lk, max_lk);
+  for (int lq = min_lq > 1 ? min_lq : 1; lq <= max_lq; lq = next(lq, max_lq))
+    for (int lk = min_lk > 1 ? min_lk : 1; lk <= max_lk; lk = next(lk, max_lk))
+      for (int g : {min_group, max_group}) used[attn_path(np, lq, lk, dh, g, H, p.mma_opt, p.mma_align)] = true;
   for (int path = 0; path < AP_COUNT; ++path) {
     if (!used[path]) continue;
     p.path = path;
@@ -1162,6 +1172,19 @@ extern "C" int comet_attention_varlen_planes_f32(const float* q, long long q_ld,
     if (rc != COMET_OK) return rc;
   }
   return COMET_OK;
+}
+
+extern "C" int comet_attention_varlen_planes_f32(const float* q, long long q_ld, long long q_step, const float* k,
+                                                 long long k_ld, long long k_step, const float* v, void* out_planes,
+                                                 long long o_plane_stride, long long o_ld, int np, int items, int H, int dh,
+                                                 const int* q_off, const int* q_len, const int* k_off, const int* k_len,
+                                                 int min_lq, int max_lq, int min_lk, int max_lk, int group,
+                                                 comet_stream_t stream) {
+  COMET_REQUIRE(min_lq >= 1 && min_lk >= 1, "bad varlen attention lengths (Lq in [%d, %d], Lk in [%d, %d])", min_lq, max_lq,
+                min_lk, max_lk);
+  return comet_attention_varlen_grouped_planes_f32(q, q_ld, q_step, k, k_ld, k_step, v, out_planes, o_plane_stride, o_ld, np,
+                                                   items, H, dh, q_off, q_len, k_off, k_len, min_lq, max_lq, min_lk, max_lk,
+                                                   nullptr, group, group, stream);
 }
 
 extern "C" int comet_add_planes_f32(const float* a, const float* b, void* planes, long long plane_stride, int np, long long n,

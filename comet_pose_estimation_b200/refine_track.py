@@ -172,10 +172,11 @@ class ShallowEncoder(nn.Module):
         return self._fused_result(out, (31 // self.stride, 31 // self.stride), defer_upsample)
 
     def encode_packed_patches_of(self, images: torch.Tensor, topleft: torch.Tensor, seq_of_track: torch.Tensor,
-                                 defer_upsample: bool = True):
+                                 defer_upsample: bool = True, num_frames: torch.Tensor = None):
         """``encode_patches_of`` for P tracks packed from the sequences of ``images`` (B,S,3,H,W): ``topleft`` (P,S,2)
         corners, ``seq_of_track`` (P,) the sequence of each track.  Maps in (track, frame) order, each one bit-identical
-        to ``encode_patches_of`` on the same patch."""
+        to ``encode_patches_of`` on the same patch.  ``num_frames`` (B,) int32 on the device, or None: sequence b has
+        num_frames[b] real frames; the pixels of the other frames are never read and their maps are zeros."""
         from . import _lib
         from ._dev import stream_ptr
 
@@ -186,9 +187,15 @@ class ShallowEncoder(nn.Module):
         seq32 = seq_of_track.to(device=images.device, dtype=torch.int32).contiguous()
         out = torch.empty((P * S, 16, 16, 32), dtype=torch.float32, device=images.device)
         with torch.cuda.device(images.device):
-            _lib.check(_lib.lib.comet_shallow_encoder_from_images_ragged_f32(
-                img.data_ptr(), tl32.data_ptr(), seq32.data_ptr(), self.packed_parameters().data_ptr(), out.data_ptr(), P, B,
-                S, H, W, float(self.norm1.eps), stream_ptr(images.device)))
+            if num_frames is None:
+                _lib.check(_lib.lib.comet_shallow_encoder_from_images_ragged_f32(
+                    img.data_ptr(), tl32.data_ptr(), seq32.data_ptr(), self.packed_parameters().data_ptr(), out.data_ptr(), P,
+                    B, S, H, W, float(self.norm1.eps), stream_ptr(images.device)))
+            else:
+                nf32 = num_frames.to(device=images.device, dtype=torch.int32).contiguous()
+                _lib.check(_lib.lib.comet_shallow_encoder_from_images_varlen_f32(
+                    img.data_ptr(), tl32.data_ptr(), seq32.data_ptr(), nf32.data_ptr(), self.packed_parameters().data_ptr(),
+                    out.data_ptr(), P, B, S, H, W, float(self.norm1.eps), stream_ptr(images.device)))
         return self._fused_result(out, (31 // self.stride, 31 // self.stride), defer_upsample)
 
     def forward(self, x, defer_upsample: bool = False):
@@ -251,18 +258,22 @@ def extract_patches(images: torch.Tensor, topleft: torch.Tensor, psize: int) -> 
 
 
 def refine_track(images, fine_fnet, fine_tracker, coarse_pred, pradius=15, sradius=2, compute_score=False,
-                 num_tracks=None):
+                 num_tracks=None, num_frames=None):
     """refine_track.py:26-171.  ``images`` (B,S,3,H,W); ``coarse_pred`` (B,S,N,2) pixels ->
     (refined_tracks (B,S,N,2), score (B,S,N) | None).
 
     ``num_tracks`` (B ints or a 1-D tensor): ``coarse_pred`` is a padded batch; sequence b's tracks get what the call on
     that sequence alone returns (including the score quirk as it behaves for one sequence: every window of sequence b
-    is cut from the frame-0 map of its own first track), entries of padded tracks are 0."""
-    if num_tracks is not None:
+    is cut from the frame-0 map of its own first track), entries of padded tracks are 0.  ``num_frames`` (likewise):
+    sequence b has the first ``num_frames[b]`` frames; the images of the others are never read and their entries are 0."""
+    if num_tracks is not None or num_frames is not None:
         from .utils import check_num_tracks
 
-        counts = check_num_tracks(num_tracks, coarse_pred.shape[0], coarse_pred.shape[2])
-        return _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, sradius, compute_score, counts)
+        B, S, N = coarse_pred.shape[:3]
+        counts = check_num_tracks([N] * B if num_tracks is None else num_tracks, B, N)
+        frames = None if num_frames is None else check_num_tracks(num_frames, B, S)
+        return _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, sradius, compute_score, counts,
+                                    frames)
     B, S, N, _ = coarse_pred.shape
     _, _, _, H, W = images.shape
     psize = pradius * 2 + 1
@@ -331,10 +342,11 @@ def refine_track(images, fine_fnet, fine_tracker, coarse_pred, pradius=15, sradi
     return refined_tracks, score
 
 
-def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, sradius, compute_score, counts):
+def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, sradius, compute_score, counts, frames=None):
     """The fine tracker works per track, so the real tracks of all sequences run as ONE packed batch of P = sum(counts)
     tracks, without per-sequence padding: the fused encoder reads each track's patches from its own sequence's frames.  Configurations
-    without the fused encoder run the per-sequence definition."""
+    without the fused encoder run the per-sequence definition.  ``frames``: per-sequence frame counts (None: all S); each
+    packed track then runs its own sequence's frame count through the fine tracker."""
     from .base_track_predictor import BaseTrackerPredictor
 
     B, S, N, _ = coarse_pred.shape
@@ -348,11 +360,12 @@ def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, 
         refined = coarse_pred.new_zeros(coarse_pred.shape)
         score = coarse_pred.new_zeros((B, S, N)) if compute_score else None
         for b, n in enumerate(counts):
-            r, sc = refine_track(images[b:b + 1], fine_fnet, fine_tracker, coarse_pred[b:b + 1, :, :n], pradius, sradius,
-                                 compute_score)
-            refined[b, :, :n] = r[0]
+            sb = S if frames is None else frames[b]
+            r, sc = refine_track(images[b:b + 1, :sb], fine_fnet, fine_tracker, coarse_pred[b:b + 1, :sb, :n], pradius,
+                                 sradius, compute_score)
+            refined[b, :sb, :n] = r[0]
             if compute_score:
-                score[b, :, :n] = sc[0]
+                score[b, :sb, :n] = sc[0]
         return refined, score
 
     # The packed count is rounded up to one of four buckets per octave, so that the fine transformer's captured graphs
@@ -372,7 +385,8 @@ def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, 
     topleft_raw = track_int - pradius
     topleft = torch.stack([topleft_raw[..., 0].clamp(0, W - psize), topleft_raw[..., 1].clamp(0, H - psize)], dim=-1)
 
-    half, size = fine_fnet.encode_packed_patches_of(images, topleft, seq, defer_upsample=True)
+    dev_frames = None if frames is None else torch.tensor(frames, dtype=torch.int32, device=dev)
+    half, size = fine_fnet.encode_packed_patches_of(images, topleft, seq, defer_upsample=True, num_frames=dev_frames)
     Hs, Ws = half.shape[-2:]
     C_out = half.shape[1]
     half = half.contiguous(memory_format=torch.channels_last)
@@ -386,37 +400,47 @@ def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, 
         patch_feat = _resize(half, size).reshape(P_cap, S, C_out, psize, psize)
 
     patch_query_points = (track_frac[:, 0] + pradius).reshape(P_cap, 2).unsqueeze(1)
-    fine_lists, _, _, query_point_feat, _ = fine_tracker(
-        query_points=patch_query_points, fmaps=patch_feat, iters=6, return_feat=True, TRACKorPOSE=False)
+    if frames is None:
+        fine_lists, _, _, query_point_feat, _ = fine_tracker(
+            query_points=patch_query_points, fmaps=patch_feat, iters=6, return_feat=True, TRACKorPOSE=False)
+    else:
+        fine_lists, _, _, query_point_feat, _ = fine_tracker(
+            query_points=patch_query_points, fmaps=patch_feat, iters=6, return_feat=True, TRACKorPOSE=False,
+            num_frames=dev_frames[seq])
     fine_pred_track = fine_lists[-1][:P].clone()                           # (P, S, 1, 2), relative to the patch corner
     refined_p = fine_lists[-1][:P].squeeze(-2) + topleft_raw[:P]           # (P, S, 2)
     refined_p[:, 0] = query_points[:P]
+    if frames is not None:
+        refined_p = refined_p.masked_fill((torch.arange(S, device=dev)[None, :] >= dev_frames[seq_real][:, None])[..., None],
+                                          0.0)
     refined = coarse_pred.new_zeros(coarse_pred.shape)
     refined[seq_real, :, loc] = refined_p
 
     score = None
     if compute_score:
         score = _score_ragged(query_point_feat[:P].reshape(P, C_out), patch_feat, fine_pred_track, sradius, psize, counts,
-                              first, B, N, S, C_out)
+                              first, B, N, S, C_out, frames)
     return refined, score
 
 
-def _score_ragged(query_point_feat, patch_feat, fine_pred_track, sradius, psize, counts, first, B, N, S, C_out):
+def _score_ragged(query_point_feat, patch_feat, fine_pred_track, sradius, psize, counts, first, B, N, S, C_out,
+                  frames=None):
     """``compute_score_fn`` of every sequence of a packed batch at once, each as the single-sequence call computes it:
     its windows cut from the frame-0 map of its first track, at the corners of its own k-th track in (n, s) order re-read
-    as (s, n).  -> (B, S, N), zeros for padded tracks."""
+    as (s, n), with the sequence's own frame count as S.  -> (B, S, N), zeros for padded tracks and frames."""
     dev = fine_pred_track.device
     ssize = sradius * 2 + 1
     cnt = torch.tensor(counts, device=dev)
+    frm = torch.tensor([S] * B if frames is None else frames, device=dev)
     corner = (fine_pred_track.floor().int() - sradius).clamp(0, psize - ssize).squeeze(2)   # (P, S, 2) = (x, y)
     bb = torch.arange(B, device=dev)[:, None, None].expand(B, S - 1, N)
     sp = torch.arange(1, S, device=dev)[None, :, None].expand(B, S - 1, N)
     nn_ = torch.arange(N, device=dev)[None, None, :].expand(B, S - 1, N)
-    nb = cnt[bb]
-    real = nn_ < nb
+    nb, sb = cnt[bb], frm[bb]
+    real = (nn_ < nb) & (sp < sb)
     k = sp * nb + nn_                                   # position (s, n) of sequence b reads window k of its (n, s) list
-    src_track = torch.where(real, first[bb] + k // S, first[bb])
-    src_frame = torch.where(real, k % S, torch.zeros_like(k))
+    src_track = torch.where(real, first[bb] + k // sb, first[bb])
+    src_frame = torch.where(real, k % sb, torch.zeros_like(k))
     b_r, src_track, src_frame = bb[real], src_track[real], src_frame[real]
     q = query_point_feat[first[b_r] + nn_[real]]       # (M, C)
     cx = corner[src_track, src_frame, 0].long()

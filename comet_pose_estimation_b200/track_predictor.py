@@ -93,9 +93,19 @@ class TrackerPredictor(nn.Module):
             assert B == 1, "now we only support processing one scene during inference"
         return self._encode_frames(images)
 
-    def _encode_frames(self, images):
-        """(B,S,3,H,W) -> (B,S,128,h,w): one encoder call over all B*S frames."""
+    def _encode_frames(self, images, frames=None):
+        """(B,S,3,H,W) -> (B,S,128,h,w): one encoder call over all B*S frames.  ``frames`` (B ints): only the first
+        frames[b] frames of sequence b are read and encoded (in one call: the instance norms are per frame); the maps of
+        the others are zeros."""
         B, S, C, H, W = images.shape
+        if frames is not None:
+            fm = self._encode_frames(torch.cat([images[b, :n] for b, n in enumerate(frames)])[None])[0]
+            out = fm.new_zeros((B, S) + tuple(fm.shape[1:]))
+            at = 0
+            for b, n in enumerate(frames):
+                out[b, :n] = fm[at:at + n]
+                at += n
+            return out
         x = images.reshape(B * S, C, H, W)
         if self.coarse_down_ratio > 1:
             # F.interpolate(scale_factor=1/down_ratio, bilinear, align_corners=True): output size floor(H / down_ratio)
@@ -129,13 +139,27 @@ class TrackerPredictor(nn.Module):
         return out
 
     @torch.no_grad()
-    def track_batch(self, images, query_points, num_tracks=None, coarse_iters=4, fine_tracking=True):
-        """``track`` for B sequences in one call: images (B,S,3,H,W) (same S and image size for all), ``query_points``
+    def track_batch(self, images, query_points, num_tracks=None, coarse_iters=4, fine_tracking=True, num_frames=None):
+        """``track`` for B sequences in one call: images (B,S,3,H,W) (same image size for all), ``query_points``
         a list of B tensors (N_b, 2) or a padded (B, N_max, 2) tensor with ``num_tracks`` (B,) (None: every sequence
         has N_max tracks).  Returns ``track``'s dict with padded tensors (entries of tracks n >= N_b are 0) plus
         ``num_tracks`` (B,) int64; ``split_batch`` cuts it into per-sequence dicts.  Sequence b gets what ``track``
-        returns for it alone (up to the rounding of the iterated loop)."""
-        B = images.shape[0]
+        returns for it alone (up to the rounding of the iterated loop).
+
+        Sequences of different lengths: ``images`` a list of B tensors (S_b,3,H,W), or the padded (B,S_max,3,H,W) with
+        ``num_frames`` (B,) (1 <= S_b <= S_max).  Frames s >= S_b of a padded tensor are never read; every output entry
+        of such a frame is 0, ``pred_score`` is normalised over the real frames of each track, and the dict gets
+        ``num_frames`` (B,) int64."""
+        if isinstance(images, (list, tuple)):
+            slens = [int(x.shape[0]) for x in images]
+            assert num_frames is None or check_num_tracks(num_frames, len(images), max(slens)) == slens, \
+                "num_frames disagrees with the image lists"
+            padded = images[0].new_zeros((len(images), max(slens)) + tuple(images[0].shape[1:]))
+            for b, x in enumerate(images):
+                padded[b, :x.shape[0]] = x
+            images, num_frames = padded, slens
+        B, S = images.shape[:2]
+        frames = None if num_frames is None else check_num_tracks(num_frames, B, S)
         if isinstance(query_points, (list, tuple)):
             assert len(query_points) == B, f"{len(query_points)} query tensors for {B} sequences"
             lens = [int(q.shape[0]) for q in query_points]
@@ -149,6 +173,8 @@ class TrackerPredictor(nn.Module):
         assert query_points.dim() == 3 and query_points.shape[0] == B and query_points.shape[2] == 2
         N = query_points.shape[1]
         counts = check_num_tracks([N] * B if num_tracks is None else num_tracks, B, N)
+        if frames is not None:
+            return self._track_batch_frames(images, query_points, counts, frames, coarse_iters, fine_tracking)
         fmaps = self._encode_frames(images)
         coarse_list, vis, track_feats, query_feat, conf = self.coarse_predictor(
             query_points=query_points, fmaps=fmaps, iters=coarse_iters, down_ratio=self.coarse_down_ratio, is_train=False,
@@ -169,16 +195,59 @@ class TrackerPredictor(nn.Module):
         out["num_tracks"] = torch.tensor(counts, dtype=torch.int64)
         return out
 
+    def _track_batch_frames(self, images, query_points, counts, frames, coarse_iters, fine_tracking):
+        """``track_batch`` with per-sequence frame counts (validated lists)."""
+        B, S = images.shape[:2]
+        N = query_points.shape[1]
+        fmaps = self._encode_frames(images, frames)
+        coarse_list, vis, track_feats, query_feat, conf = self.coarse_predictor(
+            query_points=query_points, fmaps=fmaps, iters=coarse_iters, down_ratio=self.coarse_down_ratio, is_train=False,
+            return_feat=True, TRACKorPOSE=False, num_tracks=counts, num_frames=frames)
+        coarse = coarse_list[-1]
+        out = {"coarse_pred_track_list": coarse_list, "coarse_pred_track": coarse, "vis": vis, "conf": conf}
+        real = padded_mask(counts, frames, S, N, coarse.device)
+        if fine_tracking:
+            refined, score = refine_track(images, self.fine_fnet, self.fine_predictor, coarse, compute_score=True,
+                                          num_tracks=counts, num_frames=frames)
+            out["refine_pred_track"] = refined
+            out["track_score"] = score
+            out["pred_score"] = inverted_score_padded(score, real)
+        else:
+            out["refine_pred_track"] = coarse
+            out["pred_score"] = torch.ones_like(vis) * real
+        out["num_tracks"] = torch.tensor(counts, dtype=torch.int64)
+        out["num_frames"] = torch.tensor(frames, dtype=torch.int64)
+        return out
+
+
+def padded_mask(counts, frames, S: int, N: int, device) -> torch.Tensor:
+    """(B, S, N) bool: entry (b, s, n) is a real frame and track of a padded batch."""
+    c = torch.tensor(counts, device=device)
+    f = torch.tensor(frames, device=device)
+    return ((torch.arange(S, device=device)[None, :, None] < f[:, None, None])
+            & (torch.arange(N, device=device)[None, None, :] < c[:, None, None]))
+
+
+def inverted_score_padded(track_score: torch.Tensor, real: torch.Tensor, eps: float = 1e-6) -> torch.Tensor:
+    """``inverted_score`` of a padded batch: each track normalised by its maximum over its real frames only (a padded
+    score of 0 would invert to 1e6 and become the maximum); padded entries are 0."""
+    inv = (1.0 / (track_score + eps)).masked_fill(~real, 0.0)
+    m = inv.max(dim=1, keepdim=True)[0]
+    return inv / torch.where(m > 0, m, torch.ones_like(m))
+
 
 def split_batch(out):
-    """``track_batch``'s padded dict -> list of per-sequence dicts with exactly ``track``'s keys and shapes."""
+    """``track_batch``'s padded dict -> list of per-sequence dicts with exactly ``track``'s keys and shapes (cut along
+    the frame axis too when the dict has ``num_frames``)."""
     counts = [int(n) for n in out["num_tracks"]]
+    frames = [int(s) for s in out["num_frames"]] if "num_frames" in out else [None] * len(counts)
 
-    def cut(v, b, n):
+    def cut(v, b, n, s):
         if v is None:
             return None
         if isinstance(v, list):
-            return [cut(x, b, n) for x in v]
-        return v[b:b + 1, :, :n]
+            return [cut(x, b, n, s) for x in v]
+        return v[b:b + 1, :s, :n]
 
-    return [{k: cut(v, b, n) for k, v in out.items() if k != "num_tracks"} for b, n in enumerate(counts)]
+    return [{k: cut(v, b, n, s) for k, v in out.items() if k not in ("num_tracks", "num_frames")}
+            for b, (n, s) in enumerate(zip(counts, frames))]

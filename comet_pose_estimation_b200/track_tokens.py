@@ -83,9 +83,10 @@ class TrackTokenizer:
 
     def __init__(self, corr: Union[CorrBlock, EfficientCorrBlock, torch.Tensor], coords0: torch.Tensor,
                  tdim: int, num_levels: Optional[int] = None, radius: Optional[int] = None,
-                 padding_mode: Optional[str] = None, num_tracks=None):
+                 padding_mode: Optional[str] = None, num_tracks=None, num_frames=None):
         """``num_tracks`` (B ints or a 1-D tensor): the queries form a padded batch; queries n >= num_tracks[b] are
-        padding, their token rows are zeros and cost no correlation work."""
+        padding, their token rows are zeros and cost no correlation work.  ``num_frames`` (likewise): sequence b has the
+        first num_frames[b] of the S frames; the token rows of the others are zeros and read nothing."""
         if isinstance(corr, (torch.Tensor, Upsampled2x)):
             assert num_levels is not None and radius is not None
             self.radius = radius
@@ -105,6 +106,12 @@ class TrackTokenizer:
 
             counts = check_num_tracks(num_tracks, coords0.shape[0], coords0.shape[1])
             self.num_tracks = torch.tensor(counts, dtype=torch.int32).to(coords0.device)
+        self.num_frames = None
+        if num_frames is not None:
+            from .utils import check_num_tracks
+
+            frames = check_num_tracks(num_frames, coords0.shape[0], p.S)
+            self.num_frames = torch.tensor(frames, dtype=torch.int32).to(coords0.device)
 
     def tokens(self, coords: torch.Tensor, track_feats: torch.Tensor, out: Optional[torch.Tensor] = None):
         """coords (B,S,N,2), track_feats (B,S,N,latent) (any outer strides) -> (B,N,S,D_tok) float32."""
@@ -123,13 +130,16 @@ class TrackTokenizer:
         else:
             assert out.shape == (B, N, S, self.tdim) and out.is_contiguous() and out.dtype == torch.float32
         with torch.cuda.device(c.device):
-            nt = self.num_tracks
+            nt, nf = self.num_tracks, self.num_frames
             if B * S * N and _use_tc(p, t, self.radius, self.padding_mode):
                 head = (p.split.data_ptr(), t.data_ptr(), t.stride(0), t.stride(1), t.stride(2),
                         c.data_ptr(), c.stride(0), c.stride(1), c.stride(2), self.pos.data_ptr(), out.data_ptr())
                 tail = (B, S, N, p.C, p.H, p.W, p.num_levels, self.radius, pad_mode(self.padding_mode), prec_mode(),
                         self.tdim, _tc_workspace(p, N).data_ptr(), stream_ptr(c.device))
-                if nt is None:
+                if nf is not None:
+                    _lib.check(lib.comet_tc_track_tokens_varlen_f32(*head, None if nt is None else nt.data_ptr(),
+                                                                    nf.data_ptr(), *tail))
+                elif nt is None:
                     _lib.check(lib.comet_tc_track_tokens_f32(*head, *tail))
                 else:
                     _lib.check(lib.comet_tc_track_tokens_ragged_f32(*head, nt.data_ptr(), *tail))
@@ -138,7 +148,10 @@ class TrackTokenizer:
                     c.data_ptr(), c.stride(0), c.stride(1), c.stride(2), self.pos.data_ptr(), out.data_ptr())
             tail = (B, S, N, p.C, p.H, p.W, p.num_levels, self.radius, pad_mode(self.padding_mode), prec_mode(),
                     p.layout, self.tdim, stream_ptr(c.device))
-            if nt is None:
+            if nf is not None:
+                _lib.check(lib.comet_track_tokens_varlen_f32(*head, None if nt is None else nt.data_ptr(), nf.data_ptr(),
+                                                             *tail))
+            elif nt is None:
                 _lib.check(lib.comet_track_tokens_f32(*head, *tail))
             else:
                 _lib.check(lib.comet_track_tokens_ragged_f32(*head, nt.data_ptr(), *tail))

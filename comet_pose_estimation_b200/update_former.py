@@ -93,34 +93,45 @@ class EfficientUpdateFormer(nn.Module):
                 CrossAttnBlock(hidden_size, hidden_size, num_heads, mlp_ratio) for _ in range(space_depth))
             assert len(self.time_blocks) >= len(self.space_virtual2point_blocks)
 
-    def forward(self, input_tensor, mask=None, num_tracks=None):
+    def forward(self, input_tensor, mask=None, num_tracks=None, num_frames=None):
         """``num_tracks`` (B ints or a 1-D tensor): ``input_tensor`` is a padded batch (B, N_max, T, input_dim) of sequences
-        with ``num_tracks[b]`` tracks each.  Sequence b's rows get what the forward of ``input_tensor[b:b+1, :num_tracks[b]]``
-        alone returns; rows past its count are zeros."""
-        if num_tracks is not None:
-            assert mask is None, "num_tracks and mask cannot be combined"
+        with ``num_tracks[b]`` tracks each.  ``num_frames`` (likewise): sequence b has ``num_frames[b]`` of the T frames.
+        Sequence b's rows get what the forward of ``input_tensor[b:b+1, :num_tracks[b], :num_frames[b]]`` alone returns;
+        rows past its counts are zeros."""
+        ragged = num_tracks is not None or num_frames is not None
+        if ragged:
+            assert mask is None, "num_tracks / num_frames and mask cannot be combined"
             from .utils import check_num_tracks
 
-            counts = check_num_tracks(num_tracks, input_tensor.shape[0], input_tensor.shape[1])
+            B, N, T = input_tensor.shape[:3]
+            counts = None if num_tracks is None else check_num_tracks(num_tracks, B, N)
+            frames = None if num_frames is None else check_num_tracks(num_frames, B, T)
         if (USE_TC_KERNELS and mask is None and input_tensor.is_cuda and not torch.is_grad_enabled()):
             from . import update_former_tc as tc
 
-            if tc.supported(self, input_tensor) and (num_tracks is None or tc.ragged_supported(self)):
+            if tc.supported(self, input_tensor) and (not ragged or tc.ragged_supported(self)):
                 autocast = torch.is_autocast_enabled("cuda") and torch.get_autocast_dtype("cuda") == torch.bfloat16
-                if num_tracks is not None:
-                    dev_counts = torch.tensor(counts, dtype=torch.int32).to(input_tensor.device, non_blocking=True)
-                    return tc.forward_ragged(self, input_tensor.float(), 1 if autocast else 3, dev_counts)
+                if ragged:
+                    dev = input_tensor.device
+                    dev_counts = None if counts is None else torch.tensor(counts, dtype=torch.int32).to(dev, non_blocking=True)
+                    dev_frames = None if frames is None else torch.tensor(frames, dtype=torch.int32).to(dev, non_blocking=True)
+                    if dev_frames is None:
+                        return tc.forward_ragged(self, input_tensor.float(), 1 if autocast else 3, dev_counts)
+                    return tc.forward_ragged(self, input_tensor.float(), 1 if autocast else 3, dev_counts, dev_frames)
                 return tc.forward(self, input_tensor.float(), 1 if autocast else 3)
-        if num_tracks is not None:
-            return self._forward_ragged_torch(input_tensor, counts)
+        if ragged:
+            return self._forward_ragged_torch(input_tensor, counts, frames)
         return self._forward_torch(input_tensor, mask)
 
-    def _forward_ragged_torch(self, input_tensor, counts):
+    def _forward_ragged_torch(self, input_tensor, counts, frames=None):
         """The per-sequence definition of the ragged forward: each sequence alone, re-padded with zeros."""
-        outs = [self._forward_torch(input_tensor[b:b + 1, :n]) for b, n in enumerate(counts)]
-        out = outs[0].new_zeros((input_tensor.shape[0], input_tensor.shape[1]) + tuple(outs[0].shape[2:]))
-        for b, (o, n) in enumerate(zip(outs, counts)):
-            out[b, :n] = o[0]
+        B, N, T = input_tensor.shape[:3]
+        counts = [N] * B if counts is None else counts
+        frames = [T] * B if frames is None else frames
+        outs = [self._forward_torch(input_tensor[b:b + 1, :n, :s]) for b, (n, s) in enumerate(zip(counts, frames))]
+        out = outs[0].new_zeros((B, N, T) + tuple(outs[0].shape[3:]))
+        for b, (o, n, s) in enumerate(zip(outs, counts, frames)):
+            out[b, :n, :s] = o[0]
         return out
 
     def _forward_torch(self, input_tensor, mask=None):

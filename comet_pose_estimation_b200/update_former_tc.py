@@ -137,19 +137,22 @@ class _Run:
                                                   self.stream))
         return op
 
-    def attention_varlen(self, q, k, v, H: int, dh: int, step: int, items, q_off, q_len, k_off, k_len, lq, lk, group: int,
+    def attention_varlen(self, q, k, v, H: int, dh: int, step: int, items, q_off, q_len, k_off, k_len, lq, lk, group,
                          rows_out: int, D: int, zero: bool = False):
         """Every item of ``items`` in one call: item i's position j is row ``q_off[i] + j * step`` of q / of the output
-        and row ``k_off[i] + j * step`` of k / v (int32 device arrays); ``lq`` / ``lk`` bound the lengths.  ``zero``: the
-        output rows no item writes (padded queries) are zeros instead of unset."""
+        and row ``k_off[i] + j * step`` of k / v (int32 device arrays); ``lq`` / ``lk`` bound the lengths (0 skips an
+        item).  ``group``: the problem count that selects each item's kernel family, an int or ``(groups, lo, hi)`` with
+        ``groups`` an int32 device array of per-item counts in [lo, hi].  ``zero``: the output rows no item writes
+        (padded queries) are zeros instead of unset."""
         op = self.new_planes(rows_out, D)
         if zero:
             op.zero_()
         assert k.stride(0) == v.stride(0)
-        _lib.check(lib.comet_attention_varlen_planes_f32(
+        groups, glo, ghi = (None, group, group) if isinstance(group, int) else group
+        _lib.check(lib.comet_attention_varlen_grouped_planes_f32(
             q.data_ptr(), q.stride(0), step, k.data_ptr(), k.stride(0), step, v.data_ptr(), op.data_ptr(), op.stride(0),
             op.stride(1), self.np, items, H, dh, q_off.data_ptr(), q_len.data_ptr(), k_off.data_ptr(), k_len.data_ptr(),
-            lq[0], lq[1], lk[0], lk[1], group, self.stream))
+            lq[0], lq[1], lk[0], lk[1], None if groups is None else groups.data_ptr(), glo, ghi, self.stream))
         return op
 
     def mlp_tail(self, y: torch.Tensor, blk, out: torch.Tensor):
@@ -188,18 +191,19 @@ class _Run:
         self.mlp_tail(y, blk, out=x)
 
 
-    def self_block_varlen(self, x: torch.Tensor, blk, H: int, step: int, lay, group: int):
-        """``self_block`` on the virtual-track rows of every sequence at once (one attention problem per (sequence, frame))."""
+    def self_block_varlen(self, x: torch.Tensor, blk, H: int, step: int, items: int, off, length, lrange, group):
+        """``self_block`` over ``items`` sequences of rows at once: item i has ``length[i]`` positions at rows
+        ``off[i] + j * step`` (the virtual tracks of every (sequence, frame), or the frames of every track)."""
         rows, D = x.shape
         xn, xnp = self.layernorm(x, blk.norm1, want_f32=True)
         qkv, _ = self.linear(xnp, blk.attn.in_proj_weight, blk.attn.in_proj_bias)
-        ctx = self.attention_varlen(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], H, D // H, step, lay.items, lay.vir_off,
-                                    lay.vir_len, lay.vir_off, lay.vir_len, (lay.V, lay.V), (lay.V, lay.V), group, rows, D)
+        ctx = self.attention_varlen(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], H, D // H, step, items, off, length, off,
+                                    length, lrange, lrange, group, rows, D, zero=lrange[0] != lrange[1])
         y, _ = self.linear(ctx, blk.attn.out_proj.weight, blk.attn.out_proj.bias, resid=xn)
         self.mlp_tail(y, blk, out=x)
 
     def cross_block_varlen(self, x: torch.Tensor, ctxt: torch.Tensor, blk, H: int, step: int, items: int, q_off, q_len, k_off,
-                           k_len, lq, lk, group: int):
+                           k_len, lq, lk, group):
         """``cross_block`` of every sequence at once: item i attends from its rows of ``x`` to its rows of ``ctxt``."""
         rows, D = x.shape
         xn, xnp = self.layernorm(x, blk.norm1, want_f32=True)
@@ -221,15 +225,17 @@ _MAX_GRAPHS = 4
 
 
 class _Captured:
-    """``counts`` given: the ragged forward, captured for the capacity of ``x`` (B, N_cap, T, Din); the track counts are
-    read from a device buffer, so one graph serves every set of counts up to N_cap."""
+    """``counts`` given: the ragged forward, captured for the capacity of ``x`` (B, N_cap, T, Din); the track counts (and
+    ``frames``, the frame counts) are read from device buffers, so one graph serves every set of counts up to N_cap
+    (and T)."""
 
-    def __init__(self, m, x: torch.Tensor, np_: int, counts: torch.Tensor = None):
+    def __init__(self, m, x: torch.Tensor, np_: int, counts: torch.Tensor = None, frames: torch.Tensor = None):
         self.x = torch.empty_like(x)
         self.x.copy_(x)
         self.counts = None if counts is None else counts.clone()
+        self.frames = None if frames is None else frames.clone()
         run = (lambda: forward_eager(m, self.x, np_)) if counts is None else (
-            lambda: forward_ragged_eager(m, self.x, np_, self.counts))
+            lambda: forward_ragged_eager(m, self.x, np_, self.counts, self.frames))
         side = torch.cuda.Stream(device=x.device)
         side.wait_stream(torch.cuda.current_stream(x.device))
         with torch.cuda.stream(side):                      # warm-up: weight planes, kernel attributes, allocator
@@ -239,7 +245,7 @@ class _Captured:
         with torch.cuda.graph(self.graph):
             self.out = run()
 
-    def __call__(self, x: torch.Tensor, counts: torch.Tensor = None) -> torch.Tensor:
+    def __call__(self, x: torch.Tensor, counts: torch.Tensor = None, frames: torch.Tensor = None) -> torch.Tensor:
         if counts is None:
             self.x.copy_(x, non_blocking=True)
         else:
@@ -247,6 +253,8 @@ class _Captured:
             self.x[:, :n].copy_(x, non_blocking=True)
             self.x[:, n:].zero_()
             self.counts.copy_(counts, non_blocking=True)
+            if frames is not None:
+                self.frames.copy_(frames, non_blocking=True)
         self.graph.replay()
         if counts is None:
             return self.out.clone()
@@ -284,19 +292,25 @@ def ragged_supported(m) -> bool:
     return not m.add_space_attn or m.num_virtual_tracks > 32
 
 
-def forward_ragged(m, x: torch.Tensor, np_: int, counts: torch.Tensor) -> torch.Tensor:
+def forward_ragged(m, x: torch.Tensor, np_: int, counts: torch.Tensor, frames: torch.Tensor = None) -> torch.Tensor:
     """``EfficientUpdateFormer.forward`` of B sequences at once: tokens ``x`` (B, N_max, T, input_dim), ``counts`` (B,)
     int32 on the device (1 <= counts[b] <= N_max).  Sequence b's rows n < counts[b] get what the forward of that
-    sequence alone gives; its rows n >= counts[b] are zeros."""
+    sequence alone gives; its rows n >= counts[b] are zeros.  ``frames`` (B,) int32 on the device (1 <= frames[b] <= T),
+    or None: sequence b has frames[b] frames, and its rows of frames t >= frames[b] are zeros too.  ``counts=None`` with
+    ``frames``: every sequence has N_max tracks (no track padding is added)."""
     B, N, T, Din = x.shape
-    ncap = (N + RAGGED_TRACK_QUANTUM - 1) // RAGGED_TRACK_QUANTUM * RAGGED_TRACK_QUANTUM
+    if counts is None:
+        counts = torch.full((B,), N, dtype=torch.int32, device=x.device)
+        ncap = N
+    else:
+        ncap = (N + RAGGED_TRACK_QUANTUM - 1) // RAGGED_TRACK_QUANTUM * RAGGED_TRACK_QUANTUM
     if not USE_CUDA_GRAPH or torch.cuda.is_current_stream_capturing():
         xp = x.new_zeros((B, ncap, T, Din))
         xp[:, :N] = x
-        return forward_ragged_eager(m, xp, np_, counts)[:, :N]
+        return forward_ragged_eager(m, xp, np_, counts, frames)[:, :N]
     if not hasattr(m, "_tc_graphs"):
         m._tc_graphs = {}
-    key = ("ragged", B, ncap, T, Din, np_, str(x.device), _weights_tag(m))
+    key = ("ragged", B, ncap, T, Din, np_, str(x.device), _weights_tag(m)) + (() if frames is None else ("frames",))
     g = m._tc_graphs.get(key)
     if g is None:
         while len(m._tc_graphs) >= _MAX_GRAPHS:
@@ -304,16 +318,23 @@ def forward_ragged(m, x: torch.Tensor, np_: int, counts: torch.Tensor) -> torch.
         xp = x.new_zeros((B, ncap, T, Din))
         xp[:, :N] = x
         with torch.cuda.device(x.device):
-            g = m._tc_graphs[key] = _Captured(m, xp, np_, counts)
+            g = m._tc_graphs[key] = _Captured(m, xp, np_, counts, frames)
         m._tc_captures = getattr(m, "_tc_captures", 0) + 1
-    return g(x, counts)
+    return g(x, counts, frames)
 
 
 class _RaggedLayout:
     """Device index arrays of the space attention over B sequences: item i = (sequence b, frame t) = b * T + t.  Point
-    rows are (b, n, t) -> (b * N_cap + n) * T + t, virtual rows (b, v, t) -> (b * V + v) * T + t of their own block."""
+    rows are (b, n, t) -> (b * N_cap + n) * T + t, virtual rows (b, v, t) -> (b * V + v) * T + t of their own block.
 
-    def __init__(self, counts: torch.Tensor, B: int, ncap: int, V: int, T: int):
+    ``space_group``: the problem count that picks each space item's kernel family, the frame count of the single call.
+
+    With ``frames`` (frame counts), the space items of frames t >= frames[b] have length 0 and choose their family for
+    frames[b] problems, and the time attention is varlen too: item k = track k of the (points, then virtual tracks) row
+    order, rows k * T + t for t < frames of its sequence; its kernel family is chosen for the problem count
+    counts[b] + V of the single-sequence call."""
+
+    def __init__(self, counts: torch.Tensor, B: int, ncap: int, V: int, T: int, frames: torch.Tensor = None):
         dev = counts.device
         b = torch.arange(B, device=dev, dtype=torch.int32).repeat_interleave(T)
         t = torch.arange(T, device=dev, dtype=torch.int32).repeat(B)
@@ -322,9 +343,26 @@ class _RaggedLayout:
         self.vir_off = (b * (V * T) + t).contiguous()
         self.pts_len = counts.to(torch.int32).repeat_interleave(T).contiguous()
         self.vir_len = torch.full((B * T,), V, dtype=torch.int32, device=dev)
+        self.vir_lq = (V, V)
+        self.pts_lq = (1, ncap)
+        self.space_group = T
+        if frames is not None:
+            live = (t < frames.to(torch.int32).repeat_interleave(T)).to(torch.int32)
+            self.pts_len = (self.pts_len * live).contiguous()
+            self.vir_len = (self.vir_len * live).contiguous()
+            self.vir_lq = (0, V)
+            self.pts_lq = (0, ncap)
+            self.space_group = (frames.to(torch.int32).repeat_interleave(T).contiguous(), 1, T)
+            seq = torch.cat([torch.arange(B, device=dev, dtype=torch.int32).repeat_interleave(ncap),
+                             torch.arange(B, device=dev, dtype=torch.int32).repeat_interleave(V)])
+            self.tracks = B * (ncap + V)
+            self.trk_off = (torch.arange(self.tracks, device=dev, dtype=torch.int32) * T).contiguous()
+            self.trk_len = frames.to(torch.int32)[seq].contiguous()
+            self.trk_group = (counts.to(torch.int32)[seq] + V).contiguous()
+            self.trk_grange = (1 + V, ncap + V)
 
 
-def forward_ragged_eager(m, x: torch.Tensor, np_: int, counts: torch.Tensor) -> torch.Tensor:
+def forward_ragged_eager(m, x: torch.Tensor, np_: int, counts: torch.Tensor, frames: torch.Tensor = None) -> torch.Tensor:
     """Ragged forward for x (B, N_cap, T, input_dim).  Tokens are laid out as all sequences' point rows followed by all
     sequences' virtual rows, so every LayerNorm and GEMM of a block is one launch over all sequences and the space
     attention is one varlen launch per kernel family.  Padded point rows are never keys or queries of the space
@@ -344,17 +382,22 @@ def forward_ragged_eager(m, x: torch.Tensor, np_: int, counts: torch.Tensor) -> 
         pts, vir = flat[:P], flat[P:]
         if V:
             vir.view(B, V, T, D)[:] = m.virual_tracks                                        # (1, V, 1, D) broadcast
-            lay = _RaggedLayout(counts, B, Nc, V, T)
+        lay = _RaggedLayout(counts, B, Nc, V, T, frames) if V or frames is not None else None
         every = len(m.time_blocks) // len(m.space_virtual_blocks) if V else 0
         j = 0
         for i, tb in enumerate(m.time_blocks):
-            run.self_block(flat, tb, B * (Nc + V), T, T, 1, H)                               # time attention per track
+            if frames is None:
+                run.self_block(flat, tb, B * (Nc + V), T, T, 1, H)                           # time attention per track
+            else:
+                run.self_block_varlen(flat, tb, H, 1, lay.tracks, lay.trk_off, lay.trk_len, (1, T),
+                                      (lay.trk_group, *lay.trk_grange))
             if V and i % every == 0:
                 run.cross_block_varlen(vir, pts, m.space_virtual2point_blocks[j], H, T, lay.items, lay.vir_off, lay.vir_len,
-                                       lay.pts_off, lay.pts_len, (V, V), (1, Nc), T)
-                run.self_block_varlen(vir, m.space_virtual_blocks[j], H, T, lay, T)
+                                       lay.pts_off, lay.pts_len, lay.vir_lq, lay.pts_lq, lay.space_group)
+                run.self_block_varlen(vir, m.space_virtual_blocks[j], H, T, lay.items, lay.vir_off, lay.vir_len, lay.vir_lq,
+                                      lay.space_group)
                 run.cross_block_varlen(pts, vir, m.space_point2virtual_blocks[j], H, T, lay.items, lay.pts_off, lay.pts_len,
-                                       lay.vir_off, lay.vir_len, (1, Nc), (V, V), T)
+                                       lay.vir_off, lay.vir_len, lay.pts_lq, lay.vir_lq, lay.space_group)
                 j += 1
         sp = run.new_planes(P, D)
         _lib.check(lib.comet_add_planes_f32(pts.data_ptr(), skip.data_ptr(), sp.data_ptr(), sp.stride(0), np_, P * D,
@@ -362,7 +405,10 @@ def forward_ragged_eager(m, x: torch.Tensor, np_: int, counts: torch.Tensor) -> 
         out, _ = run.linear(sp, m.flow_head.weight, m.flow_head.bias)
         out = out.view(B, Nc, T, -1)
         real = torch.arange(Nc, device=x.device)[None, :] < counts[:, None]
-        return out.masked_fill_(~real[:, :, None, None], 0.0)
+        if frames is None:
+            return out.masked_fill_(~real[:, :, None, None], 0.0)
+        live = torch.arange(T, device=x.device)[None, :] < frames[:, None]                    # (B, T)
+        return out.masked_fill_(~(real[:, :, None] & live[:, None, :])[..., None], 0.0)
 
 
 def forward_eager(m, x: torch.Tensor, np_: int) -> torch.Tensor:

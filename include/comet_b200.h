@@ -156,6 +156,15 @@ int comet_track_tokens_ragged_f32(const float* fmaps, const float* pyr, const fl
                                   long long c_sn, const float* pos_emb, float* tokens, const int* num_tracks, int B, int S,
                                   int N, int C, int H, int W, int L, int r, int pad_mode, int prec_mode, int pyr_layout,
                                   int D_tok, comet_stream_t stream);
+/* The same with per-sequence track counts and / or frame counts (num_tracks, num_frames: (B,) int32 in DEVICE memory, each
+ * nullable).  Rows of frames s >= num_frames[b] are written as zeros and read nothing; every other row equals
+ * comet_track_tokens_f32 on sequence b alone.  Frame counts are also served for COMET_PYR_UP2_SOURCE (track counts are
+ * not); neither is served for the other C == 32 layouts. */
+int comet_track_tokens_varlen_f32(const float* fmaps, const float* pyr, const float* track_feats, long long t_sb,
+                                  long long t_ss, long long t_sn, const float* coords, long long c_sb, long long c_ss,
+                                  long long c_sn, const float* pos_emb, float* tokens, const int* num_tracks,
+                                  const int* num_frames, int B, int S, int N, int C, int H, int W, int L, int r, int pad_mode,
+                                  int prec_mode, int pyr_layout, int D_tok, comet_stream_t stream);
 
 /* sampled_pos_emb = sample_features4d(get_2d_sincos_pos_embed(D,(H,W)), coords[:,0])
  * (base_track_predictor.py:200-208; utils.py:724-755, :942-974): the float64 table is evaluated on the fly at
@@ -234,6 +243,11 @@ int comet_shallow_encoder_from_images_f32(const float* images, const int* toplef
 int comet_shallow_encoder_from_images_ragged_f32(const float* images, const int* topleft, const int* seq_of_track,
                                                  const float* packed, float* out, int P, int B, int S, int H, int W,
                                                  float eps, comet_stream_t stream);
+/* The same for sequences with different frame counts: num_frames (B,) int32 in device memory, or NULL (= the call above).
+ * The pixels of frames s >= num_frames[seq_of_track[p]] are never read, and their maps are written as zeros. */
+int comet_shallow_encoder_from_images_varlen_f32(const float* images, const int* topleft, const int* seq_of_track,
+                                                 const int* num_frames, const float* packed, float* out, int P, int B, int S,
+                                                 int H, int W, float eps, comet_stream_t stream);
 
 /* ---- sin/cos encodings: comet/models/utils.py:37-101, :724-832 ----------- */
 /* get_2d_embedding(xy, C, cat_coords): xy (M,2) contiguous -> out (M, 2*C [+2 in front if cat_coords]). */
@@ -274,6 +288,13 @@ int comet_tc_track_tokens_ragged_f32(const void* split, const float* track_feats
                                      const float* pos_emb, float* tokens, const int* num_tracks, int B, int S, int N, int C,
                                      int H, int W, int L, int r, int pad_mode, int prec_mode, int D_tok, void* workspace,
                                      comet_stream_t stream);
+/* The same with per-sequence track counts and / or frame counts (each nullable, device memory).  A padded frame sorts no
+ * query, so each of its tiles is an empty one-row job, and the pre-kernel writes its token rows as zeros. */
+int comet_tc_track_tokens_varlen_f32(const void* split, const float* track_feats, long long t_sb, long long t_ss,
+                                     long long t_sn, const float* coords, long long c_sb, long long c_ss, long long c_sn,
+                                     const float* pos_emb, float* tokens, const int* num_tracks, const int* num_frames,
+                                     int B, int S, int N, int C, int H, int W, int L, int r, int pad_mode, int prec_mode,
+                                     int D_tok, void* workspace, comet_stream_t stream);
 /* vols: HOST array of L device pointers, level l = (B*S, N, H_l*W_l) float32. */
 int comet_tc_corr_volume_f32(const void* split, const float* targets, long long t_sb, long long t_ss, long long t_sn,
                              float* const* vols, int B, int S, int N, int C, int H, int W, int L, int prec_mode,
@@ -314,12 +335,23 @@ int comet_attention_planes_f32(const float* q, long long q_sb, long long q_si, c
  * value position j is row k_off[i] + j*k_step of k and v (row pitch k_ld), with q_len[i] / k_len[i] positions.  The four
  * int32 arrays live in DEVICE memory; every length must lie in [min_lq, max_lq] / [min_lk, max_lk].  Item i gets exactly
  * the arithmetic comet_attention_planes_f32 uses for (Lq, Lk, dh, np) with B = group problems of that shape (same kernel
- * family, same key split).  Items with at most 32 queries AND at most 32 keys are not served. */
+ * family, same key split).  min_lq / min_lk must be at least 1. */
 int comet_attention_varlen_planes_f32(const float* q, long long q_ld, long long q_step, const float* k, long long k_ld,
                                       long long k_step, const float* v, void* out_planes, long long o_plane_stride,
                                       long long o_ld, int np, int items, int H, int dh, const int* q_off, const int* q_len,
                                       const int* k_off, const int* k_len, int min_lq, int max_lq, int min_lk, int max_lk,
                                       int group, comet_stream_t stream);
+/* The same with lengths that may be 0 (the item is skipped and its output rows are not written) and a per-item problem
+ * count: item i's kernel family is the one comet_attention_planes_f32 uses with B = groups[i] (int32, device memory, each
+ * in [min_group, max_group]); groups NULL: B = max_group (= min_group) for every item.  The time attention of sequences
+ * with different frame counts is one such call: item = track, length = its sequence's frame count, group = that
+ * sequence's track count plus the virtual tracks. */
+int comet_attention_varlen_grouped_planes_f32(const float* q, long long q_ld, long long q_step, const float* k, long long k_ld,
+                                              long long k_step, const float* v, void* out_planes, long long o_plane_stride,
+                                              long long o_ld, int np, int items, int H, int dh, const int* q_off,
+                                              const int* q_len, const int* k_off, const int* k_len, int min_lq, int max_lq,
+                                              int min_lk, int max_lk, const int* groups, int min_group, int max_group,
+                                              comet_stream_t stream);
 /* planes of a + b (contiguous float32 vectors of n elements): `tokens + init_tokens` before the flow head (blocks.py:344). */
 int comet_add_planes_f32(const float* a, const float* b, void* planes, long long plane_stride, int np, long long n,
                          comet_stream_t stream);
