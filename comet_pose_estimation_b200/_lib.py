@@ -45,6 +45,8 @@ SIGNATURES = {
                                            _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p]),
     "comet_track_tokens_varlen_f32": (_i, [_p, _p, _p, _ll, _ll, _ll, _p, _ll, _ll, _ll, _p, _p, _p, _p,
                                            _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p]),
+    "comet_track_tokens_indexed_f32": (_i, [_p, _p, _p, _ll, _ll, _ll, _p, _ll, _ll, _ll, _p, _p, _p, _p, _p, _i,
+                                            _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p]),
     "comet_sampled_pos_emb_f32": (_i, [_p, _ll, _ll, _p, _i, _i, _i, _i, _i, _p]),
     "comet_bilinear_sampler4d_f32": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p]),
     "comet_bilinear_sampler5d_f32": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p]),
@@ -61,6 +63,8 @@ SIGNATURES = {
     "comet_shallow_encoder_from_images_f32": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, C.c_float, _p]),
     "comet_shallow_encoder_from_images_ragged_f32": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, C.c_float, _p]),
     "comet_shallow_encoder_from_images_varlen_f32": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, C.c_float, _p]),
+    "comet_shallow_encoder_from_images_indexed_f32": (_i, [_p, _p, _p, _p, _p, _i, _p, _p, _i, _i, _i, _i, _i, C.c_float,
+                                                           _p]),
     "comet_embed2d_f32": (_i, [_p, _p, _ll, _i, _i, _p]),
     "comet_sincos1d_from_grid_f32": (_i, [_p, _p, _ll, _i, _p]),
     "comet_sincos2d_f32": (_i, [_p, _i, _i, _i, _p]),
@@ -76,6 +80,8 @@ SIGNATURES = {
                                               _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p]),
     "comet_tc_track_tokens_varlen_f32": (_i, [_p, _p, _ll, _ll, _ll, _p, _ll, _ll, _ll, _p, _p, _p, _p,
                                               _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p]),
+    "comet_tc_track_tokens_indexed_f32": (_i, [_p, _p, _ll, _ll, _ll, _p, _ll, _ll, _ll, _p, _p, _p, _p, _p, _i,
+                                               _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p]),
     "comet_tc_corr_volume_f32": (_i, [_p, _p, _ll, _ll, _ll, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p]),
     "comet_tc_status": (_i, []),
     "comet_split_planes_f32": (_i, [_p, _ll, _p, _ll, _ll, _ll, _i, _i, _p]),

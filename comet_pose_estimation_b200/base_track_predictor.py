@@ -47,18 +47,35 @@ class BaseTrackerPredictor(nn.Module):
             self.vis_predictor = nn.Sequential(nn.Linear(latent_dim, 1))
 
     def forward(self, query_points, fmaps=None, iters=4, return_feat=False, down_ratio=1, is_train=False,
-                track_feats=None, TRACKorPOSE=True, ind=0, num_tracks=None, num_frames=None):
+                track_feats=None, TRACKorPOSE=True, ind=0, num_tracks=None, num_frames=None, frame_index=None):
         """``num_tracks`` (B ints or a 1-D tensor, ``TRACKorPOSE=False`` only): ``query_points`` (B, N_max, 2) is a padded
         batch of sequences with different track counts.  Sequence b's tracks get what a call on that sequence alone
         computes (up to rounding); every output entry of a padded track (n >= num_tracks[b]) is 0.  ``num_frames``
         (likewise): sequence b has the first ``num_frames[b]`` of the S frames of ``fmaps``; every output entry of a padded
-        frame is 0, and the tracks of padded frames start at 0 and receive zero updates."""
+        frame is 0, and the tracks of padded frames start at 0 and receive zero updates.
+
+        ``frame_index`` ((B', S) integer tensor, ``TRACKorPOSE=False`` only): ``fmaps`` (B_src, S, C, H, W) holds source
+        frames and ``query_points`` (B', N_max, 2) a batch of B' items; item i sees source frame ``frame_index[i, s]``
+        (flat index into the B_src * S frames) at position s.  The result is the forward on the gathered maps
+        ``fmaps.flatten(0, 1)[frame_index]``: on the GPU the pyramid is prepared once over the source frames and the token
+        kernels read it through the table; elsewhere the gathered maps are built and the ordinary path runs."""
+        if frame_index is not None:
+            assert not TRACKorPOSE, "frame_index is served with TRACKorPOSE=False only"
+            assert isinstance(fmaps, torch.Tensor) and fmaps.dim() == 5, "frame_index needs fmaps (B_src, S, C, H, W)"
+            assert frame_index.dim() == 2 and frame_index.shape == (query_points.shape[0], fmaps.shape[1]), \
+                f"frame_index must be (B', S) = ({query_points.shape[0]}, {fmaps.shape[1]}), got {tuple(frame_index.shape)}"
+            if not fmaps.is_cuda:
+                gathered = fmaps.flatten(0, 1)[frame_index.long()].reshape((-1,) + tuple(fmaps.shape[1:]))
+                return self.forward(query_points, gathered, iters, return_feat, down_ratio, is_train, track_feats,
+                                    TRACKorPOSE, ind, num_tracks, num_frames)
+            frame_index = frame_index.to(fmaps.device)
         counts = frames = None
+        B_items = query_points.shape[0] if frame_index is not None else fmaps.shape[0]
         if num_frames is not None:
             assert not TRACKorPOSE, "num_frames is served with TRACKorPOSE=False only"
             from .utils import check_num_tracks
 
-            frames = check_num_tracks(num_frames, fmaps.shape[0], fmaps.shape[1])
+            frames = check_num_tracks(num_frames, B_items, fmaps.shape[1])
             live = torch.arange(fmaps.shape[1], device=query_points.device)[None, :] < torch.tensor(
                 frames, device=query_points.device)[:, None]                                  # (B, S)
         if num_tracks is not None:
@@ -73,7 +90,9 @@ class BaseTrackerPredictor(nn.Module):
             B, S, N, D = query_points.shape
         else:
             B, N, D = query_points.shape
-        B, S, C, HH, WW = fmaps.shape
+        _, S, C, HH, WW = fmaps.shape
+        if frame_index is None:
+            B = fmaps.shape[0]
         assert D == 2
         if down_ratio > 1:  # guards BOTH divisions (SURVEY A.6 i)
             query_points = query_points / float(down_ratio)
@@ -85,7 +104,10 @@ class BaseTrackerPredictor(nn.Module):
         if frames is not None:
             coords = coords * live[:, :, None, None]
 
-        if isinstance(fmaps, Upsampled2x):
+        if frame_index is not None:
+            # each item's position-0 map: a gather of B' maps (the same values the gathered copy would hold)
+            query_track_feat = sample_features4d(fmaps.flatten(0, 1)[frame_index[:, 0].long()], coords[:, 0])
+        elif isinstance(fmaps, Upsampled2x):
             # bilinear sample (border) of the 2x-1 up-sampling at p == bilinear sample of its source at p / 2
             query_track_feat = sample_features4d(fmaps.src[:, 0], coords[:, 0] * 0.5)
         else:
@@ -98,7 +120,8 @@ class BaseTrackerPredictor(nn.Module):
         else:
             fcorr_fn = CorrBlock(fmaps, num_levels=self.corr_levels, radius=self.corr_radius)
         # sampled_pos_emb depends on coords[:, 0] only, which the loop pins -> computed once, not per iteration
-        tokenizer = TrackTokenizer(fcorr_fn, coords[:, 0], self.transformer_dim, num_tracks=counts, num_frames=frames)
+        tokenizer = TrackTokenizer(fcorr_fn, coords[:, 0], self.transformer_dim, num_tracks=counts, num_frames=frames,
+                                   frame_index=frame_index)
 
         coord_preds = []
         for _ in range(iters):

@@ -164,10 +164,11 @@ def _make_pyramid(fmaps, num_levels: int, radius: int, padding_mode: str):
     return _Pyramid(fmaps, num_levels)
 
 
-def _tc_workspace(pyr: "_Pyramid", N: int) -> torch.Tensor:
+def _tc_workspace(pyr: "_Pyramid", N: int, BS: Optional[int] = None) -> torch.Tensor:
     """Scratch of the tensor path, one buffer per CUDA stream (two streams driving the same CorrBlock never share a
-    plan).  It grows only when a larger N arrives: under CUDA-graph capture call once with the largest N first."""
-    need = lib.comet_tc_workspace_bytes(pyr.B * pyr.S, N)
+    plan).  It grows only when a larger N arrives: under CUDA-graph capture call once with the largest N first.  ``BS``:
+    the (item, position) frames of the call when they differ from the pyramid's (a frame table)."""
+    need = lib.comet_tc_workspace_bytes(pyr.B * pyr.S if BS is None else BS, N)
     key = stream_ptr(pyr.fmaps0.device)
     ws = pyr._ws.get(key)
     if ws is None or ws.numel() * 4 < need:

@@ -43,7 +43,8 @@ __global__ void __launch_bounds__(256) corr_lookup_kernel(const LookupParams p) 
   const int n = (int)(q % p.N);
   const int s = (int)((q / p.N) % p.S);
   const int b = (int)(q / ((long long)p.N * p.S));
-  const long long bs = (long long)b * p.S + s;
+  long long bs = (long long)b * p.S + s;
+  if (TOKENS && p.fidx) bs = min(max(__ldg(p.fidx + bs), 0), p.BS_src - 1);   // the frame this (item, position) reads
   if (TOKENS && ((p.ntr && n >= __ldg(p.ntr + b)) || (p.nfr && s >= __ldg(p.nfr + b)))) {   // padded query / frame: zero row
     float* zp = p.out + (((long long)b * p.N + n) * p.S + s) * p.D_tok;
     for (int d = lane; d < p.D_tok; d += 32) zp[d] = 0.f;
@@ -201,7 +202,8 @@ __global__ void __launch_bounds__(256, 2) corr_lookup_c32_kernel(const LookupPar
   const int n = (int)(q % p.N);
   const int s = (int)((q / p.N) % p.S);
   const int b = (int)(q / ((long long)p.N * p.S));
-  const long long bs = (long long)b * p.S + s;
+  long long bs = (long long)b * p.S + s;
+  if (TOKENS && p.fidx) bs = min(max(__ldg(p.fidx + bs), 0), p.BS_src - 1);   // the frame this (item, position) reads
 
   const float* cp = p.coords + b * p.c_sb + s * p.c_ss + n * p.c_sn;
   const float cx = __ldg(cp), cy = __ldg(cp + 1);
@@ -384,7 +386,8 @@ __global__ void __launch_bounds__(256, 1) corr_lookup_c32_tma_kernel(const __gri
     const int n = (int)(q % p.N);
     const int s = (int)((q / p.N) % p.S);
     const int b = (int)(q / ((long long)p.N * p.S));
-    const int bs = b * p.S + s;
+    int bs = b * p.S + s;
+    if (TOKENS && p.fidx) bs = min(max(__ldg(p.fidx + bs), 0), p.BS_src - 1);
     AxisWindow ax[3], ay[3];
 #pragma unroll
     for (int l = 0; l < 3; ++l) {
@@ -608,7 +611,7 @@ static int launch_lookup(const LookupParams& p, cudaStream_t stream) {
       const int G2 = 2 * p.r + 2;
       for (int l = p.cl0 ? 0 : 1; l < p.L; ++l) {
         const float* base = l == 0 ? p.fmaps : p.pyr + p.lvlOff[l];
-        int rc = encode_level_map(&maps.m[l], base, p.B * p.S, p.lvlH[l], p.lvlW[l], G2);
+        int rc = encode_level_map(&maps.m[l], base, p.fidx ? p.BS_src : p.B * p.S, p.lvlH[l], p.lvlW[l], G2);
         if (rc != COMET_OK) return rc;
       }
       const int sms = device_sm_count_if_sm100();
@@ -704,9 +707,9 @@ extern "C" int comet_corr_lookup_f32(const float* fmaps, const float* pyr, const
 
 static int track_tokens(const float* fmaps, const float* pyr, const float* track_feats, long long t_sb, long long t_ss,
                         long long t_sn, const float* coords, long long c_sb, long long c_ss, long long c_sn,
-                        const float* pos_emb, float* tokens, const int* num_tracks, const int* num_frames, int B, int S, int N,
-                        int C, int H, int W, int L, int r, int pad_mode, int prec_mode, int pyr_layout, int D_tok,
-                        comet_stream_t stream) {
+                        const float* pos_emb, float* tokens, const int* num_tracks, const int* num_frames,
+                        const int* frame_index, int BS_src, int B, int S, int N, int C, int H, int W, int L, int r,
+                        int pad_mode, int prec_mode, int pyr_layout, int D_tok, comet_stream_t stream) {
   LookupParams p{};
   int rc = fill_params(p, fmaps, pyr, track_feats, t_sb, t_ss, t_sn, 0, coords, c_sb, c_ss, c_sn, B, S, N, C, H, W,
                        L, r, pad_mode, prec_mode, pyr_layout);
@@ -716,8 +719,16 @@ static int track_tokens(const float* fmaps, const float* pyr, const float* track
   COMET_REQUIRE(D_tok >= need, "D_tok=%d smaller than the %d token channels", D_tok, need);
   COMET_REQUIRE((long long)B * S * N == 0 || (tokens && pos_emb), "null tokens / pos_emb pointer");
   p.out = tokens; p.pos = pos_emb; p.D_tok = D_tok; p.ntr = num_tracks; p.nfr = num_frames;
+  if (frame_index) {
+    // the pyramid holds BS_src frames: its level offsets follow from that count, not from B * S
+    COMET_REQUIRE(BS_src >= 1, "BS_src must be positive with a frame table (got %d)", BS_src);
+    Levels lv = make_levels(BS_src, C, H, W, L);
+    for (int l = 0; l < L; ++l) p.lvlOff[l] = lv.off[l];
+    p.fidx = frame_index; p.BS_src = BS_src;
+  }
   if (pyr_layout == COMET_PYR_UP2_SOURCE) {
     COMET_REQUIRE(!num_tracks, "per-sequence query counts are not served by COMET_PYR_UP2_SOURCE");
+    COMET_REQUIRE(!frame_index, "frame tables are not served by COMET_PYR_UP2_SOURCE");
     rc = up2_supported(C, H, W, L, r, pad_mode);
     if (rc != COMET_OK) return rc;
     return launch_lookup_up2<true>(p, fmaps, pyr, (cudaStream_t)stream);
@@ -730,8 +741,8 @@ extern "C" int comet_track_tokens_f32(const float* fmaps, const float* pyr, cons
                                       long long c_ss, long long c_sn, const float* pos_emb, float* tokens, int B,
                                       int S, int N, int C, int H, int W, int L, int r, int pad_mode, int prec_mode,
                                       int pyr_layout, int D_tok, comet_stream_t stream) {
-  return track_tokens(fmaps, pyr, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, nullptr, nullptr, B,
-                      S, N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok, stream);
+  return track_tokens(fmaps, pyr, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, nullptr, nullptr, nullptr,
+                      B * S, B, S, N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok, stream);
 }
 
 extern "C" int comet_track_tokens_ragged_f32(const float* fmaps, const float* pyr, const float* track_feats, long long t_sb,
@@ -741,7 +752,7 @@ extern "C" int comet_track_tokens_ragged_f32(const float* fmaps, const float* py
                                              int pad_mode, int prec_mode, int pyr_layout, int D_tok, comet_stream_t stream) {
   COMET_REQUIRE((long long)B * S * N == 0 || num_tracks, "null num_tracks");
   return track_tokens(fmaps, pyr, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks, nullptr,
-                      B, S, N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok, stream);
+                      nullptr, B * S, B, S, N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok, stream);
 }
 
 extern "C" int comet_track_tokens_varlen_f32(const float* fmaps, const float* pyr, const float* track_feats, long long t_sb,
@@ -751,5 +762,16 @@ extern "C" int comet_track_tokens_varlen_f32(const float* fmaps, const float* py
                                              int W, int L, int r, int pad_mode, int prec_mode, int pyr_layout, int D_tok,
                                              comet_stream_t stream) {
   return track_tokens(fmaps, pyr, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks,
-                      num_frames, B, S, N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok, stream);
+                      num_frames, nullptr, B * S, B, S, N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok, stream);
+}
+
+extern "C" int comet_track_tokens_indexed_f32(const float* fmaps, const float* pyr, const float* track_feats, long long t_sb,
+                                              long long t_ss, long long t_sn, const float* coords, long long c_sb,
+                                              long long c_ss, long long c_sn, const float* pos_emb, float* tokens,
+                                              const int* num_tracks, const int* num_frames, const int* frame_index, int BS_src,
+                                              int B, int S, int N, int C, int H, int W, int L, int r, int pad_mode,
+                                              int prec_mode, int pyr_layout, int D_tok, comet_stream_t stream) {
+  return track_tokens(fmaps, pyr, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks,
+                      num_frames, frame_index, BS_src, B, S, N, C, H, W, L, r, pad_mode, prec_mode, pyr_layout, D_tok,
+                      stream);
 }

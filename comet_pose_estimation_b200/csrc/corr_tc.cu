@@ -115,7 +115,8 @@ struct __align__(16) JobRec {
   int mnf;            // query tile (bits 0-15) | number of runs (16-23) | flags (24-31)
   uint32_t t0p, t1p;  // run i: first tile / one past the last tile in byte i (global tile numbering of tile_info, < 256)
   int own_lo, own_hi; // level-0 jobs: the window rows ("tops") whose output this job writes
-  int pad0, pad1;
+  int src;            // frame of the packed pyramid the job's tiles are read from (== bs without a frame table)
+  int pad1;
   __host__ __device__ int mt() const { return mnf & 0xffff; }
   __host__ __device__ int nseg() const { return (mnf >> 16) & 0xff; }
   __host__ __device__ int flags() const { return (mnf >> 24) & 0xff; }
@@ -139,6 +140,8 @@ struct Params {
   int red;                                            // tokens: windows are ADDED to the rows (MODE_REDUCE); tc_pre_kernel writes pos_emb there
   const int* ntr;                                     // tokens: (B,) query count of each sequence (queries n >= ntr[b] are padding), or null
   const int* nfr;                                     // tokens: (B,) frame count of each sequence (frames s >= nfr[b] are padding), or null
+  const int* fidx;                                    // tokens: (B,S) packed-pyramid frame of each (item, position), or null (identity)
+  int BS_src;                                         // frames of the packed pyramid (fidx entries are clamped to [0, BS_src))
   float* vol[5]; int volume_mode;                      // volume mode: per-level (BS,N,H_l,W_l)
   int B, S, N, L, r, npass, bf16;
   int BS, mtiles, npad, nsplit, npyr, nchunk, njobs;
@@ -343,7 +346,7 @@ __device__ __forceinline__ JobRec load_job(const Params& p, int job) {
     d[0] = ldg_pin(s);
     d[1] = ldg_pin(s + 1);
   } else {
-    r.bs = 0; r.mnf = 0; r.t0p = 0; r.t1p = 0; r.own_lo = 0; r.own_hi = 0; r.pad0 = 0; r.pad1 = 0;
+    r.bs = 0; r.mnf = 0; r.t0p = 0; r.t1p = 0; r.own_lo = 0; r.own_hi = 0; r.src = 0; r.pad1 = 0;
   }
   return r;
 }
@@ -381,6 +384,9 @@ __device__ __forceinline__ void plan_frame(const Params& p, int* __restrict__ pe
   const bool track = p.mtiles <= PLAN_MAX_MT;  // else: sorted, but every job covers the full maps
   int Nb = p.ntr ? min(max(__ldg(p.ntr + b), 0), p.N) : p.N;   // padded queries are not sorted: no tile, no job work
   if (p.nfr && s >= __ldg(p.nfr + b)) Nb = 0;                   // padded frame: every tile of it is an empty job
+  // the frame table is read here, once per frame, into the job records: the producer warp already loads those, so the
+  // operand ring gains no dependent global load
+  const int src = p.fidx ? min(max(__ldg(p.fidx + bs), 0), p.BS_src - 1) : bs;
 
   for (int i = threadIdx.x; i < PLAN_BINS; i += blockDim.x) hist[i] = 0;
   if (track)
@@ -434,7 +440,7 @@ __device__ __forceinline__ void plan_frame(const Params& p, int* __restrict__ pe
     const int mt = idx / p.nchunk, c = idx - mt * p.nchunk;
     JobRec jr;
     jr.bs = bs; jr.t0p = 0; jr.t1p = 0;
-    jr.own_lo = -BIG; jr.own_hi = BIG; jr.pad0 = 0; jr.pad1 = 0;
+    jr.own_lo = -BIG; jr.own_hi = BIG; jr.src = src; jr.pad1 = 0;
     int nseg = 0, flags = 0;
     auto rows_of = [&](int l, int& R0, int& R1) {
       if (full || !track) { R0 = 0; R1 = (MAP >> l) - 1; }
@@ -815,7 +821,7 @@ corr_tc_kernel(const Params p) {
       auto prefetch = [&]() {
         if (pf.job < p.njobs) {
           asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;"
-                       ::"l"(p.split + ((long long)pf.cur.bs * NTILES + pf.t) * STAGE_BYTES), "r"(nbytes) : "memory");
+                       ::"l"(p.split + ((long long)pf.cur.src * NTILES + pf.t) * STAGE_BYTES), "r"(nbytes) : "memory");
           cursor_next(pf);
         }
       };
@@ -831,9 +837,9 @@ corr_tc_kernel(const Params p) {
         } else {
           mbar_expect_tx(&full[stage], nbytes);
 #if COMET_TC_EVICT_FIRST
-          bulk_load_hint(dst, p.split + ((long long)ld.cur.bs * NTILES + ld.t) * STAGE_BYTES, nbytes, &full[stage], l2_policy);
+          bulk_load_hint(dst, p.split + ((long long)ld.cur.src * NTILES + ld.t) * STAGE_BYTES, nbytes, &full[stage], l2_policy);
 #else
-          bulk_load(dst, p.split + ((long long)ld.cur.bs * NTILES + ld.t) * STAGE_BYTES, nbytes, &full[stage]);
+          bulk_load(dst, p.split + ((long long)ld.cur.src * NTILES + ld.t) * STAGE_BYTES, nbytes, &full[stage]);
 #endif
         }
 #if COMET_TC_L2PF > 0
@@ -940,7 +946,7 @@ corr_tc_kernel(const Params p) {
       {
         const int4 r0 = mb[TILE_M + 2 * wq], r1 = mb[TILE_M + 2 * wq + 1];
         jr.bs = r0.x; jr.mnf = r0.y; jr.t0p = (uint32_t)r0.z; jr.t1p = (uint32_t)r0.w;
-        jr.own_lo = r1.x; jr.own_hi = r1.y; jr.pad0 = 0; jr.pad1 = 0;
+        jr.own_lo = r1.x; jr.own_hi = r1.y; jr.src = r1.z; jr.pad1 = 0;
       }
       const int4 slot = mb[q];
       const int n = slot.x;
@@ -1644,8 +1650,8 @@ extern "C" int comet_tc_corr_lookup_f32(const void* split, const float* targets,
 
 static int tc_track_tokens(const void* split, const float* track_feats, long long t_sb, long long t_ss, long long t_sn,
                            const float* coords, long long c_sb, long long c_ss, long long c_sn, const float* pos_emb,
-                           float* tokens, const int* num_tracks, const int* num_frames, int B, int S, int N, int C, int H,
-                           int W, int L, int r,
+                           float* tokens, const int* num_tracks, const int* num_frames, const int* frame_index, int BS_src,
+                           int B, int S, int N, int C, int H, int W, int L, int r,
                            int pad_mode, int prec_mode, int D_tok, void* workspace, comet_stream_t stream) {
   tc::Params p{};
   int rc = tc_common(p, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, B, S, N, C, H, W, L, r, pad_mode,
@@ -1653,9 +1659,11 @@ static int tc_track_tokens(const void* split, const float* track_feats, long lon
   if (rc != COMET_OK) return rc;
   const int need = 2 * C + 2 + L * (2 * r + 1) * (2 * r + 1);
   COMET_REQUIRE(D_tok >= need, "D_tok=%d smaller than the %d token channels", D_tok, need);
+  COMET_REQUIRE(!frame_index || BS_src >= 1, "BS_src must be positive with a frame table (got %d)", BS_src);
   if ((long long)B * S * N == 0) return COMET_OK;
   COMET_REQUIRE(split && track_feats && coords && pos_emb && tokens, "null pointer");
   p.out = tokens; p.pos = pos_emb; p.D_tok = D_tok; p.tokens = 1; p.ntr = num_tracks; p.nfr = num_frames;
+  p.fidx = frame_index; p.BS_src = BS_src;
   return tc::launch(p, split, workspace, (cudaStream_t)stream);
 }
 
@@ -1664,8 +1672,8 @@ extern "C" int comet_tc_track_tokens_f32(const void* split, const float* track_f
                                          long long c_sn, const float* pos_emb, float* tokens, int B, int S, int N,
                                          int C, int H, int W, int L, int r, int pad_mode, int prec_mode, int D_tok,
                                          void* workspace, comet_stream_t stream) {
-  return tc_track_tokens(split, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, nullptr, nullptr, B,
-                         S, N, C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace, stream);
+  return tc_track_tokens(split, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, nullptr, nullptr,
+                         nullptr, B * S, B, S, N, C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace, stream);
 }
 
 extern "C" int comet_tc_track_tokens_ragged_f32(const void* split, const float* track_feats, long long t_sb, long long t_ss,
@@ -1675,7 +1683,7 @@ extern "C" int comet_tc_track_tokens_ragged_f32(const void* split, const float* 
                                                 int prec_mode, int D_tok, void* workspace, comet_stream_t stream) {
   COMET_REQUIRE((long long)B * S * N == 0 || num_tracks, "null num_tracks");
   return tc_track_tokens(split, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks, nullptr,
-                         B, S, N, C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace, stream);
+                         nullptr, B * S, B, S, N, C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace, stream);
 }
 
 extern "C" int comet_tc_track_tokens_varlen_f32(const void* split, const float* track_feats, long long t_sb, long long t_ss,
@@ -1685,7 +1693,18 @@ extern "C" int comet_tc_track_tokens_varlen_f32(const void* split, const float* 
                                                 int pad_mode, int prec_mode, int D_tok, void* workspace,
                                                 comet_stream_t stream) {
   return tc_track_tokens(split, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks,
-                         num_frames, B, S, N, C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace, stream);
+                         num_frames, nullptr, B * S, B, S, N, C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace, stream);
+}
+
+extern "C" int comet_tc_track_tokens_indexed_f32(const void* split, const float* track_feats, long long t_sb, long long t_ss,
+                                                 long long t_sn, const float* coords, long long c_sb, long long c_ss,
+                                                 long long c_sn, const float* pos_emb, float* tokens, const int* num_tracks,
+                                                 const int* num_frames, const int* frame_index, int BS_src, int B, int S, int N,
+                                                 int C, int H, int W, int L, int r, int pad_mode, int prec_mode, int D_tok,
+                                                 void* workspace, comet_stream_t stream) {
+  return tc_track_tokens(split, track_feats, t_sb, t_ss, t_sn, coords, c_sb, c_ss, c_sn, pos_emb, tokens, num_tracks,
+                         num_frames, frame_index, BS_src, B, S, N, C, H, W, L, r, pad_mode, prec_mode, D_tok, workspace,
+                         stream);
 }
 
 extern "C" int comet_tc_corr_volume_f32(const void* split, const float* targets, long long t_sb, long long t_ss,

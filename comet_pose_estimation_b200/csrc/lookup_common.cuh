@@ -21,6 +21,8 @@ struct LookupParams {
   const float* pos;  // TOKENS: (B,N,D_tok)
   const int* ntr;    // TOKENS: (B,) query count of each sequence (rows n >= ntr[b] are written as zeros), or null
   const int* nfr;    // TOKENS: (B,) frame count of each sequence (rows s >= nfr[b] are written as zeros), or null
+  const int* fidx;   // TOKENS: (B,S) frame of fmaps / pyr that (item b, position s) reads, or null (b * S + s)
+  int BS_src;        // TOKENS with fidx: frames of fmaps / pyr (entries are clamped to [0, BS_src))
   int D_tok;
   int B, S, N, C, L, r;
   int pad_border, bf16;

@@ -293,6 +293,8 @@ struct Params {
   int nseq;                // packed tracks: number of sequences in `src`
   const int* num_frames;   // packed tracks, nullable: sequence b has num_frames[b] real frames; the patches of the others
                            // are not read and their maps are written as zeros
+  const int* frame_index;  // packed tracks, nullable: (nseq, S) image frame that frame s of sequence b reads (else b * S + s)
+  long long nframes_src;   // packed tracks with frame_index: frames of `src` (entries are clamped to [0, nframes_src))
   float eps;
 };
 
@@ -319,12 +321,15 @@ __device__ __forceinline__ void prefetch_pixels(const Params& p, long long pair,
       const int n = (int)(bn % p.N);
       long long b = bn / p.N;
       const int* tl = p.topleft + ((b * p.S + s) * p.N + n) * 2;
+      long long frame = b * p.S + s;
       if (p.seq_of_track) {
         b = min(max(__ldg(p.seq_of_track + n), 0), p.nseq - 1);
         tl = p.topleft + ((long long)n * p.S + s) * 2;
+        frame = b * p.S + s;
+        if (p.frame_index) frame = min(max((long long)__ldg(p.frame_index + frame), 0LL), p.nframes_src - 1);
       }
       const int x0 = min(max(__ldg(tl), 0), p.W - PSZ), y0 = min(max(__ldg(tl + 1), 0), p.H - PSZ);
-      base[g] = p.src + (b * p.S + s) * 3 * p.sc + (long long)y0 * p.sy + (long long)x0 * p.sx;
+      base[g] = p.src + frame * 3 * p.sc + (long long)y0 * p.sy + (long long)x0 * p.sx;
     } else {
       base[g] = p.src + pi * p.sn;
     }
@@ -630,19 +635,29 @@ extern "C" int comet_shallow_encoder_from_images_f32(const float* images, const 
   return launch_shallow_encoder(p, stream);
 }
 
-extern "C" int comet_shallow_encoder_from_images_varlen_f32(const float* images, const int* topleft, const int* seq_of_track,
-                                                            const int* num_frames, const float* packed, float* out, int P, int B,
-                                                            int S, int H, int W, float eps, comet_stream_t stream) {
+extern "C" int comet_shallow_encoder_from_images_indexed_f32(const float* images, const int* topleft, const int* seq_of_track,
+                                                             const int* num_frames, const int* frame_index, int BS_src,
+                                                             const float* packed, float* out, int P, int B, int S, int H, int W,
+                                                             float eps, comet_stream_t stream) {
   COMET_REQUIRE(P >= 0 && B >= 1 && S >= 0 && H >= senc::PSZ && W >= senc::PSZ, "bad shape");
+  COMET_REQUIRE(!frame_index || BS_src >= 1, "BS_src must be positive with a frame table (got %d)", BS_src);
   if ((long long)P * S == 0) return COMET_OK;
   COMET_REQUIRE(images && topleft && seq_of_track && packed && out, "null pointer");
   COMET_REQUIRE(((uintptr_t)packed % 16) == 0, "packed parameters must be 16-byte aligned");
   senc::Params p{};
   p.src = images; p.topleft = topleft; p.seq_of_track = seq_of_track; p.num_frames = num_frames; p.packed = packed; p.out = out;
+  p.frame_index = frame_index; p.nframes_src = BS_src;
   p.P = (long long)P * S;
   p.sn = 0; p.sc = (long long)H * W; p.sy = W; p.sx = 1;
   p.S = S; p.N = P; p.H = H; p.W = W; p.nseq = B; p.eps = eps;
   return launch_shallow_encoder(p, stream);
+}
+
+extern "C" int comet_shallow_encoder_from_images_varlen_f32(const float* images, const int* topleft, const int* seq_of_track,
+                                                            const int* num_frames, const float* packed, float* out, int P, int B,
+                                                            int S, int H, int W, float eps, comet_stream_t stream) {
+  return comet_shallow_encoder_from_images_indexed_f32(images, topleft, seq_of_track, num_frames, nullptr, B * S, packed, out, P,
+                                                       B, S, H, W, eps, stream);
 }
 
 extern "C" int comet_shallow_encoder_from_images_ragged_f32(const float* images, const int* topleft, const int* seq_of_track,

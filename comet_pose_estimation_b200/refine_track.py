@@ -172,11 +172,16 @@ class ShallowEncoder(nn.Module):
         return self._fused_result(out, (31 // self.stride, 31 // self.stride), defer_upsample)
 
     def encode_packed_patches_of(self, images: torch.Tensor, topleft: torch.Tensor, seq_of_track: torch.Tensor,
-                                 defer_upsample: bool = True, num_frames: torch.Tensor = None):
+                                 defer_upsample: bool = True, num_frames: torch.Tensor = None,
+                                 frame_index: torch.Tensor = None):
         """``encode_patches_of`` for P tracks packed from the sequences of ``images`` (B,S,3,H,W): ``topleft`` (P,S,2)
         corners, ``seq_of_track`` (P,) the sequence of each track.  Maps in (track, frame) order, each one bit-identical
         to ``encode_patches_of`` on the same patch.  ``num_frames`` (B,) int32 on the device, or None: sequence b has
-        num_frames[b] real frames; the pixels of the other frames are never read and their maps are zeros."""
+        num_frames[b] real frames; the pixels of the other frames are never read and their maps are zeros.
+
+        ``frame_index`` (B', S) integer tensor on the device: the tracks belong to B' items (``seq_of_track`` and
+        ``num_frames`` index items) and frame s of item i is image frame ``frame_index[i, s]`` of the B * S frames of
+        ``images``."""
         from . import _lib
         from ._dev import stream_ptr
 
@@ -187,7 +192,14 @@ class ShallowEncoder(nn.Module):
         seq32 = seq_of_track.to(device=images.device, dtype=torch.int32).contiguous()
         out = torch.empty((P * S, 16, 16, 32), dtype=torch.float32, device=images.device)
         with torch.cuda.device(images.device):
-            if num_frames is None:
+            if frame_index is not None:
+                nf32 = None if num_frames is None else num_frames.to(device=images.device, dtype=torch.int32).contiguous()
+                fi32 = frame_index.to(device=images.device, dtype=torch.int32).contiguous()
+                _lib.check(_lib.lib.comet_shallow_encoder_from_images_indexed_f32(
+                    img.data_ptr(), tl32.data_ptr(), seq32.data_ptr(), None if nf32 is None else nf32.data_ptr(),
+                    fi32.data_ptr(), B * S, self.packed_parameters().data_ptr(), out.data_ptr(), P, fi32.shape[0], S, H, W,
+                    float(self.norm1.eps), stream_ptr(images.device)))
+            elif num_frames is None:
                 _lib.check(_lib.lib.comet_shallow_encoder_from_images_ragged_f32(
                     img.data_ptr(), tl32.data_ptr(), seq32.data_ptr(), self.packed_parameters().data_ptr(), out.data_ptr(), P,
                     B, S, H, W, float(self.norm1.eps), stream_ptr(images.device)))
@@ -258,22 +270,30 @@ def extract_patches(images: torch.Tensor, topleft: torch.Tensor, psize: int) -> 
 
 
 def refine_track(images, fine_fnet, fine_tracker, coarse_pred, pradius=15, sradius=2, compute_score=False,
-                 num_tracks=None, num_frames=None):
+                 num_tracks=None, num_frames=None, frame_index=None):
     """refine_track.py:26-171.  ``images`` (B,S,3,H,W); ``coarse_pred`` (B,S,N,2) pixels ->
     (refined_tracks (B,S,N,2), score (B,S,N) | None).
 
     ``num_tracks`` (B ints or a 1-D tensor): ``coarse_pred`` is a padded batch; sequence b's tracks get what the call on
     that sequence alone returns (including the score quirk as it behaves for one sequence: every window of sequence b
     is cut from the frame-0 map of its own first track), entries of padded tracks are 0.  ``num_frames`` (likewise):
-    sequence b has the first ``num_frames[b]`` frames; the images of the others are never read and their entries are 0."""
-    if num_tracks is not None or num_frames is not None:
+    sequence b has the first ``num_frames[b]`` frames; the images of the others are never read and their entries are 0.
+
+    ``frame_index`` ((B', S) integer tensor): ``coarse_pred`` (B', S, N, 2) is a batch of items that read the frames of
+    ``images`` (B_src, S, 3, H, W) in their own order -- item i's frame s is image frame ``frame_index[i, s]`` of the
+    B_src * S frames -- and ``num_tracks`` / ``num_frames`` count per item.  The result is the call on the gathered
+    images ``images.flatten(0, 1)[frame_index]``; the patch encoder reads through the table, nothing is gathered."""
+    if num_tracks is not None or num_frames is not None or frame_index is not None:
         from .utils import check_num_tracks
 
         B, S, N = coarse_pred.shape[:3]
         counts = check_num_tracks([N] * B if num_tracks is None else num_tracks, B, N)
         frames = None if num_frames is None else check_num_tracks(num_frames, B, S)
+        if frame_index is not None:
+            assert frame_index.dim() == 2 and tuple(frame_index.shape) == (B, S) and images.shape[1] == S, \
+                f"frame_index must be (B', S) = ({B}, {S}) with images of S frames"
         return _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, sradius, compute_score, counts,
-                                    frames)
+                                    frames, frame_index)
     B, S, N, _ = coarse_pred.shape
     _, _, _, H, W = images.shape
     psize = pradius * 2 + 1
@@ -342,11 +362,13 @@ def refine_track(images, fine_fnet, fine_tracker, coarse_pred, pradius=15, sradi
     return refined_tracks, score
 
 
-def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, sradius, compute_score, counts, frames=None):
+def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, sradius, compute_score, counts, frames=None,
+                         frame_index=None):
     """The fine tracker works per track, so the real tracks of all sequences run as ONE packed batch of P = sum(counts)
     tracks, without per-sequence padding: the fused encoder reads each track's patches from its own sequence's frames.  Configurations
     without the fused encoder run the per-sequence definition.  ``frames``: per-sequence frame counts (None: all S); each
-    packed track then runs its own sequence's frame count through the fine tracker."""
+    packed track then runs its own sequence's frame count through the fine tracker.  ``frame_index``: the sequences are
+    items reading the frames of ``images`` through the table (see ``refine_track``)."""
     from .base_track_predictor import BaseTrackerPredictor
 
     B, S, N, _ = coarse_pred.shape
@@ -357,6 +379,8 @@ def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, 
              and isinstance(fine_tracker, BaseTrackerPredictor) and not torch.is_grad_enabled() and images.shape[2] == 3
              and psize == 31 and fine_fnet._fused_ok(images, psize, psize))
     if not fused:
+        if frame_index is not None:
+            images = images.flatten(0, 1)[frame_index.to(images.device).long()].reshape((B,) + tuple(images.shape[1:]))
         refined = coarse_pred.new_zeros(coarse_pred.shape)
         score = coarse_pred.new_zeros((B, S, N)) if compute_score else None
         for b, n in enumerate(counts):
@@ -386,7 +410,8 @@ def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, 
     topleft = torch.stack([topleft_raw[..., 0].clamp(0, W - psize), topleft_raw[..., 1].clamp(0, H - psize)], dim=-1)
 
     dev_frames = None if frames is None else torch.tensor(frames, dtype=torch.int32, device=dev)
-    half, size = fine_fnet.encode_packed_patches_of(images, topleft, seq, defer_upsample=True, num_frames=dev_frames)
+    half, size = fine_fnet.encode_packed_patches_of(images, topleft, seq, defer_upsample=True, num_frames=dev_frames,
+                                                    frame_index=None if frame_index is None else frame_index.to(dev))
     Hs, Ws = half.shape[-2:]
     C_out = half.shape[1]
     half = half.contiguous(memory_format=torch.channels_last)

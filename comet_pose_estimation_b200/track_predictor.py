@@ -22,7 +22,7 @@ import torch.nn.functional as F
 
 from .base_track_predictor import BaseTrackerPredictor
 from .refine_track import ShallowEncoder, _inorm, _ResidualBlock, _resize, inverted_score, refine_track
-from .utils import check_num_tracks
+from .utils import check_num_tracks, check_query_frames, query_frame_items
 
 
 class BasicEncoder(nn.Module):
@@ -117,11 +117,19 @@ class TrackerPredictor(nn.Module):
         return fmaps.reshape(B, S, -1, fmaps.shape[-2], fmaps.shape[-1])
 
     @torch.no_grad()
-    def track(self, images, query_points, coarse_iters=4, fine_tracking=True):
+    def track(self, images, query_points, coarse_iters=4, fine_tracking=True, query_frames=None):
         """The tracker part of ``COMET.forward_all`` (E2Epose2.py:176-239): images (B,S,3,H,W) in the model's
         normalisation, ``query_points`` (B,N,2) pixels of frame 0 -> dict with ``coarse_pred_track`` /
         ``refine_pred_track`` (B,S,N,2), ``pred_score`` (the inverted, normalised track confidence the camera predictor
-        consumes), ``vis`` and the per-iteration coarse list."""
+        consumes), ``vis`` and the per-iteration coarse list.
+
+        ``query_frames`` ((1, N) or (N,) integers): track n starts on frame ``query_frames[n]`` and ``query_points[:, n]``
+        are pixels of that frame; see ``track_batch``.  The dict then also holds ``query_frames`` (1, N) int64."""
+        if query_frames is not None:
+            assert images.shape[0] == 1, "now we only support processing one scene during inference"
+            qf = query_frames.reshape(1, -1) if isinstance(query_frames, torch.Tensor) else torch.tensor([list(query_frames)])
+            return split_batch(self.track_batch(images, query_points, coarse_iters=coarse_iters, fine_tracking=fine_tracking,
+                                                query_frames=qf))[0]
         fmaps = self.process_images_to_fmaps(images)
         coarse_list, vis, track_feats, query_feat, conf = self.coarse_predictor(
             query_points=query_points, fmaps=fmaps, iters=coarse_iters, down_ratio=self.coarse_down_ratio, is_train=False,
@@ -139,7 +147,8 @@ class TrackerPredictor(nn.Module):
         return out
 
     @torch.no_grad()
-    def track_batch(self, images, query_points, num_tracks=None, coarse_iters=4, fine_tracking=True, num_frames=None):
+    def track_batch(self, images, query_points, num_tracks=None, coarse_iters=4, fine_tracking=True, num_frames=None,
+                    query_frames=None):
         """``track`` for B sequences in one call: images (B,S,3,H,W) (same image size for all), ``query_points``
         a list of B tensors (N_b, 2) or a padded (B, N_max, 2) tensor with ``num_tracks`` (B,) (None: every sequence
         has N_max tracks).  Returns ``track``'s dict with padded tensors (entries of tracks n >= N_b are 0) plus
@@ -149,7 +158,15 @@ class TrackerPredictor(nn.Module):
         Sequences of different lengths: ``images`` a list of B tensors (S_b,3,H,W), or the padded (B,S_max,3,H,W) with
         ``num_frames`` (B,) (1 <= S_b <= S_max).  Frames s >= S_b of a padded tensor are never read; every output entry
         of such a frame is 0, ``pred_score`` is normalised over the real frames of each track, and the dict gets
-        ``num_frames`` (B,) int64."""
+        ``num_frames`` (B,) int64.
+
+        Tracks that start on any frame: ``query_frames`` gives each track's query frame t_n (a list of B integer tensors
+        (N_b,), or a padded (B, N_max) tensor; None: all 0), and ``query_points`` are pixels of that frame.  Track n of
+        sequence b with t_n = q gets what this call returns for it on one item: sequence b's images with frames 0 and q
+        swapped, the tracks of sequence b whose query frame is q (in their order), S_b frames -- with every per-frame
+        output swapped back.  Tracks of different query frames do not interact.  The frames are encoded once whatever
+        the number of query frames; every item reads them through a frame table.  The dict gets ``query_frames``
+        (B, N_max) int64.  Query frames all 0 run exactly the path without them."""
         if isinstance(images, (list, tuple)):
             slens = [int(x.shape[0]) for x in images]
             assert num_frames is None or check_num_tracks(num_frames, len(images), max(slens)) == slens, \
@@ -173,6 +190,13 @@ class TrackerPredictor(nn.Module):
         assert query_points.dim() == 3 and query_points.shape[0] == B and query_points.shape[2] == 2
         N = query_points.shape[1]
         counts = check_num_tracks([N] * B if num_tracks is None else num_tracks, B, N)
+        if query_frames is not None:
+            qf = check_query_frames(query_frames, counts, [S] * B if frames is None else frames)
+            if any(t for q in qf for t in q):
+                return self._track_batch_query_frames(images, query_points, counts, frames, qf, coarse_iters, fine_tracking)
+            out = self.track_batch(images, query_points, counts, coarse_iters, fine_tracking, frames)
+            out["query_frames"] = torch.zeros((B, N), dtype=torch.int64)
+            return out
         if frames is not None:
             return self._track_batch_frames(images, query_points, counts, frames, coarse_iters, fine_tracking)
         fmaps = self._encode_frames(images)
@@ -220,6 +244,65 @@ class TrackerPredictor(nn.Module):
         return out
 
 
+    def _track_batch_query_frames(self, images, query_points, counts, frames, qf, coarse_iters, fine_tracking):
+        """``track_batch`` with per-track query frames (validated lists): one item per (sequence, query frame), one
+        encoder pass over the source frames, one predictor and one ``refine_track`` call over the items, results
+        scattered back to (sequence, frame, track) order."""
+        B, S = images.shape[:2]
+        N = query_points.shape[1]
+        dev = query_points.device
+        items, frame_index = query_frame_items(qf, [S] * B if frames is None else frames, S)
+        item_counts = [len(ns) for _, _, ns in items]
+        item_frames = None if frames is None else [frames[b] for b, _, _ in items]
+        item_b = torch.tensor([b for b, _, ns in items for _ in ns], device=dev)        # (M,) per real track
+        item_i = torch.tensor([i for i, (_, _, ns) in enumerate(items) for _ in ns], device=dev)
+        item_j = torch.tensor([j for _, _, ns in items for j in range(len(ns))], device=dev)
+        item_n = torch.tensor([n for _, _, ns in items for n in ns], device=dev)
+        q_items = query_points.new_zeros((len(items), max(item_counts), 2))
+        q_items[item_i, item_j] = query_points[item_b, item_n]
+        # position s of item i shows frame swap(s) of its sequence, and the swap is its own inverse
+        pos_of_frame = (frame_index - torch.tensor([b * S for b, _, _ in items])[:, None]).to(dev)   # (B', S)
+
+        fmaps = self._encode_frames(images, frames)
+        coarse_list, vis, track_feats, query_feat, conf = self.coarse_predictor(
+            query_points=q_items, fmaps=fmaps, iters=coarse_iters, down_ratio=self.coarse_down_ratio, is_train=False,
+            return_feat=True, TRACKorPOSE=False, num_tracks=item_counts, num_frames=item_frames, frame_index=frame_index)
+        coarse = coarse_list[-1]
+        Si, Ni = coarse.shape[1], coarse.shape[2]
+        out = {"coarse_pred_track_list": coarse_list, "coarse_pred_track": coarse, "vis": vis, "conf": conf}
+        real = padded_mask(item_counts, [Si] * len(items) if item_frames is None else item_frames, Si, Ni, coarse.device)
+        if fine_tracking:
+            refined, score = refine_track(images, self.fine_fnet, self.fine_predictor, coarse, compute_score=True,
+                                          num_tracks=item_counts, num_frames=item_frames, frame_index=frame_index)
+            out["refine_pred_track"] = refined
+            out["track_score"] = score
+            out["pred_score"] = inverted_score(score) * real if item_frames is None else inverted_score_padded(score, real)
+        else:
+            out["refine_pred_track"] = coarse
+            out["pred_score"] = torch.ones_like(vis) * real
+
+        def scatter(v):
+            if v is None:
+                return None
+            if isinstance(v, list):
+                return [scatter(x) for x in v]
+            idx = pos_of_frame.reshape(pos_of_frame.shape + (1,) * (v.dim() - 2)).expand((-1, -1) + tuple(v.shape[2:]))
+            v = v.gather(1, idx)                                    # (B', S, N_cap, ...) in each sequence's frame order
+            res = v.new_zeros((B, S, N) + tuple(v.shape[3:]))
+            res[item_b, :, item_n] = v[item_i, :, item_j]
+            return res
+
+        out = {k: scatter(v) for k, v in out.items()}
+        out["num_tracks"] = torch.tensor(counts, dtype=torch.int64)
+        if frames is not None:
+            out["num_frames"] = torch.tensor(frames, dtype=torch.int64)
+        qf_pad = torch.zeros((B, N), dtype=torch.int64)
+        for b, q in enumerate(qf):
+            qf_pad[b, :len(q)] = torch.tensor(q, dtype=torch.int64)
+        out["query_frames"] = qf_pad
+        return out
+
+
 def padded_mask(counts, frames, S: int, N: int, device) -> torch.Tensor:
     """(B, S, N) bool: entry (b, s, n) is a real frame and track of a padded batch."""
     c = torch.tensor(counts, device=device)
@@ -238,7 +321,7 @@ def inverted_score_padded(track_score: torch.Tensor, real: torch.Tensor, eps: fl
 
 def split_batch(out):
     """``track_batch``'s padded dict -> list of per-sequence dicts with exactly ``track``'s keys and shapes (cut along
-    the frame axis too when the dict has ``num_frames``)."""
+    the frame axis too when the dict has ``num_frames``; ``query_frames`` is cut to (1, N_b))."""
     counts = [int(n) for n in out["num_tracks"]]
     frames = [int(s) for s in out["num_frames"]] if "num_frames" in out else [None] * len(counts)
 
@@ -247,6 +330,8 @@ def split_batch(out):
             return None
         if isinstance(v, list):
             return [cut(x, b, n, s) for x in v]
+        if v.dim() == 2:                                    # per-track keys (B, N_max): query_frames
+            return v[b:b + 1, :n]
         return v[b:b + 1, :s, :n]
 
     return [{k: cut(v, b, n, s) for k, v in out.items() if k not in ("num_tracks", "num_frames")}

@@ -83,10 +83,14 @@ class TrackTokenizer:
 
     def __init__(self, corr: Union[CorrBlock, EfficientCorrBlock, torch.Tensor], coords0: torch.Tensor,
                  tdim: int, num_levels: Optional[int] = None, radius: Optional[int] = None,
-                 padding_mode: Optional[str] = None, num_tracks=None, num_frames=None):
+                 padding_mode: Optional[str] = None, num_tracks=None, num_frames=None, frame_index=None):
         """``num_tracks`` (B ints or a 1-D tensor): the queries form a padded batch; queries n >= num_tracks[b] are
         padding, their token rows are zeros and cost no correlation work.  ``num_frames`` (likewise): sequence b has the
-        first num_frames[b] of the S frames; the token rows of the others are zeros and read nothing."""
+        first num_frames[b] of the S frames; the token rows of the others are zeros and read nothing.
+
+        ``frame_index`` (B', S) integer tensor: the pyramid holds B_src * S source frames and the B' items of
+        ``coords0`` read them in their own order -- item i sees source frame ``frame_index[i, s]`` (flat index) at
+        position s.  The pyramid is prepared once; counts, coordinates and tokens are per item."""
         if isinstance(corr, (torch.Tensor, Upsampled2x)):
             assert num_levels is not None and radius is not None
             self.radius = radius
@@ -100,6 +104,15 @@ class TrackTokenizer:
         self.tdim = tdim
         p = self._pyr
         self.pos = sampled_pos_emb(coords0, tdim, p.H, p.W)
+        self.frame_index = None
+        self.B = p.B
+        if frame_index is not None:
+            assert frame_index.shape == (coords0.shape[0], p.S), \
+                f"frame_index must be (B', S) = ({coords0.shape[0]}, {p.S}), got {tuple(frame_index.shape)}"
+            fi = frame_index.to(device=coords0.device, dtype=torch.int32).contiguous()
+            assert bool(((fi >= 0) & (fi < p.B * p.S)).all()), f"frame_index outside [0, {p.B * p.S})"
+            self.frame_index = fi
+            self.B = coords0.shape[0]
         self.num_tracks = None
         if num_tracks is not None:
             from .utils import check_num_tracks
@@ -110,7 +123,7 @@ class TrackTokenizer:
         if num_frames is not None:
             from .utils import check_num_tracks
 
-            frames = check_num_tracks(num_frames, coords0.shape[0], p.S)
+            frames = check_num_tracks(num_frames, self.B, p.S)
             self.num_frames = torch.tensor(frames, dtype=torch.int32).to(coords0.device)
 
     def tokens(self, coords: torch.Tensor, track_feats: torch.Tensor, out: Optional[torch.Tensor] = None):
@@ -119,7 +132,7 @@ class TrackTokenizer:
         B, S, N, D = coords.shape
         assert D == 2
         assert track_feats.shape == (B, S, N, p.C), "track_feats must be (B,S,N,latent) with latent == C"
-        assert S == p.S and B == p.B
+        assert S == p.S and B == self.B
         require_cuda(coords, "coords")
         require_cuda(track_feats, "track_feats")
         require_no_grad(coords, track_feats)
@@ -130,13 +143,17 @@ class TrackTokenizer:
         else:
             assert out.shape == (B, N, S, self.tdim) and out.is_contiguous() and out.dtype == torch.float32
         with torch.cuda.device(c.device):
-            nt, nf = self.num_tracks, self.num_frames
+            nt, nf, fi = self.num_tracks, self.num_frames, self.frame_index
             if B * S * N and _use_tc(p, t, self.radius, self.padding_mode):
                 head = (p.split.data_ptr(), t.data_ptr(), t.stride(0), t.stride(1), t.stride(2),
                         c.data_ptr(), c.stride(0), c.stride(1), c.stride(2), self.pos.data_ptr(), out.data_ptr())
                 tail = (B, S, N, p.C, p.H, p.W, p.num_levels, self.radius, pad_mode(self.padding_mode), prec_mode(),
-                        self.tdim, _tc_workspace(p, N).data_ptr(), stream_ptr(c.device))
-                if nf is not None:
+                        self.tdim, _tc_workspace(p, N, B * S).data_ptr(), stream_ptr(c.device))
+                if fi is not None:
+                    _lib.check(lib.comet_tc_track_tokens_indexed_f32(
+                        *head, None if nt is None else nt.data_ptr(), None if nf is None else nf.data_ptr(), fi.data_ptr(),
+                        p.B * p.S, *tail))
+                elif nf is not None:
                     _lib.check(lib.comet_tc_track_tokens_varlen_f32(*head, None if nt is None else nt.data_ptr(),
                                                                     nf.data_ptr(), *tail))
                 elif nt is None:
@@ -148,7 +165,11 @@ class TrackTokenizer:
                     c.data_ptr(), c.stride(0), c.stride(1), c.stride(2), self.pos.data_ptr(), out.data_ptr())
             tail = (B, S, N, p.C, p.H, p.W, p.num_levels, self.radius, pad_mode(self.padding_mode), prec_mode(),
                     p.layout, self.tdim, stream_ptr(c.device))
-            if nf is not None:
+            if fi is not None:
+                _lib.check(lib.comet_track_tokens_indexed_f32(*head, None if nt is None else nt.data_ptr(),
+                                                              None if nf is None else nf.data_ptr(), fi.data_ptr(),
+                                                              p.B * p.S, *tail))
+            elif nf is not None:
                 _lib.check(lib.comet_track_tokens_varlen_f32(*head, None if nt is None else nt.data_ptr(), nf.data_ptr(),
                                                              *tail))
             elif nt is None:

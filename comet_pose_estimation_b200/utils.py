@@ -216,3 +216,47 @@ def check_num_tracks(num_tracks, B: int, N_max: int) -> list:
     assert len(vals) == B, f"num_tracks has {len(vals)} entries for a batch of {B} sequences"
     assert all(1 <= v <= N_max for v in vals), f"num_tracks {vals} outside [1, {N_max}]"
     return vals
+
+
+def check_query_frames(query_frames, counts, frames) -> list:
+    """Per-track query frames of a padded batch -> list of B lists of Python ints (list b has counts[b] entries, each in
+    [0, frames[b])).  ``query_frames``: a list of B 1-D tensors / sequences with counts[b] entries, or a padded
+    (B, N_max) tensor (entries of padded tracks are ignored).  Anything else raises AssertionError."""
+    B = len(counts)
+    if isinstance(query_frames, torch.Tensor):
+        assert query_frames.dim() == 2 and query_frames.shape[0] == B and query_frames.shape[1] >= max(counts), \
+            f"query_frames must be (B, N_max) = ({B}, >= {max(counts)}), got shape {tuple(query_frames.shape)}"
+        assert not query_frames.is_floating_point(), "query_frames must be integers"
+        rows = query_frames.tolist()
+        vals = [[int(t) for t in rows[b][:n]] for b, n in enumerate(counts)]
+    else:
+        vals = []
+        for q in query_frames:
+            if isinstance(q, torch.Tensor):
+                assert q.dim() == 1 and not q.is_floating_point(), "each query_frames entry must be a 1-D integer tensor"
+                q = q.tolist()
+            vals.append([int(t) for t in q])
+        assert len(vals) == B, f"query_frames has {len(vals)} entries for a batch of {B} sequences"
+        assert [len(v) for v in vals] == list(counts), \
+            f"query_frames lengths {[len(v) for v in vals]} disagree with the track counts {list(counts)}"
+    for b, (v, s) in enumerate(zip(vals, frames)):
+        assert all(0 <= t < s for t in v), f"query_frames of sequence {b} outside [0, {s})"
+    return vals
+
+
+def query_frame_items(query_frames, frames, S_max: int):
+    """Items of a batch with per-track query frames (validated lists, see ``check_query_frames``): the tracks of
+    sequence b with query frame q form item (b, q); items are ordered by (b, q), tracks inside an item keep their order.
+    -> (items, frame_index): ``items`` a list of (b, q, track indices); ``frame_index`` (B', S_max) int64 on the CPU,
+    entry (i, s) the flat index into the B * S_max source frames of the frame that item i sees at position s: sequence
+    b's frames with 0 and q swapped; padded positions s >= frames[b] keep their identity index."""
+    items = []
+    for b, qf in enumerate(query_frames):
+        for q in sorted(set(qf)):
+            items.append((b, q, [n for n, t in enumerate(qf) if t == q]))
+    frame_index = torch.empty((len(items), S_max), dtype=torch.int64)
+    for i, (b, q, _) in enumerate(items):
+        order = list(range(S_max))
+        order[0], order[q] = q, 0
+        frame_index[i] = torch.tensor(order) + b * S_max
+    return items, frame_index

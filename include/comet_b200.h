@@ -165,6 +165,18 @@ int comet_track_tokens_varlen_f32(const float* fmaps, const float* pyr, const fl
                                   long long c_sn, const float* pos_emb, float* tokens, const int* num_tracks,
                                   const int* num_frames, int B, int S, int N, int C, int H, int W, int L, int r, int pad_mode,
                                   int prec_mode, int pyr_layout, int D_tok, comet_stream_t stream);
+/* The same for B items that read the BS_src frames of fmaps / pyr (pyramid of all BS_src frames, as comet_pyramid_f32 lays it
+ * out for BS = BS_src) in their own order: frame_index (B,S) int32 in device memory gives the frame that item b reads at
+ * position s (entries outside [0, BS_src) are clamped).  Coordinates, track features, position embedding and tokens stay
+ * per (item, position); num_tracks / num_frames keep their meaning.  Every row equals comet_track_tokens_varlen_f32 on
+ * fmaps gathered as fmaps.reshape(BS_src, ...)[frame_index].  frame_index NULL is comet_track_tokens_varlen_f32.  The
+ * C == 32 layouts serve a frame table without counts; COMET_PYR_UP2_SOURCE serves none. */
+int comet_track_tokens_indexed_f32(const float* fmaps, const float* pyr, const float* track_feats, long long t_sb,
+                                   long long t_ss, long long t_sn, const float* coords, long long c_sb, long long c_ss,
+                                   long long c_sn, const float* pos_emb, float* tokens, const int* num_tracks,
+                                   const int* num_frames, const int* frame_index, int BS_src, int B, int S, int N, int C, int H,
+                                   int W, int L, int r, int pad_mode, int prec_mode, int pyr_layout, int D_tok,
+                                   comet_stream_t stream);
 
 /* sampled_pos_emb = sample_features4d(get_2d_sincos_pos_embed(D,(H,W)), coords[:,0])
  * (base_track_predictor.py:200-208; utils.py:724-755, :942-974): the float64 table is evaluated on the fly at
@@ -248,6 +260,13 @@ int comet_shallow_encoder_from_images_ragged_f32(const float* images, const int*
 int comet_shallow_encoder_from_images_varlen_f32(const float* images, const int* topleft, const int* seq_of_track,
                                                  const int* num_frames, const float* packed, float* out, int P, int B, int S,
                                                  int H, int W, float eps, comet_stream_t stream);
+/* The same where frame s of sequence b reads image frame frame_index[b * S + s] of the BS_src frames of `images`
+ * ((BS_src, 3, H, W) viewed flat; frame_index (B,S) int32 in device memory, entries clamped to [0, BS_src)) instead of
+ * frame b * S + s.  frame_index NULL is the call above. */
+int comet_shallow_encoder_from_images_indexed_f32(const float* images, const int* topleft, const int* seq_of_track,
+                                                  const int* num_frames, const int* frame_index, int BS_src,
+                                                  const float* packed, float* out, int P, int B, int S, int H, int W,
+                                                  float eps, comet_stream_t stream);
 
 /* ---- sin/cos encodings: comet/models/utils.py:37-101, :724-832 ----------- */
 /* get_2d_embedding(xy, C, cat_coords): xy (M,2) contiguous -> out (M, 2*C [+2 in front if cat_coords]). */
@@ -295,6 +314,16 @@ int comet_tc_track_tokens_varlen_f32(const void* split, const float* track_feats
                                      const float* pos_emb, float* tokens, const int* num_tracks, const int* num_frames,
                                      int B, int S, int N, int C, int H, int W, int L, int r, int pad_mode, int prec_mode,
                                      int D_tok, void* workspace, comet_stream_t stream);
+/* The same for B items that read the BS_src frames of `split` (comet_tc_prepare_f32 with BS = BS_src) in their own order:
+ * frame_index (B,S) int32 in device memory, entries clamped to [0, BS_src).  The plan kernel reads each frame's entry once
+ * and stores it in that frame's job records, from which the operand producer addresses its tiles.  Everything else stays
+ * per (item, position), including `workspace` (comet_tc_workspace_bytes(B*S, N)).  Rows are bit-identical to
+ * comet_tc_track_tokens_varlen_f32 on a split prepared from the gathered frames.  frame_index NULL is that call. */
+int comet_tc_track_tokens_indexed_f32(const void* split, const float* track_feats, long long t_sb, long long t_ss,
+                                      long long t_sn, const float* coords, long long c_sb, long long c_ss, long long c_sn,
+                                      const float* pos_emb, float* tokens, const int* num_tracks, const int* num_frames,
+                                      const int* frame_index, int BS_src, int B, int S, int N, int C, int H, int W, int L,
+                                      int r, int pad_mode, int prec_mode, int D_tok, void* workspace, comet_stream_t stream);
 /* vols: HOST array of L device pointers, level l = (B*S, N, H_l*W_l) float32. */
 int comet_tc_corr_volume_f32(const void* split, const float* targets, long long t_sb, long long t_ss, long long t_sn,
                              float* const* vols, int B, int S, int N, int C, int H, int W, int L, int prec_mode,
