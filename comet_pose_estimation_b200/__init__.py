@@ -33,6 +33,7 @@ from .utils import (  # noqa: F401
 from .track_tokens import TrackTokenizer, sampled_pos_emb, transformer_dim  # noqa: F401
 from .update_former import EfficientUpdateFormer  # noqa: F401
 from .base_track_predictor import BaseTrackerPredictor  # noqa: F401
+from .packed_frames import PackedFrames  # noqa: F401
 from .refine_track import ShallowEncoder, compute_score_fn, extract_patches, inverted_score, refine_track  # noqa: F401
 from .track_predictor import BasicEncoder, TrackerPredictor, split_batch  # noqa: F401
 

@@ -65,6 +65,8 @@ SIGNATURES = {
     "comet_shallow_encoder_from_images_varlen_f32": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, C.c_float, _p]),
     "comet_shallow_encoder_from_images_indexed_f32": (_i, [_p, _p, _p, _p, _p, _i, _p, _p, _i, _i, _i, _i, _i, C.c_float,
                                                            _p]),
+    "comet_shallow_encoder_from_images_packed_f32": (_i, [_p, _p, _p, _ll, _p, _p, _p, _p, _p, _p, _i, _i, _i, C.c_float,
+                                                          _p]),
     "comet_embed2d_f32": (_i, [_p, _p, _ll, _i, _i, _p]),
     "comet_sincos1d_from_grid_f32": (_i, [_p, _p, _ll, _i, _p]),
     "comet_sincos2d_f32": (_i, [_p, _i, _i, _i, _p]),

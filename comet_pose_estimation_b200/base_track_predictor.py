@@ -47,7 +47,8 @@ class BaseTrackerPredictor(nn.Module):
             self.vis_predictor = nn.Sequential(nn.Linear(latent_dim, 1))
 
     def forward(self, query_points, fmaps=None, iters=4, return_feat=False, down_ratio=1, is_train=False,
-                track_feats=None, TRACKorPOSE=True, ind=0, num_tracks=None, num_frames=None, frame_index=None):
+                track_feats=None, TRACKorPOSE=True, ind=0, num_tracks=None, num_frames=None, frame_index=None,
+                group_items=None):
         """``num_tracks`` (B ints or a 1-D tensor, ``TRACKorPOSE=False`` only): ``query_points`` (B, N_max, 2) is a padded
         batch of sequences with different track counts.  Sequence b's tracks get what a call on that sequence alone
         computes (up to rounding); every output entry of a padded track (n >= num_tracks[b]) is 0.  ``num_frames``
@@ -58,8 +59,47 @@ class BaseTrackerPredictor(nn.Module):
         frames and ``query_points`` (B', N_max, 2) a batch of B' items; item i sees source frame ``frame_index[i, s]``
         (flat index into the B_src * S frames) at position s.  The result is the forward on the gathered maps
         ``fmaps.flatten(0, 1)[frame_index]``: on the GPU the pyramid is prepared once over the source frames and the token
-        kernels read it through the table; elsewhere the gathered maps are built and the ordinary path runs."""
-        if frame_index is not None:
+        kernels read it through the table; elsewhere the gathered maps are built and the ordinary path runs.
+
+        Size groups (``TRACKorPOSE=False`` only): ``fmaps`` a list of G per-group maps (B_g, S, C, H_g, W_g) of different
+        sizes, and the items of ``query_points`` ordered group by group -- B_g items per group, or ``group_items[g]``
+        with ``frame_index``, whose rows of group g index group g's B_g * S frames.  Each item gets what the call on its
+        group alone computes (up to the rounding of the iterated loop; tokens and the first transformer pass are the
+        same bits): every group has its own pyramid, position embedding and token launch, and the update transformer
+        runs once over all items.  Elsewhere than on the GPU each group runs alone and the results are concatenated."""
+        if isinstance(fmaps, (list, tuple)):
+            assert not TRACKorPOSE, "size groups are served with TRACKorPOSE=False only"
+            fmaps = list(fmaps)
+            Bi = query_points.shape[0]
+            sizes = [f.shape[0] for f in fmaps] if group_items is None else [int(n) for n in group_items]
+            assert frame_index is None or group_items is not None, "frame_index over size groups needs group_items"
+            assert len(sizes) == len(fmaps) and all(n >= 1 for n in sizes) and sum(sizes) == Bi, \
+                f"group_items {sizes} do not cover the {Bi} items"
+            assert frame_index is not None or all(f.shape[0] == n for f, n in zip(fmaps, sizes))
+            assert all(f.dim() == 5 and f.shape[1] == fmaps[0].shape[1] for f in fmaps), "per-group fmaps (B_g, S, C, H, W)"
+            if frame_index is not None:
+                assert frame_index.dim() == 2 and tuple(frame_index.shape) == (Bi, fmaps[0].shape[1]), \
+                    f"frame_index must be (B', S) = ({Bi}, {fmaps[0].shape[1]}), got {tuple(frame_index.shape)}"
+            if not fmaps[0].is_cuda:
+                from .utils import check_num_tracks
+
+                counts = None if num_tracks is None else check_num_tracks(num_tracks, Bi, query_points.shape[1])
+                frames = None if num_frames is None else check_num_tracks(num_frames, Bi, fmaps[0].shape[1])
+                outs, at = [], 0
+                for f, n in zip(fmaps, sizes):
+                    outs.append(self.forward(query_points[at:at + n], f, iters, True, down_ratio, is_train, track_feats,
+                                             TRACKorPOSE, ind, None if counts is None else counts[at:at + n],
+                                             None if frames is None else frames[at:at + n],
+                                             None if frame_index is None else frame_index[at:at + n]))
+                    at += n
+                cat = lambda vs: None if vs[0] is None else torch.cat(vs)  # noqa: E731
+                res = ([cat([o[0][i] for o in outs]) for i in range(len(outs[0][0]))],) + tuple(
+                    cat([o[k] for o in outs]) for k in range(1, 5))
+                return res if return_feat else (res[0], res[1], res[4])
+            if frame_index is not None:
+                frame_index = frame_index.to(fmaps[0].device)
+            group_items = sizes
+        elif frame_index is not None:
             assert not TRACKorPOSE, "frame_index is served with TRACKorPOSE=False only"
             assert isinstance(fmaps, torch.Tensor) and fmaps.dim() == 5, "frame_index needs fmaps (B_src, S, C, H, W)"
             assert frame_index.dim() == 2 and frame_index.shape == (query_points.shape[0], fmaps.shape[1]), \
@@ -69,14 +109,16 @@ class BaseTrackerPredictor(nn.Module):
                 return self.forward(query_points, gathered, iters, return_feat, down_ratio, is_train, track_feats,
                                     TRACKorPOSE, ind, num_tracks, num_frames)
             frame_index = frame_index.to(fmaps.device)
+        grouped = isinstance(fmaps, list)
         counts = frames = None
-        B_items = query_points.shape[0] if frame_index is not None else fmaps.shape[0]
+        B_items = query_points.shape[0] if frame_index is not None or grouped else fmaps.shape[0]
+        S_maps = fmaps[0].shape[1] if grouped else fmaps.shape[1]
         if num_frames is not None:
             assert not TRACKorPOSE, "num_frames is served with TRACKorPOSE=False only"
             from .utils import check_num_tracks
 
-            frames = check_num_tracks(num_frames, B_items, fmaps.shape[1])
-            live = torch.arange(fmaps.shape[1], device=query_points.device)[None, :] < torch.tensor(
+            frames = check_num_tracks(num_frames, B_items, S_maps)
+            live = torch.arange(S_maps, device=query_points.device)[None, :] < torch.tensor(
                 frames, device=query_points.device)[:, None]                                  # (B, S)
         if num_tracks is not None:
             assert not TRACKorPOSE, "num_tracks is served with TRACKorPOSE=False only"
@@ -90,8 +132,8 @@ class BaseTrackerPredictor(nn.Module):
             B, S, N, D = query_points.shape
         else:
             B, N, D = query_points.shape
-        _, S, C, HH, WW = fmaps.shape
-        if frame_index is None:
+        S = S_maps
+        if frame_index is None and not grouped:
             B = fmaps.shape[0]
         assert D == 2
         if down_ratio > 1:  # guards BOTH divisions (SURVEY A.6 i)
@@ -104,7 +146,12 @@ class BaseTrackerPredictor(nn.Module):
         if frames is not None:
             coords = coords * live[:, :, None, None]
 
-        if frame_index is not None:
+        if grouped:
+            bounds = [sum(group_items[:g]) for g in range(len(fmaps) + 1)]
+            query_track_feat = torch.cat([sample_features4d(
+                f[:, 0] if frame_index is None else f.flatten(0, 1)[frame_index[r0:r1, 0].long()], coords[r0:r1, 0])
+                for f, r0, r1 in zip(fmaps, bounds[:-1], bounds[1:])])
+        elif frame_index is not None:
             # each item's position-0 map: a gather of B' maps (the same values the gathered copy would hold)
             query_track_feat = sample_features4d(fmaps.flatten(0, 1)[frame_index[:, 0].long()], coords[:, 0])
         elif isinstance(fmaps, Upsampled2x):
@@ -115,13 +162,14 @@ class BaseTrackerPredictor(nn.Module):
         track_feats = query_track_feat.unsqueeze(1).repeat(1, S, 1, 1)
         coords_backup = coords.clone()
 
-        if self.efficient_corr:
-            fcorr_fn = EfficientCorrBlock(fmaps, num_levels=self.corr_levels, radius=self.corr_radius)
+        corr_cls = EfficientCorrBlock if self.efficient_corr else CorrBlock
+        if grouped:
+            fcorr_fn = [corr_cls(f, num_levels=self.corr_levels, radius=self.corr_radius) for f in fmaps]
         else:
-            fcorr_fn = CorrBlock(fmaps, num_levels=self.corr_levels, radius=self.corr_radius)
+            fcorr_fn = corr_cls(fmaps, num_levels=self.corr_levels, radius=self.corr_radius)
         # sampled_pos_emb depends on coords[:, 0] only, which the loop pins -> computed once, not per iteration
         tokenizer = TrackTokenizer(fcorr_fn, coords[:, 0], self.transformer_dim, num_tracks=counts, num_frames=frames,
-                                   frame_index=frame_index)
+                                   frame_index=frame_index, group_items=group_items if grouped else None)
 
         coord_preds = []
         for _ in range(iters):

@@ -296,6 +296,8 @@ struct Params {
   const int* frame_index;  // packed tracks, nullable: (nseq, S) image frame that frame s of sequence b reads (else b * S + s)
   long long nframes_src;   // packed tracks with frame_index: frames of `src` (entries are clamped to [0, nframes_src))
   float eps;
+  const long long* frame_offset;  // packed frames (PACKED kernels only): frame f starts at element frame_offset[f] of `src`
+  const int* frame_hw;            // ... and is frame_hw[2f] x frame_hw[2f+1] pixels (H, W); nframes_src frames in all
 };
 
 // Packed tracks with frame counts: patch pi lies in a frame past its sequence's count.
@@ -306,9 +308,13 @@ __device__ __forceinline__ bool padded_patch(const Params& p, long long pi) {
   return s >= __ldg(p.num_frames + b);
 }
 
-// pixels of patch pair `pair` -> registers: thread <-> cells tid + 256 k of the 2 x 31 x 31 cells, 3 channels each
+// pixels of patch pair `pair` -> registers: thread <-> cells tid + 256 k of the 2 x 31 x 31 cells, 3 channels each.
+// PACKED: `src` is a packed frame buffer (packed tracks only); a patch's frame brings its own offset, size and strides.
+template <bool PACKED>
 __device__ __forceinline__ void prefetch_pixels(const Params& p, long long pair, int tid, float (&pre)[24]) {
   const float* base[G];
+  long long plane[G];      // PACKED: channel stride and row stride of each patch's frame
+  int row[G];
 #pragma unroll
   for (int g = 0; g < G; ++g) {
     long long pi = pair * G + g;
@@ -328,6 +334,16 @@ __device__ __forceinline__ void prefetch_pixels(const Params& p, long long pair,
         frame = b * p.S + s;
         if (p.frame_index) frame = min(max((long long)__ldg(p.frame_index + frame), 0LL), p.nframes_src - 1);
       }
+      if constexpr (PACKED) {
+        frame = min(max(frame, 0LL), p.nframes_src - 1);
+        const int fh = __ldg(p.frame_hw + 2 * frame), fw = __ldg(p.frame_hw + 2 * frame + 1);
+        // the corner is clamped to the patch's own frame, so no read leaves it; a frame smaller than a patch is not read
+        const int x0 = min(max(__ldg(tl), 0), fw - PSZ), y0 = min(max(__ldg(tl + 1), 0), fh - PSZ);
+        base[g] = fh < PSZ || fw < PSZ ? nullptr : p.src + __ldg(p.frame_offset + frame) + (long long)y0 * fw + x0;
+        plane[g] = (long long)fh * fw;
+        row[g] = fw;
+        continue;
+      }
       const int x0 = min(max(__ldg(tl), 0), p.W - PSZ), y0 = min(max(__ldg(tl + 1), 0), p.H - PSZ);
       base[g] = p.src + frame * 3 * p.sc + (long long)y0 * p.sy + (long long)x0 * p.sx;
     } else {
@@ -340,7 +356,13 @@ __device__ __forceinline__ void prefetch_pixels(const Params& p, long long pair,
     if (cell < G * PSZ * PSZ) {
       const int g = cell >= PSZ * PSZ ? 1 : 0, r = cell - g * (PSZ * PSZ), y = r / PSZ, x = r - y * PSZ;
       const float* b = g == 0 ? base[0] : base[1];
-      if (b) {
+      if (PACKED && b) {
+        const long long pl = g == 0 ? plane[0] : plane[1];
+        b += y * (g == 0 ? row[0] : row[1]) + x;
+        pre[3 * k] = __ldg(b);
+        pre[3 * k + 1] = __ldg(b + pl);
+        pre[3 * k + 2] = __ldg(b + 2 * pl);
+      } else if (b) {
         b += y * p.sy + x * p.sx;
         pre[3 * k] = __ldg(b);
         pre[3 * k + 1] = __ldg(b + p.sc);
@@ -365,6 +387,9 @@ __device__ __forceinline__ void store_pixels(float* smem, int tid, const float (
 
 // Persistent: CTA b encodes patch pairs b, b + gridDim.x, ...  The pixels of the next pair are loaded into registers
 // while the current pair is in its convolutions and stored once the region they share with the 8x8 / 4x4 maps is free.
+// PACKED: patches are read from a packed frame buffer (frames of different sizes); a separate instantiation, so that
+// the image and patch-tensor forms keep their code and register allocation.
+template <bool PACKED>
 __global__ void __launch_bounds__(THREADS, 1) shallow_encoder_kernel(const Params p) {
   extern __shared__ __align__(16) float smem[];
   float* red = smem + OFF_RED;
@@ -392,7 +417,7 @@ __global__ void __launch_bounds__(THREADS, 1) shallow_encoder_kernel(const Param
   stage(wb, pk + W_L1C1, 9216, tid);
   cp_async_commit();
   float pre[24];
-  prefetch_pixels(p, pair, tid, pre);
+  prefetch_pixels<PACKED>(p, pair, tid, pre);
   zero_border<XP_W, CS, false>(smem + OFF_XP, tid);
   zero_border<T1P_W, CS, false>(smem + OFF_T1P, tid);
   zero_border<IN_W, 4, true>(smem + OFF_IN, tid);
@@ -415,7 +440,7 @@ __global__ void __launch_bounds__(THREADS, 1) shallow_encoder_kernel(const Param
       store32<16, XP_W, false>(smem + g * PATCH_FLOATS + OFF_XP + ((oy + 1) * XP_W + 1 + pw) * CS + 4 * cw, acw);
     }
     __syncthreads();
-    if (has_next) prefetch_pixels(p, next, tid, pre);   // in flight until this pair's convolutions are done
+    if (has_next) prefetch_pixels<PACKED>(p, next, tid, pre);   // in flight until this pair's convolutions are done
     // the input is dead: its space now holds the padded 8x8 / 4x4 maps, whose borders must read as zero
     zero_border<10, CS, true>(smem + OFF_A8P, tid);
     zero_border<6, CS, true>(smem + OFF_A4P, tid);
@@ -592,20 +617,22 @@ extern "C" int comet_shallow_encoder_pack_f32(const float* const* params_host, f
   return launch_status("shallow_encoder_pack_kernel");
 }
 
+template <bool PACKED>
 static int launch_shallow_encoder(const senc::Params& p, comet_stream_t stream) {
   static bool configured[64] = {false};
   int dev = 0;
   COMET_CUDA(cudaGetDevice(&dev));
   COMET_REQUIRE(device_sm_count_if_sm100() > 0, "the fused patch encoder needs an sm_100 device");
   if (dev < 64 && !configured[dev]) {
-    COMET_CUDA(cudaFuncSetAttribute(senc::shallow_encoder_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, senc::SMEM_BYTES));
+    COMET_CUDA(cudaFuncSetAttribute(senc::shallow_encoder_kernel<PACKED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    senc::SMEM_BYTES));
     configured[dev] = true;
   }
   const int sms = device_sm_count_if_sm100();
   long long ctas = (p.P + senc::G - 1) / senc::G;
   if (ctas > sms) ctas = sms;    // persistent: one CTA per SM, patch pairs strided over the grid
-  senc::shallow_encoder_kernel<<<(unsigned)ctas, senc::THREADS, senc::SMEM_BYTES, (cudaStream_t)stream>>>(p);
-  return launch_status("shallow_encoder_kernel");
+  senc::shallow_encoder_kernel<PACKED><<<(unsigned)ctas, senc::THREADS, senc::SMEM_BYTES, (cudaStream_t)stream>>>(p);
+  return launch_status(PACKED ? "shallow_encoder_kernel<packed>" : "shallow_encoder_kernel");
 }
 
 extern "C" int comet_shallow_encoder_f32(const float* patches, long long sn, long long sc, long long sy, long long sx,
@@ -618,7 +645,7 @@ extern "C" int comet_shallow_encoder_f32(const float* patches, long long sn, lon
   p.src = patches; p.topleft = nullptr; p.packed = packed; p.out = out; p.P = P;
   p.sn = sn; p.sc = sc; p.sy = sy; p.sx = sx;
   p.S = 1; p.N = 1; p.H = senc::PSZ; p.W = senc::PSZ; p.eps = eps;
-  return launch_shallow_encoder(p, stream);
+  return launch_shallow_encoder<false>(p, stream);
 }
 
 extern "C" int comet_shallow_encoder_from_images_f32(const float* images, const int* topleft, const float* packed, float* out,
@@ -632,7 +659,7 @@ extern "C" int comet_shallow_encoder_from_images_f32(const float* images, const 
   p.src = images; p.topleft = topleft; p.packed = packed; p.out = out; p.P = P;
   p.sn = 0; p.sc = (long long)H * W; p.sy = W; p.sx = 1;
   p.S = S; p.N = N; p.H = H; p.W = W; p.eps = eps;
-  return launch_shallow_encoder(p, stream);
+  return launch_shallow_encoder<false>(p, stream);
 }
 
 extern "C" int comet_shallow_encoder_from_images_indexed_f32(const float* images, const int* topleft, const int* seq_of_track,
@@ -650,7 +677,26 @@ extern "C" int comet_shallow_encoder_from_images_indexed_f32(const float* images
   p.P = (long long)P * S;
   p.sn = 0; p.sc = (long long)H * W; p.sy = W; p.sx = 1;
   p.S = S; p.N = P; p.H = H; p.W = W; p.nseq = B; p.eps = eps;
-  return launch_shallow_encoder(p, stream);
+  return launch_shallow_encoder<false>(p, stream);
+}
+
+extern "C" int comet_shallow_encoder_from_images_packed_f32(const float* frames, const long long* frame_offset,
+                                                            const int* frame_hw, long long num_packed_frames,
+                                                            const int* topleft, const int* seq_of_track, const int* num_frames,
+                                                            const int* frame_index, const float* packed, float* out, int P,
+                                                            int B, int S, float eps, comet_stream_t stream) {
+  COMET_REQUIRE(P >= 0 && B >= 1 && S >= 0 && num_packed_frames >= 1, "bad shape");
+  if ((long long)P * S == 0) return COMET_OK;
+  COMET_REQUIRE(frames && frame_offset && frame_hw && topleft && seq_of_track && packed && out, "null pointer");
+  COMET_REQUIRE(((uintptr_t)packed % 16) == 0, "packed parameters must be 16-byte aligned");
+  senc::Params p{};
+  p.src = frames; p.topleft = topleft; p.seq_of_track = seq_of_track; p.num_frames = num_frames; p.packed = packed; p.out = out;
+  p.frame_index = frame_index; p.nframes_src = num_packed_frames;
+  p.frame_offset = frame_offset; p.frame_hw = frame_hw;
+  p.P = (long long)P * S;
+  p.sn = 0; p.sc = 0; p.sy = 0; p.sx = 1;
+  p.S = S; p.N = P; p.H = senc::PSZ; p.W = senc::PSZ; p.nseq = B; p.eps = eps;
+  return launch_shallow_encoder<true>(p, stream);
 }
 
 extern "C" int comet_shallow_encoder_from_images_varlen_f32(const float* images, const int* topleft, const int* seq_of_track,

@@ -210,6 +210,32 @@ class ShallowEncoder(nn.Module):
                     out.data_ptr(), P, B, S, H, W, float(self.norm1.eps), stream_ptr(images.device)))
         return self._fused_result(out, (31 // self.stride, 31 // self.stride), defer_upsample)
 
+    def encode_packed_frames_patches_of(self, frames, topleft: torch.Tensor, seq_of_track: torch.Tensor,
+                                        defer_upsample: bool = True, num_frames: torch.Tensor = None,
+                                        frame_index: torch.Tensor = None):
+        """``encode_packed_patches_of`` reading a :class:`PackedFrames` buffer of frames with different sizes: frame s of
+        item ``seq_of_track[p]`` is packed frame ``frame_index[item, s]`` ((B', S) integer tensor on the device; None:
+        item * S + s).  Each corner is clamped to its own frame.  Each map is bit-identical to
+        ``encode_packed_patches_of`` on an image tensor holding that frame."""
+        from . import _lib
+        from ._dev import stream_ptr
+
+        dev = frames.device
+        P, S = topleft.shape[:2]
+        tl32 = topleft.to(torch.int32).contiguous()
+        seq32 = seq_of_track.to(device=dev, dtype=torch.int32).contiguous()
+        nf32 = None if num_frames is None else num_frames.to(device=dev, dtype=torch.int32).contiguous()
+        fi32 = None if frame_index is None else frame_index.to(device=dev, dtype=torch.int32).contiguous()
+        B_items = fi32.shape[0] if fi32 is not None else (int(seq32.max()) + 1 if P else 1)
+        offsets, hw = frames.device_tables()
+        out = torch.empty((P * S, 16, 16, 32), dtype=torch.float32, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib.comet_shallow_encoder_from_images_packed_f32(
+                frames.data.data_ptr(), offsets.data_ptr(), hw.data_ptr(), frames.num_frames, tl32.data_ptr(),
+                seq32.data_ptr(), None if nf32 is None else nf32.data_ptr(), None if fi32 is None else fi32.data_ptr(),
+                self.packed_parameters().data_ptr(), out.data_ptr(), P, B_items, S, float(self.norm1.eps), stream_ptr(dev)))
+        return self._fused_result(out, (31 // self.stride, 31 // self.stride), defer_upsample)
+
     def forward(self, x, defer_upsample: bool = False):
         """``defer_upsample=True`` returns the map *before* the last resize together with the size that resize would
         produce -- ``(x_half, (Ho, Wo))`` -- for callers that consume the up-sampling lazily (:class:`Upsampled2x`)."""
@@ -282,15 +308,23 @@ def refine_track(images, fine_fnet, fine_tracker, coarse_pred, pradius=15, sradi
     ``frame_index`` ((B', S) integer tensor): ``coarse_pred`` (B', S, N, 2) is a batch of items that read the frames of
     ``images`` (B_src, S, 3, H, W) in their own order -- item i's frame s is image frame ``frame_index[i, s]`` of the
     B_src * S frames -- and ``num_tracks`` / ``num_frames`` count per item.  The result is the call on the gathered
-    images ``images.flatten(0, 1)[frame_index]``; the patch encoder reads through the table, nothing is gathered."""
-    if num_tracks is not None or num_frames is not None or frame_index is not None:
+    images ``images.flatten(0, 1)[frame_index]``; the patch encoder reads through the table, nothing is gathered.
+
+    ``images`` a :class:`PackedFrames` buffer (frames of different sizes; ``frame_index`` required): item i's frame s is
+    packed frame ``frame_index[i, s]``, and every frame of an item has the item's size.  Each track's patch corners are
+    clamped to its own item's (W, H); everything after the patch encoder does not depend on the image size."""
+    from .packed_frames import PackedFrames
+
+    packed = isinstance(images, PackedFrames)
+    if num_tracks is not None or num_frames is not None or frame_index is not None or packed:
         from .utils import check_num_tracks
 
         B, S, N = coarse_pred.shape[:3]
         counts = check_num_tracks([N] * B if num_tracks is None else num_tracks, B, N)
         frames = None if num_frames is None else check_num_tracks(num_frames, B, S)
+        assert not packed or frame_index is not None, "packed frames are read through frame_index"
         if frame_index is not None:
-            assert frame_index.dim() == 2 and tuple(frame_index.shape) == (B, S) and images.shape[1] == S, \
+            assert frame_index.dim() == 2 and tuple(frame_index.shape) == (B, S) and (packed or images.shape[1] == S), \
                 f"frame_index must be (B', S) = ({B}, {S}) with images of S frames"
         return _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, sradius, compute_score, counts,
                                     frames, frame_index)
@@ -368,25 +402,31 @@ def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, 
     tracks, without per-sequence padding: the fused encoder reads each track's patches from its own sequence's frames.  Configurations
     without the fused encoder run the per-sequence definition.  ``frames``: per-sequence frame counts (None: all S); each
     packed track then runs its own sequence's frame count through the fine tracker.  ``frame_index``: the sequences are
-    items reading the frames of ``images`` through the table (see ``refine_track``)."""
+    items reading the frames of ``images`` through the table (see ``refine_track``); ``images`` may be a
+    :class:`PackedFrames` buffer."""
     from .base_track_predictor import BaseTrackerPredictor
+    from .packed_frames import PackedFrames
 
     B, S, N, _ = coarse_pred.shape
-    _, _, _, H, W = images.shape
+    packed = images if isinstance(images, PackedFrames) else None
+    pix = images if packed is None else packed.data
     psize = pradius * 2 + 1
     dev = coarse_pred.device
-    fused = (USE_LIBRARY_KERNELS and DEFER_UPSAMPLE and isinstance(fine_fnet, ShallowEncoder) and images.is_cuda
-             and isinstance(fine_tracker, BaseTrackerPredictor) and not torch.is_grad_enabled() and images.shape[2] == 3
-             and psize == 31 and fine_fnet._fused_ok(images, psize, psize))
+    fused = (USE_LIBRARY_KERNELS and DEFER_UPSAMPLE and isinstance(fine_fnet, ShallowEncoder) and pix.is_cuda
+             and isinstance(fine_tracker, BaseTrackerPredictor) and not torch.is_grad_enabled()
+             and (packed is not None or images.shape[2] == 3) and psize == 31 and fine_fnet._fused_ok(pix, psize, psize))
     if not fused:
-        if frame_index is not None:
+        if packed is not None:
+            fi_host = frame_index.tolist()
+        elif frame_index is not None:
             images = images.flatten(0, 1)[frame_index.to(images.device).long()].reshape((B,) + tuple(images.shape[1:]))
         refined = coarse_pred.new_zeros(coarse_pred.shape)
         score = coarse_pred.new_zeros((B, S, N)) if compute_score else None
         for b, n in enumerate(counts):
             sb = S if frames is None else frames[b]
-            r, sc = refine_track(images[b:b + 1, :sb], fine_fnet, fine_tracker, coarse_pred[b:b + 1, :sb, :n], pradius,
-                                 sradius, compute_score)
+            img = images[b:b + 1, :sb] if packed is None else torch.cat([packed.frames(f, 1) for f in fi_host[b][:sb]])[None]
+            r, sc = refine_track(img, fine_fnet, fine_tracker, coarse_pred[b:b + 1, :sb, :n], pradius, sradius,
+                                 compute_score)
             refined[b, :sb, :n] = r[0]
             if compute_score:
                 score[b, :sb, :n] = sc[0]
@@ -407,11 +447,19 @@ def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, 
     track_int = coarse.floor().int()
     track_frac = coarse - track_int
     topleft_raw = track_int - pradius
-    topleft = torch.stack([topleft_raw[..., 0].clamp(0, W - psize), topleft_raw[..., 1].clamp(0, H - psize)], dim=-1)
-
     dev_frames = None if frames is None else torch.tensor(frames, dtype=torch.int32, device=dev)
-    half, size = fine_fnet.encode_packed_patches_of(images, topleft, seq, defer_upsample=True, num_frames=dev_frames,
-                                                    frame_index=None if frame_index is None else frame_index.to(dev))
+    if packed is None:
+        _, _, _, H, W = images.shape
+        topleft = torch.stack([topleft_raw[..., 0].clamp(0, W - psize), topleft_raw[..., 1].clamp(0, H - psize)], dim=-1)
+        half, size = fine_fnet.encode_packed_patches_of(images, topleft, seq, defer_upsample=True, num_frames=dev_frames,
+                                                        frame_index=None if frame_index is None else frame_index.to(dev))
+    else:
+        # every frame of an item has the item's size: each track is clamped to its own item's (W, H)
+        hw = packed.frame_hw[frame_index[:, 0].cpu().long()].to(dev)[seq]                # (P_cap, 2) = (H, W)
+        topleft = torch.stack([torch.minimum(topleft_raw[..., 0].clamp(min=0), hw[:, 1:2] - psize),
+                               torch.minimum(topleft_raw[..., 1].clamp(min=0), hw[:, 0:1] - psize)], dim=-1)
+        half, size = fine_fnet.encode_packed_frames_patches_of(packed, topleft, seq, defer_upsample=True,
+                                                               num_frames=dev_frames, frame_index=frame_index.to(dev))
     Hs, Ws = half.shape[-2:]
     C_out = half.shape[1]
     half = half.contiguous(memory_format=torch.channels_last)

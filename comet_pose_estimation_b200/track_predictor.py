@@ -21,8 +21,9 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .base_track_predictor import BaseTrackerPredictor
+from .packed_frames import PackedFrames
 from .refine_track import ShallowEncoder, _inorm, _ResidualBlock, _resize, inverted_score, refine_track
-from .utils import check_num_tracks, check_query_frames, query_frame_items
+from .utils import check_image_sizes, check_num_tracks, check_query_frames, query_frame_items
 
 
 class BasicEncoder(nn.Module):
@@ -106,15 +107,29 @@ class TrackerPredictor(nn.Module):
                 out[b, :n] = fm[at:at + n]
                 at += n
             return out
-        x = images.reshape(B * S, C, H, W)
+        fmaps = self._encode_flat(images.reshape(B * S, C, H, W))
+        return fmaps.reshape(B, S, -1, fmaps.shape[-2], fmaps.shape[-1])
+
+    def _encode_flat(self, x):
+        """(F,3,H,W) frames -> (F,128,h,w) maps, one encoder call."""
+        H, W = x.shape[-2:]
         if self.coarse_down_ratio > 1:
             # F.interpolate(scale_factor=1/down_ratio, bilinear, align_corners=True): output size floor(H / down_ratio)
             x = _resize(x, (int(H * (1.0 / self.coarse_down_ratio)), int(W * (1.0 / self.coarse_down_ratio))))
         # NCHW on purpose: the channels-last instance-norm kernel of this library is built for the patch encoder's many tiny
         # planes (one thread per (sample, channel)); at 16 x 64 planes of 256 x 256 it would take 20 ms (measured), the
         # NCHW kernel (one warp per plane) 2.9 ms for the whole encoder (torch ops: 5.5 ms)
-        fmaps = self.coarse_fnet(x.contiguous())
-        return fmaps.reshape(B, S, -1, fmaps.shape[-2], fmaps.shape[-1])
+        return self.coarse_fnet(x.contiguous())
+
+    def min_image_size(self, fine_tracking: bool = True) -> int:
+        """The smallest image height or width ``track`` runs: the coarse maps (side ``int(x / coarse_down_ratio) //
+        stride``) need one cell at the deepest of the ``corr_levels`` pyramid levels, and the fine tracker cuts 31x31
+        patches.  128 for the shipped configuration (down ratio 2, stride 4, 5 levels: 16x16 maps)."""
+        p = self.coarse_predictor
+        x = 31 if fine_tracking else 1
+        while int(x * (1.0 / self.coarse_down_ratio)) // p.stride < 1 << (p.corr_levels - 1):
+            x += 1
+        return x
 
     @torch.no_grad()
     def track(self, images, query_points, coarse_iters=4, fine_tracking=True, query_frames=None):
@@ -148,8 +163,8 @@ class TrackerPredictor(nn.Module):
 
     @torch.no_grad()
     def track_batch(self, images, query_points, num_tracks=None, coarse_iters=4, fine_tracking=True, num_frames=None,
-                    query_frames=None):
-        """``track`` for B sequences in one call: images (B,S,3,H,W) (same image size for all), ``query_points``
+                    query_frames=None, image_sizes=None):
+        """``track`` for B sequences in one call: images (B,S,3,H,W), ``query_points``
         a list of B tensors (N_b, 2) or a padded (B, N_max, 2) tensor with ``num_tracks`` (B,) (None: every sequence
         has N_max tracks).  Returns ``track``'s dict with padded tensors (entries of tracks n >= N_b are 0) plus
         ``num_tracks`` (B,) int64; ``split_batch`` cuts it into per-sequence dicts.  Sequence b gets what ``track``
@@ -166,7 +181,26 @@ class TrackerPredictor(nn.Module):
         swapped, the tracks of sequence b whose query frame is q (in their order), S_b frames -- with every per-frame
         output swapped back.  Tracks of different query frames do not interact.  The frames are encoded once whatever
         the number of query frames; every item reads them through a frame table.  The dict gets ``query_frames``
-        (B, N_max) int64.  Query frames all 0 run exactly the path without them."""
+        (B, N_max) int64.  Query frames all 0 run exactly the path without them.
+
+        Sequences of different image sizes: ``images`` a list of B clips (S_b,3,H_b,W_b), or the padded
+        (B,S_max,3,H_max,W_max) with ``image_sizes`` (B, 2) integers (H_b, W_b): sequence b's pixels are
+        ``images[b, :S_b, :, :H_b, :W_b]`` and no other pixel is read.  Query points and tracks are in each sequence's
+        own pixels, sequence b gets what ``track`` returns for it alone (up to the rounding of the iterated loop), with
+        ``num_tracks``, ``num_frames`` and ``query_frames`` as above, and the dict gets ``image_sizes`` (B, 2) int64.
+        Sizes below ``min_image_size()`` are refused.  Sequences are ordered into size groups whose frames are packed
+        into one buffer (:class:`PackedFrames`); the encoder and the token kernels run once per group, the update
+        transformer once over all sequences.  When all sizes are equal the one-size path runs unchanged."""
+        if image_sizes is not None or (isinstance(images, (list, tuple)) and len({tuple(x.shape[-2:]) for x in images}) > 1):
+            clips, sizes = self._sized_clips(images, num_frames, image_sizes, fine_tracking)
+            if len(set(sizes)) > 1:
+                return self._track_batch_sizes(clips, sizes, query_points, num_tracks, coarse_iters, fine_tracking,
+                                               query_frames)
+            if not isinstance(images, (list, tuple)):
+                images = images[..., :sizes[0][0], :sizes[0][1]]
+            out = self.track_batch(images, query_points, num_tracks, coarse_iters, fine_tracking, num_frames, query_frames)
+            out["image_sizes"] = torch.tensor(sizes, dtype=torch.int64)
+            return out
         if isinstance(images, (list, tuple)):
             slens = [int(x.shape[0]) for x in images]
             assert num_frames is None or check_num_tracks(num_frames, len(images), max(slens)) == slens, \
@@ -177,19 +211,8 @@ class TrackerPredictor(nn.Module):
             images, num_frames = padded, slens
         B, S = images.shape[:2]
         frames = None if num_frames is None else check_num_tracks(num_frames, B, S)
-        if isinstance(query_points, (list, tuple)):
-            assert len(query_points) == B, f"{len(query_points)} query tensors for {B} sequences"
-            lens = [int(q.shape[0]) for q in query_points]
-            assert num_tracks is None or check_num_tracks(num_tracks, B, max(lens)) == lens, \
-                "num_tracks disagrees with the query lists"
-            padded = query_points[0].new_zeros((B, max(lens), 2))
-            for b, q in enumerate(query_points):
-                padded[b, :q.shape[0]] = q
-            query_points = padded
-            num_tracks = lens
-        assert query_points.dim() == 3 and query_points.shape[0] == B and query_points.shape[2] == 2
+        query_points, counts = _padded_queries(query_points, num_tracks, B)
         N = query_points.shape[1]
-        counts = check_num_tracks([N] * B if num_tracks is None else num_tracks, B, N)
         if query_frames is not None:
             qf = check_query_frames(query_frames, counts, [S] * B if frames is None else frames)
             if any(t for q in qf for t in q):
@@ -281,18 +304,7 @@ class TrackerPredictor(nn.Module):
             out["refine_pred_track"] = coarse
             out["pred_score"] = torch.ones_like(vis) * real
 
-        def scatter(v):
-            if v is None:
-                return None
-            if isinstance(v, list):
-                return [scatter(x) for x in v]
-            idx = pos_of_frame.reshape(pos_of_frame.shape + (1,) * (v.dim() - 2)).expand((-1, -1) + tuple(v.shape[2:]))
-            v = v.gather(1, idx)                                    # (B', S, N_cap, ...) in each sequence's frame order
-            res = v.new_zeros((B, S, N) + tuple(v.shape[3:]))
-            res[item_b, :, item_n] = v[item_i, :, item_j]
-            return res
-
-        out = {k: scatter(v) for k, v in out.items()}
+        out = {k: _scatter_items(v, pos_of_frame, (item_b, item_n, item_i, item_j), B, S, N) for k, v in out.items()}
         out["num_tracks"] = torch.tensor(counts, dtype=torch.int64)
         if frames is not None:
             out["num_frames"] = torch.tensor(frames, dtype=torch.int64)
@@ -301,6 +313,142 @@ class TrackerPredictor(nn.Module):
             qf_pad[b, :len(q)] = torch.tensor(q, dtype=torch.int64)
         out["query_frames"] = qf_pad
         return out
+
+    def _sized_clips(self, images, num_frames, image_sizes, fine_tracking):
+        """Validated inputs of a batch with image sizes -> (B clips (S_b,3,H_b,W_b) (views, nothing copied), sizes as a
+        list of (H_b, W_b))."""
+        if isinstance(images, (list, tuple)):
+            clips = list(images)
+            assert all(x.dim() == 4 and x.shape[1] == 3 for x in clips), "each clip must be (S_b, 3, H_b, W_b)"
+            sizes = [(int(x.shape[2]), int(x.shape[3])) for x in clips]
+            assert image_sizes is None or check_image_sizes(image_sizes, len(clips)) == sizes, \
+                "image_sizes disagrees with the image lists"
+            slens = [int(x.shape[0]) for x in clips]
+            assert num_frames is None or check_num_tracks(num_frames, len(clips), max(slens)) == slens, \
+                "num_frames disagrees with the image lists"
+        else:
+            assert images.dim() == 5 and images.shape[2] == 3, "images must be (B, S_max, 3, H_max, W_max)"
+            B, S, _, H, W = images.shape
+            sizes = check_image_sizes(image_sizes, B)
+            assert all(h <= H and w <= W for h, w in sizes), f"image_sizes {sizes} exceed the padded {H}x{W}"
+            frames = [S] * B if num_frames is None else check_num_tracks(num_frames, B, S)
+            clips = [images[b, :frames[b], :, :h, :w] for b, (h, w) in enumerate(sizes)]
+        floor = self.min_image_size(fine_tracking)
+        assert all(min(h, w) >= floor for h, w in sizes), f"image_sizes {sizes}: this tracker needs at least {floor}x{floor}"
+        return clips, sizes
+
+    def _track_batch_sizes(self, clips, sizes, query_points, num_tracks, coarse_iters, fine_tracking, query_frames):
+        """``track_batch`` over sequences of several image sizes: one item per sequence (per (sequence, query frame) with
+        query frames), items ordered by size group, the real frames packed into one buffer.  Each group's frames are
+        encoded by one call on their zero-copy slice; the coarse predictor gets one map tensor per group, the fine side
+        reads the packed buffer; results are scattered back to (sequence, frame, track) order."""
+        B = len(clips)
+        frames = [int(c.shape[0]) for c in clips]
+        S = max(frames)
+        query_points, counts = _padded_queries(query_points, num_tracks, B)
+        N = query_points.shape[1]
+        dev = query_points.device
+        qf = None if query_frames is None else check_query_frames(query_frames, counts, frames)
+        items, frame_index = query_frame_items([[0] * n for n in counts] if qf is None else qf, frames, S)
+        packed = PackedFrames(clips)
+        group_of = {b: g for g, (_, seqs) in enumerate(packed.groups) for b in seqs}
+        order = sorted(range(len(items)), key=lambda i: group_of[items[i][0]])        # stable: by group, then (b, q)
+        items = [items[i] for i in order]
+        src = frame_index[order] - torch.tensor([b * S for b, _, _ in items])[:, None]   # (B', S) frame of its sequence
+        item_counts = [len(ns) for _, _, ns in items]
+        item_frames = None if all(f == S for f in frames) else [frames[b] for b, _, _ in items]
+        group_items = [sum(1 for b, _, _ in items if group_of[b] == g) for g in range(len(packed.groups))]
+
+        fmaps = []
+        for g, (_, seqs) in enumerate(packed.groups):
+            fm = self._encode_flat(packed.group(g))                                       # (F_g, C, h, w)
+            if all(frames[b] == S for b in seqs):
+                fmaps.append(fm.reshape((len(seqs), S) + tuple(fm.shape[1:])))
+                continue
+            grp = fm.new_zeros((len(seqs), S) + tuple(fm.shape[1:]))
+            at = 0
+            for j, b in enumerate(seqs):
+                grp[j, :frames[b]] = fm[at:at + frames[b]]
+                at += frames[b]
+            fmaps.append(grp)
+        # coarse table (only with query frames): rows of group g index group g's (sequence, frame) maps
+        local = {b: j for _, seqs in packed.groups for j, b in enumerate(seqs)}
+        coarse_index = None
+        if any(q for _, q, _ in items):
+            coarse_index = src + torch.tensor([local[b] * S for b, _, _ in items])[:, None]
+        # fine table: packed frame of each (item, position); padded positions point at a real frame and are never read
+        fine_index = torch.stack([packed.seq_first[b] + src[i].clamp(max=frames[b] - 1) for i, (b, _, _) in enumerate(items)])
+
+        item_b = torch.tensor([b for b, _, ns in items for _ in ns], device=dev)
+        item_i = torch.tensor([i for i, (_, _, ns) in enumerate(items) for _ in ns], device=dev)
+        item_j = torch.tensor([j for _, _, ns in items for j in range(len(ns))], device=dev)
+        item_n = torch.tensor([n for _, _, ns in items for n in ns], device=dev)
+        q_items = query_points.new_zeros((len(items), max(item_counts), 2))
+        q_items[item_i, item_j] = query_points[item_b, item_n]
+
+        coarse_list, vis, track_feats, query_feat, conf = self.coarse_predictor(
+            query_points=q_items, fmaps=fmaps, iters=coarse_iters, down_ratio=self.coarse_down_ratio, is_train=False,
+            return_feat=True, TRACKorPOSE=False, num_tracks=item_counts, num_frames=item_frames, frame_index=coarse_index,
+            group_items=group_items)
+        coarse = coarse_list[-1]
+        Ni = coarse.shape[2]
+        out = {"coarse_pred_track_list": coarse_list, "coarse_pred_track": coarse, "vis": vis, "conf": conf}
+        real = padded_mask(item_counts, [S] * len(items) if item_frames is None else item_frames, S, Ni, coarse.device)
+        if fine_tracking:
+            refined, score = refine_track(packed, self.fine_fnet, self.fine_predictor, coarse, compute_score=True,
+                                          num_tracks=item_counts, num_frames=item_frames, frame_index=fine_index)
+            out["refine_pred_track"] = refined
+            out["track_score"] = score
+            out["pred_score"] = inverted_score(score) * real if item_frames is None else inverted_score_padded(score, real)
+        else:
+            out["refine_pred_track"] = coarse
+            out["pred_score"] = torch.ones_like(vis) * real
+
+        # position s of item i shows frame src[i, s] of its sequence, and the swap is its own inverse
+        out = {k: _scatter_items(v, src.to(dev), (item_b, item_n, item_i, item_j), B, S, N) for k, v in out.items()}
+        out["num_tracks"] = torch.tensor(counts, dtype=torch.int64)
+        out["num_frames"] = torch.tensor(frames, dtype=torch.int64)
+        if qf is not None:
+            qf_pad = torch.zeros((B, N), dtype=torch.int64)
+            for b, q in enumerate(qf):
+                qf_pad[b, :len(q)] = torch.tensor(q, dtype=torch.int64)
+            out["query_frames"] = qf_pad
+        out["image_sizes"] = torch.tensor(sizes, dtype=torch.int64)
+        return out
+
+
+def _padded_queries(query_points, num_tracks, B: int):
+    """``track_batch``'s query points (a list of B (N_b, 2) tensors, or a padded (B, N_max, 2) tensor with optional
+    counts) -> (padded (B, N_max, 2) tensor, validated counts)."""
+    if isinstance(query_points, (list, tuple)):
+        assert len(query_points) == B, f"{len(query_points)} query tensors for {B} sequences"
+        lens = [int(q.shape[0]) for q in query_points]
+        assert num_tracks is None or check_num_tracks(num_tracks, B, max(lens)) == lens, \
+            "num_tracks disagrees with the query lists"
+        padded = query_points[0].new_zeros((B, max(lens), 2))
+        for b, q in enumerate(query_points):
+            padded[b, :q.shape[0]] = q
+        query_points = padded
+        num_tracks = lens
+    assert query_points.dim() == 3 and query_points.shape[0] == B and query_points.shape[2] == 2
+    N = query_points.shape[1]
+    return query_points, check_num_tracks([N] * B if num_tracks is None else num_tracks, B, N)
+
+
+def _scatter_items(v, pos_of_frame, idx, B: int, S: int, N: int):
+    """An output (B', S, N_cap, ...) of a batch of items -> (B, S, N, ...) in (sequence, frame, track) order: position s
+    of item i shows frame ``pos_of_frame[i, s]`` of its sequence, and real track j of item i is track ``item_n`` of
+    sequence ``item_b`` (``idx`` = (item_b, item_n, item_i, item_j), one entry per real track).  Lists map per entry."""
+    if v is None:
+        return None
+    if isinstance(v, list):
+        return [_scatter_items(x, pos_of_frame, idx, B, S, N) for x in v]
+    item_b, item_n, item_i, item_j = idx
+    g = pos_of_frame.reshape(pos_of_frame.shape + (1,) * (v.dim() - 2)).expand((-1, -1) + tuple(v.shape[2:]))
+    v = v.gather(1, g)                                      # (B', S, N_cap, ...) in each sequence's frame order
+    res = v.new_zeros((B, S, N) + tuple(v.shape[3:]))
+    res[item_b, :, item_n] = v[item_i, :, item_j]
+    return res
 
 
 def padded_mask(counts, frames, S: int, N: int, device) -> torch.Tensor:
@@ -321,7 +469,8 @@ def inverted_score_padded(track_score: torch.Tensor, real: torch.Tensor, eps: fl
 
 def split_batch(out):
     """``track_batch``'s padded dict -> list of per-sequence dicts with exactly ``track``'s keys and shapes (cut along
-    the frame axis too when the dict has ``num_frames``; ``query_frames`` is cut to (1, N_b))."""
+    the frame axis too when the dict has ``num_frames``; ``query_frames`` is cut to (1, N_b); ``image_sizes`` is
+    dropped)."""
     counts = [int(n) for n in out["num_tracks"]]
     frames = [int(s) for s in out["num_frames"]] if "num_frames" in out else [None] * len(counts)
 
@@ -334,5 +483,5 @@ def split_batch(out):
             return v[b:b + 1, :n]
         return v[b:b + 1, :s, :n]
 
-    return [{k: cut(v, b, n, s) for k, v in out.items() if k not in ("num_tracks", "num_frames")}
+    return [{k: cut(v, b, n, s) for k, v in out.items() if k not in ("num_tracks", "num_frames", "image_sizes")}
             for b, (n, s) in enumerate(zip(counts, frames))]

@@ -32,8 +32,10 @@ def transformer_dim(corr_levels: int, corr_radius: int, latent_dim: int, fine: b
 # (D, H, W, device) -> channel-last sin/cos table (H, W, D).  The reference rebuilds and uploads the table every
 # iteration; here it is kept, LRU-bounded (a tracker uses two shapes: coarse 10.9 MB, fine 0.8 MB).  The building
 # stream is synchronised once, so later readers on any stream (or inside a CUDA-graph capture) need no event.
+# A batch of several image sizes (track_batch's size groups) uses one coarse table per map size: the bound leaves room
+# for 15 sizes besides the fine table, so such batches build no table after their first call.
 _TABLES = OrderedDict()
-_TABLES_MAX = 8
+_TABLES_MAX = 16
 
 
 def _sincos_table_cl(embed_dim: int, H: int, W: int, device) -> torch.Tensor:
@@ -81,16 +83,44 @@ class TrackTokenizer:
     """Per tracker call state of the fused token path: the feature pyramid (built once), the sampled 2-D
     position embedding (built once) and a ``tokens(coords, track_feats)`` method run every iteration."""
 
-    def __init__(self, corr: Union[CorrBlock, EfficientCorrBlock, torch.Tensor], coords0: torch.Tensor,
+    def __init__(self, corr: Union[CorrBlock, EfficientCorrBlock, torch.Tensor, list], coords0: torch.Tensor,
                  tdim: int, num_levels: Optional[int] = None, radius: Optional[int] = None,
-                 padding_mode: Optional[str] = None, num_tracks=None, num_frames=None, frame_index=None):
+                 padding_mode: Optional[str] = None, num_tracks=None, num_frames=None, frame_index=None,
+                 group_items=None):
         """``num_tracks`` (B ints or a 1-D tensor): the queries form a padded batch; queries n >= num_tracks[b] are
         padding, their token rows are zeros and cost no correlation work.  ``num_frames`` (likewise): sequence b has the
         first num_frames[b] of the S frames; the token rows of the others are zeros and read nothing.
 
         ``frame_index`` (B', S) integer tensor: the pyramid holds B_src * S source frames and the B' items of
         ``coords0`` read them in their own order -- item i sees source frame ``frame_index[i, s]`` (flat index) at
-        position s.  The pyramid is prepared once; counts, coordinates and tokens are per item."""
+        position s.  The pyramid is prepared once; counts, coordinates and tokens are per item.
+
+        Size groups: ``corr`` a list of G per-group correlation blocks or maps (B_g, S, C, H_g, W_g), maps of different
+        sizes.  The items of ``coords0`` are ordered group by group: group g has ``group_items[g]`` items (default
+        B_g; required with ``frame_index``, whose rows of group g index group g's B_g * S frames).  Each group gets its
+        own pyramid and position embedding, and ``tokens`` issues one launch per group into that group's rows of one
+        token buffer: the rows are what the call on that group alone computes."""
+        self._groups = None
+        if isinstance(corr, (list, tuple)):
+            from .utils import check_num_tracks
+
+            sizes = [c.shape[0] if isinstance(c, torch.Tensor) else c._pyr.B for c in corr] if group_items is None \
+                else list(group_items)
+            assert frame_index is None or group_items is not None, "frame_index over size groups needs group_items"
+            assert len(sizes) == len(corr) and all(n >= 1 for n in sizes) and sum(sizes) == coords0.shape[0], \
+                f"group_items {sizes} do not cover the {coords0.shape[0]} items"
+            B = coords0.shape[0]
+            counts = None if num_tracks is None else check_num_tracks(num_tracks, B, coords0.shape[1])
+            frames = None if num_frames is None else check_num_tracks(num_frames, B, 1 << 30)
+            self._groups, at = [], 0
+            for c, n in zip(corr, sizes):
+                self._groups.append((at, at + n, TrackTokenizer(
+                    c, coords0[at:at + n], tdim, num_levels, radius, padding_mode,
+                    None if counts is None else counts[at:at + n], None if frames is None else frames[at:at + n],
+                    None if frame_index is None else frame_index[at:at + n])))
+                at += n
+            self.tdim, self.B = tdim, B
+            return
         if isinstance(corr, (torch.Tensor, Upsampled2x)):
             assert num_levels is not None and radius is not None
             self.radius = radius
@@ -128,6 +158,14 @@ class TrackTokenizer:
 
     def tokens(self, coords: torch.Tensor, track_feats: torch.Tensor, out: Optional[torch.Tensor] = None):
         """coords (B,S,N,2), track_feats (B,S,N,latent) (any outer strides) -> (B,N,S,D_tok) float32."""
+        if self._groups is not None:
+            B, S, N, _ = coords.shape
+            assert B == self.B
+            if out is None:
+                out = torch.empty((B, N, S, self.tdim), dtype=torch.float32, device=coords.device)
+            for r0, r1, tok in self._groups:
+                tok.tokens(coords[r0:r1], track_feats[r0:r1], out[r0:r1])
+            return out
         p = self._pyr
         B, S, N, D = coords.shape
         assert D == 2

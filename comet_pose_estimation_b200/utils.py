@@ -218,6 +218,17 @@ def check_num_tracks(num_tracks, B: int, N_max: int) -> list:
     return vals
 
 
+def check_image_sizes(image_sizes, B: int) -> list:
+    """Per-sequence image sizes (a (B, 2) integer tensor or nested sequence of (H, W)) -> list of B (H, W) tuples of
+    positive Python ints.  Anything else raises AssertionError."""
+    t = image_sizes if isinstance(image_sizes, torch.Tensor) else torch.as_tensor(image_sizes)
+    assert t.dim() == 2 and tuple(t.shape) == (B, 2), f"image_sizes must be (B, 2) = ({B}, 2), got shape {tuple(t.shape)}"
+    assert not t.is_floating_point() and not t.is_complex() and t.dtype != torch.bool, "image_sizes must be integers"
+    vals = [(int(h), int(w)) for h, w in t.tolist()]
+    assert all(h >= 1 and w >= 1 for h, w in vals), f"image_sizes {vals} must be positive"
+    return vals
+
+
 def check_query_frames(query_frames, counts, frames) -> list:
     """Per-track query frames of a padded batch -> list of B lists of Python ints (list b has counts[b] entries, each in
     [0, frames[b])).  ``query_frames``: a list of B 1-D tensors / sequences with counts[b] entries, or a padded

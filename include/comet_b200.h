@@ -267,6 +267,16 @@ int comet_shallow_encoder_from_images_indexed_f32(const float* images, const int
                                                   const int* num_frames, const int* frame_index, int BS_src,
                                                   const float* packed, float* out, int P, int B, int S, int H, int W,
                                                   float eps, comet_stream_t stream);
+/* The same reading a packed frame buffer of frames with different sizes: frame f starts at element frame_offset[f] of
+ * `frames` (int64) and is frame_hw[2f] x frame_hw[2f+1] pixels (H, W; int32), stored (3, H, W) contiguous; both tables
+ * in device memory, num_packed_frames entries.  Frame ids (b * S + s, or frame_index[b * S + s]) index the packed frames
+ * and are clamped to [0, num_packed_frames).  Each corner is clamped to its own frame, [0, W_f - 31] x [0, H_f - 31], so
+ * no read leaves the frame; a frame smaller than 31x31 is not read.  Each map is bit-identical to
+ * comet_shallow_encoder_from_images_indexed_f32 on a buffer holding that frame. */
+int comet_shallow_encoder_from_images_packed_f32(const float* frames, const long long* frame_offset, const int* frame_hw,
+                                                 long long num_packed_frames, const int* topleft, const int* seq_of_track,
+                                                 const int* num_frames, const int* frame_index, const float* packed,
+                                                 float* out, int P, int B, int S, float eps, comet_stream_t stream);
 
 /* ---- sin/cos encodings: comet/models/utils.py:37-101, :724-832 ----------- */
 /* get_2d_embedding(xy, C, cat_coords): xy (M,2) contiguous -> out (M, 2*C [+2 in front if cat_coords]). */
