@@ -55,15 +55,16 @@ class BaseTrackerPredictor(nn.Module):
         (likewise): sequence b has the first ``num_frames[b]`` of the S frames of ``fmaps``; every output entry of a padded
         frame is 0, and the tracks of padded frames start at 0 and receive zero updates.
 
-        ``frame_index`` ((B', S) integer tensor, ``TRACKorPOSE=False`` only): ``fmaps`` (B_src, S, C, H, W) holds source
-        frames and ``query_points`` (B', N_max, 2) a batch of B' items; item i sees source frame ``frame_index[i, s]``
-        (flat index into the B_src * S frames) at position s.  The result is the forward on the gathered maps
+        ``frame_index`` ((B', S) integer tensor, ``TRACKorPOSE=False`` only): ``fmaps`` (B_src, S_src, C, H, W) holds
+        source frames (any S_src) and ``query_points`` (B', N_max, 2) a batch of B' items of S positions; item i sees
+        source frame ``frame_index[i, s]`` (flat index into the B_src * S_src frames) at position s, and any source frame
+        may appear any number of times.  The result is the forward on the gathered maps
         ``fmaps.flatten(0, 1)[frame_index]``: on the GPU the pyramid is prepared once over the source frames and the token
         kernels read it through the table; elsewhere the gathered maps are built and the ordinary path runs.
 
         Size groups (``TRACKorPOSE=False`` only): ``fmaps`` a list of G per-group maps (B_g, S, C, H_g, W_g) of different
         sizes, and the items of ``query_points`` ordered group by group -- B_g items per group, or ``group_items[g]``
-        with ``frame_index``, whose rows of group g index group g's B_g * S frames.  Each item gets what the call on its
+        with ``frame_index``, whose rows of group g index group g's B_g * S_g source frames (S_g may differ per group).  Each item gets what the call on its
         group alone computes (up to the rounding of the iterated loop; tokens and the first transformer pass are the
         same bits): every group has its own pyramid, position embedding and token launch, and the update transformer
         runs once over all items.  Elsewhere than on the GPU each group runs alone and the results are concatenated."""
@@ -76,15 +77,17 @@ class BaseTrackerPredictor(nn.Module):
             assert len(sizes) == len(fmaps) and all(n >= 1 for n in sizes) and sum(sizes) == Bi, \
                 f"group_items {sizes} do not cover the {Bi} items"
             assert frame_index is not None or all(f.shape[0] == n for f, n in zip(fmaps, sizes))
-            assert all(f.dim() == 5 and f.shape[1] == fmaps[0].shape[1] for f in fmaps), "per-group fmaps (B_g, S, C, H, W)"
+            assert all(f.dim() == 5 and (frame_index is not None or f.shape[1] == fmaps[0].shape[1]) for f in fmaps), \
+                "per-group fmaps (B_g, S, C, H, W)"
             if frame_index is not None:
-                assert frame_index.dim() == 2 and tuple(frame_index.shape) == (Bi, fmaps[0].shape[1]), \
-                    f"frame_index must be (B', S) = ({Bi}, {fmaps[0].shape[1]}), got {tuple(frame_index.shape)}"
+                assert frame_index.dim() == 2 and frame_index.shape[0] == Bi, \
+                    f"frame_index must be (B', S) with B' = {Bi}, got {tuple(frame_index.shape)}"
+            S_items = fmaps[0].shape[1] if frame_index is None else frame_index.shape[1]
             if not fmaps[0].is_cuda:
                 from .utils import check_num_tracks
 
                 counts = None if num_tracks is None else check_num_tracks(num_tracks, Bi, query_points.shape[1])
-                frames = None if num_frames is None else check_num_tracks(num_frames, Bi, fmaps[0].shape[1])
+                frames = None if num_frames is None else check_num_tracks(num_frames, Bi, S_items)
                 outs, at = [], 0
                 for f, n in zip(fmaps, sizes):
                     outs.append(self.forward(query_points[at:at + n], f, iters, True, down_ratio, is_train, track_feats,
@@ -102,17 +105,20 @@ class BaseTrackerPredictor(nn.Module):
         elif frame_index is not None:
             assert not TRACKorPOSE, "frame_index is served with TRACKorPOSE=False only"
             assert isinstance(fmaps, torch.Tensor) and fmaps.dim() == 5, "frame_index needs fmaps (B_src, S, C, H, W)"
-            assert frame_index.dim() == 2 and frame_index.shape == (query_points.shape[0], fmaps.shape[1]), \
-                f"frame_index must be (B', S) = ({query_points.shape[0]}, {fmaps.shape[1]}), got {tuple(frame_index.shape)}"
+            assert frame_index.dim() == 2 and frame_index.shape[0] == query_points.shape[0], \
+                f"frame_index must be (B', S) with B' = {query_points.shape[0]}, got {tuple(frame_index.shape)}"
             if not fmaps.is_cuda:
-                gathered = fmaps.flatten(0, 1)[frame_index.long()].reshape((-1,) + tuple(fmaps.shape[1:]))
+                gathered = fmaps.flatten(0, 1)[frame_index.long()]                     # (B', S, C, H, W)
                 return self.forward(query_points, gathered, iters, return_feat, down_ratio, is_train, track_feats,
                                     TRACKorPOSE, ind, num_tracks, num_frames)
             frame_index = frame_index.to(fmaps.device)
         grouped = isinstance(fmaps, list)
         counts = frames = None
         B_items = query_points.shape[0] if frame_index is not None or grouped else fmaps.shape[0]
-        S_maps = fmaps[0].shape[1] if grouped else fmaps.shape[1]
+        if frame_index is not None:
+            S_maps = frame_index.shape[1]                     # positions of the items, not source frames of the maps
+        else:
+            S_maps = fmaps[0].shape[1] if grouped else fmaps.shape[1]
         if num_frames is not None:
             assert not TRACKorPOSE, "num_frames is served with TRACKorPOSE=False only"
             from .utils import check_num_tracks

@@ -5,9 +5,13 @@ group in batch order) and their real frames are copied, group by group, into one
 (3, H_f, W_f) contiguous at element ``frame_offset[f]``.  Nothing is padded to the largest size, so a batch that mixes
 1080p clips with 512x512 clips holds each frame at its own size.  A group's frames are contiguous, so the encoder reads
 a group as a zero-copy (F_g, 3, H, W) view; the patch encoder reads any frame through the offset and size tables
-(``comet_shallow_encoder_from_images_packed_f32``)."""
+(``comet_shallow_encoder_from_images_packed_f32``).
+
+Clips that share frames of a video (``track_batch(clip_frames=...)``) are served from one such buffer too:
+:func:`pack_referenced_frames` packs each distinct referenced frame once, and the clips read it through a frame table."""
 from __future__ import annotations
 
+import bisect
 from typing import List, Sequence, Tuple
 
 import torch
@@ -75,3 +79,24 @@ class PackedFrames:
         if self._dev is None:
             self._dev = (self.frame_offset.to(self.device), self.frame_hw.to(self.device).contiguous())
         return self._dev
+
+
+def pack_referenced_frames(videos: Sequence[torch.Tensor], clip_frames: Sequence[Sequence[int]]):
+    """The distinct frames that clips reference, packed once.  ``videos``: V tensors (T_v, 3, H_v, W_v) whose frames are
+    numbered one after another, video 0 first; ``clip_frames``: B lists of frame numbers (validated).  The referenced
+    frames are cut into runs of consecutive frames of one video; each run is a zero-copy view of its video and is copied
+    into the buffer once, so frames that no clip references are never read.  -> (``PackedFrames`` whose "sequences" are
+    the runs, ``ids``: B lists, ``ids[b][s]`` the packed frame of ``clip_frames[b][s]``)."""
+    first = [0]
+    for v in videos:
+        first.append(first[-1] + int(v.shape[0]))
+    runs = []                                          # [video, first frame in the video, count]
+    for t in sorted({t for c in clip_frames for t in c}):
+        v = bisect.bisect_right(first, t) - 1
+        if runs and runs[-1][0] == v and runs[-1][1] + runs[-1][2] == t - first[v]:
+            runs[-1][2] += 1
+        else:
+            runs.append([v, t - first[v], 1])
+    packed = PackedFrames([videos[v][t0:t0 + n] for v, t0, n in runs])
+    packed_of = {first[v] + t0 + k: packed.seq_first[r] + k for r, (v, t0, n) in enumerate(runs) for k in range(n)}
+    return packed, [[packed_of[t] for t in c] for c in clip_frames]

@@ -180,13 +180,14 @@ class ShallowEncoder(nn.Module):
         num_frames[b] real frames; the pixels of the other frames are never read and their maps are zeros.
 
         ``frame_index`` (B', S) integer tensor on the device: the tracks belong to B' items (``seq_of_track`` and
-        ``num_frames`` index items) and frame s of item i is image frame ``frame_index[i, s]`` of the B * S frames of
-        ``images``."""
+        ``num_frames`` index items) and frame s of item i is image frame ``frame_index[i, s]`` of the B * S_src frames of
+        ``images`` (B, S_src, 3, H, W), any S_src; a frame may be read by any number of (item, position) entries."""
         from . import _lib
         from ._dev import stream_ptr
 
-        B, S, _, H, W = images.shape
-        P = topleft.shape[0]
+        B, S_src, _, H, W = images.shape
+        P, S = topleft.shape[:2]
+        assert frame_index is not None or S_src == S, "images and corners disagree on the frame count"
         img = images.contiguous()
         tl32 = topleft.to(torch.int32).contiguous()
         seq32 = seq_of_track.to(device=images.device, dtype=torch.int32).contiguous()
@@ -197,7 +198,7 @@ class ShallowEncoder(nn.Module):
                 fi32 = frame_index.to(device=images.device, dtype=torch.int32).contiguous()
                 _lib.check(_lib.lib.comet_shallow_encoder_from_images_indexed_f32(
                     img.data_ptr(), tl32.data_ptr(), seq32.data_ptr(), None if nf32 is None else nf32.data_ptr(),
-                    fi32.data_ptr(), B * S, self.packed_parameters().data_ptr(), out.data_ptr(), P, fi32.shape[0], S, H, W,
+                    fi32.data_ptr(), B * S_src, self.packed_parameters().data_ptr(), out.data_ptr(), P, fi32.shape[0], S, H, W,
                     float(self.norm1.eps), stream_ptr(images.device)))
             elif num_frames is None:
                 _lib.check(_lib.lib.comet_shallow_encoder_from_images_ragged_f32(
@@ -306,8 +307,9 @@ def refine_track(images, fine_fnet, fine_tracker, coarse_pred, pradius=15, sradi
     sequence b has the first ``num_frames[b]`` frames; the images of the others are never read and their entries are 0.
 
     ``frame_index`` ((B', S) integer tensor): ``coarse_pred`` (B', S, N, 2) is a batch of items that read the frames of
-    ``images`` (B_src, S, 3, H, W) in their own order -- item i's frame s is image frame ``frame_index[i, s]`` of the
-    B_src * S frames -- and ``num_tracks`` / ``num_frames`` count per item.  The result is the call on the gathered
+    ``images`` (B_src, S_src, 3, H, W), any S_src, in their own order -- item i's frame s is image frame
+    ``frame_index[i, s]`` of the B_src * S_src frames, and a frame may be read by any number of items and positions --
+    and ``num_tracks`` / ``num_frames`` count per item.  The result is the call on the gathered
     images ``images.flatten(0, 1)[frame_index]``; the patch encoder reads through the table, nothing is gathered.
 
     ``images`` a :class:`PackedFrames` buffer (frames of different sizes; ``frame_index`` required): item i's frame s is
@@ -324,8 +326,8 @@ def refine_track(images, fine_fnet, fine_tracker, coarse_pred, pradius=15, sradi
         frames = None if num_frames is None else check_num_tracks(num_frames, B, S)
         assert not packed or frame_index is not None, "packed frames are read through frame_index"
         if frame_index is not None:
-            assert frame_index.dim() == 2 and tuple(frame_index.shape) == (B, S) and (packed or images.shape[1] == S), \
-                f"frame_index must be (B', S) = ({B}, {S}) with images of S frames"
+            assert frame_index.dim() == 2 and tuple(frame_index.shape) == (B, S), \
+                f"frame_index must be (B', S) = ({B}, {S})"
         return _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, sradius, compute_score, counts,
                                     frames, frame_index)
     B, S, N, _ = coarse_pred.shape
@@ -419,7 +421,7 @@ def _refine_track_ragged(images, fine_fnet, fine_tracker, coarse_pred, pradius, 
         if packed is not None:
             fi_host = frame_index.tolist()
         elif frame_index is not None:
-            images = images.flatten(0, 1)[frame_index.to(images.device).long()].reshape((B,) + tuple(images.shape[1:]))
+            images = images.flatten(0, 1)[frame_index.to(images.device).long()]          # (B', S, 3, H, W)
         refined = coarse_pred.new_zeros(coarse_pred.shape)
         score = coarse_pred.new_zeros((B, S, N)) if compute_score else None
         for b, n in enumerate(counts):

@@ -21,9 +21,9 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .base_track_predictor import BaseTrackerPredictor
-from .packed_frames import PackedFrames
+from .packed_frames import PackedFrames, pack_referenced_frames
 from .refine_track import ShallowEncoder, _inorm, _ResidualBlock, _resize, inverted_score, refine_track
-from .utils import check_image_sizes, check_num_tracks, check_query_frames, query_frame_items
+from .utils import check_clip_frames, check_image_sizes, check_num_tracks, check_query_frames, clip_items, query_frame_items
 
 
 class BasicEncoder(nn.Module):
@@ -163,7 +163,7 @@ class TrackerPredictor(nn.Module):
 
     @torch.no_grad()
     def track_batch(self, images, query_points, num_tracks=None, coarse_iters=4, fine_tracking=True, num_frames=None,
-                    query_frames=None, image_sizes=None):
+                    query_frames=None, image_sizes=None, clip_frames=None):
         """``track`` for B sequences in one call: images (B,S,3,H,W), ``query_points``
         a list of B tensors (N_b, 2) or a padded (B, N_max, 2) tensor with ``num_tracks`` (B,) (None: every sequence
         has N_max tracks).  Returns ``track``'s dict with padded tensors (entries of tracks n >= N_b are 0) plus
@@ -190,7 +190,20 @@ class TrackerPredictor(nn.Module):
         ``num_tracks``, ``num_frames`` and ``query_frames`` as above, and the dict gets ``image_sizes`` (B, 2) int64.
         Sizes below ``min_image_size()`` are refused.  Sequences are ordered into size groups whose frames are packed
         into one buffer (:class:`PackedFrames`); the encoder and the token kernels run once per group, the update
-        transformer once over all sequences.  When all sizes are equal the one-size path runs unchanged."""
+        transformer once over all sequences.  When all sizes are equal the one-size path runs unchanged.
+
+        Clips that share frames of a video: ``images`` the source video (T,3,H,W), or a list of videos (T_v,3,H_v,W_v)
+        whose frames are numbered one after another, video 0 first; ``clip_frames`` a list of B 1-D integer tensors or
+        sequences (S_b,): clip b is made of the frames with those numbers, in that order (repeats and frames shared
+        between clips allowed; all frames of a clip of one size).  The call returns what this call returns for the
+        gathered clips ``[flat_frames[clip_frames[b]] for b in range(B)]`` with the same ``query_points``,
+        ``num_tracks`` and ``query_frames`` (query frames are clip positions), up to the rounding of the iterated loop:
+        the same keys and padding, ``num_frames`` included, and ``image_sizes`` when the sizes differ.  ``num_frames``
+        and ``image_sizes``, if given, must agree with the clips.  Each referenced frame is copied once, encoded once and
+        prepared into the coarse pyramid once; frames no clip references are never read."""
+        if clip_frames is not None:
+            return self._track_batch_clips(images, clip_frames, query_points, num_tracks, coarse_iters, fine_tracking,
+                                           num_frames, query_frames, image_sizes)
         if image_sizes is not None or (isinstance(images, (list, tuple)) and len({tuple(x.shape[-2:]) for x in images}) > 1):
             clips, sizes = self._sized_clips(images, num_frames, image_sizes, fine_tracking)
             if len(set(sizes)) > 1:
@@ -338,46 +351,69 @@ class TrackerPredictor(nn.Module):
         return clips, sizes
 
     def _track_batch_sizes(self, clips, sizes, query_points, num_tracks, coarse_iters, fine_tracking, query_frames):
-        """``track_batch`` over sequences of several image sizes: one item per sequence (per (sequence, query frame) with
-        query frames), items ordered by size group, the real frames packed into one buffer.  Each group's frames are
-        encoded by one call on their zero-copy slice; the coarse predictor gets one map tensor per group, the fine side
-        reads the packed buffer; results are scattered back to (sequence, frame, track) order."""
+        """``track_batch`` over sequences of several image sizes: the real frames packed into one buffer, and clip b made
+        of its own consecutive packed frames (see ``_track_clips``)."""
         B = len(clips)
         frames = [int(c.shape[0]) for c in clips]
-        S = max(frames)
         query_points, counts = _padded_queries(query_points, num_tracks, B)
+        qf = None if query_frames is None else check_query_frames(query_frames, counts, frames)
+        packed = PackedFrames(clips)
+        clip_ids = [list(range(packed.seq_first[b], packed.seq_first[b] + frames[b])) for b in range(B)]
+        out = self._track_clips(packed, clip_ids, query_points, counts, qf, coarse_iters, fine_tracking)
+        out["image_sizes"] = torch.tensor(sizes, dtype=torch.int64)
+        return out
+
+    def _track_batch_clips(self, images, clip_frames, query_points, num_tracks, coarse_iters, fine_tracking, num_frames,
+                           query_frames, image_sizes):
+        """``track_batch(clip_frames=...)``: validated inputs -> the distinct referenced frames packed once, then
+        ``_track_clips``."""
+        videos = [images] if isinstance(images, torch.Tensor) else list(images)
+        assert len(videos) >= 1 and all(isinstance(v, torch.Tensor) and v.dim() == 4 and v.shape[1] == 3 for v in videos), \
+            "with clip_frames, images must be a video (T, 3, H, W) or a list of videos (T_v, 3, H_v, W_v)"
+        assert len({v.device for v in videos}) == 1, "the videos must be on one device"
+        hw_of = [tuple(int(x) for x in v.shape[-2:]) for v in videos for _ in range(v.shape[0])]   # per source frame
+        clips = check_clip_frames(clip_frames, len(hw_of))
+        B = len(clips)
+        sizes = []
+        for b, c in enumerate(clips):
+            hws = sorted({hw_of[t] for t in c})
+            assert len(hws) == 1, f"clip {b} mixes frame sizes {hws}"
+            sizes.append(hws[0])
+        frames = [len(c) for c in clips]
+        assert num_frames is None or check_num_tracks(num_frames, B, max(frames)) == frames, \
+            "num_frames disagrees with the clips"
+        assert image_sizes is None or check_image_sizes(image_sizes, B) == sizes, "image_sizes disagrees with the clips"
+        floor = self.min_image_size(fine_tracking)
+        assert all(min(h, w) >= floor for h, w in sizes), f"image_sizes {sizes}: this tracker needs at least {floor}x{floor}"
+        query_points, counts = _padded_queries(query_points, num_tracks, B)
+        qf = None if query_frames is None else check_query_frames(query_frames, counts, frames)
+        packed, clip_ids = pack_referenced_frames(videos, clips)
+        out = self._track_clips(packed, clip_ids, query_points, counts, qf, coarse_iters, fine_tracking)
+        if len(set(sizes)) > 1:
+            out["image_sizes"] = torch.tensor(sizes, dtype=torch.int64)
+        return out
+
+    def _track_clips(self, packed, clip_ids, query_points, counts, qf, coarse_iters, fine_tracking):
+        """The batch of clips over a packed source buffer: clip b is made of the packed frames ``clip_ids[b]``, all of one
+        size, in any order, with repeats and frames shared between clips.  One item per clip (per (clip, query position)
+        with query frames ``qf``, validated lists), items ordered by size group; each item reads its frames through a
+        row of the item table (``clip_items``).  Each group's packed frames are encoded by one call on their zero-copy
+        slice, and the coarse predictor gets them as one source pool per group; the fine side reads the packed buffer;
+        results are scattered back to (clip, position, track) order."""
+        B = len(clip_ids)
+        frames = [len(c) for c in clip_ids]
+        S = max(frames)
         N = query_points.shape[1]
         dev = query_points.device
-        qf = None if query_frames is None else check_query_frames(query_frames, counts, frames)
-        items, frame_index = query_frame_items([[0] * n for n in counts] if qf is None else qf, frames, S)
-        packed = PackedFrames(clips)
-        group_of = {b: g for g, (_, seqs) in enumerate(packed.groups) for b in seqs}
-        order = sorted(range(len(items)), key=lambda i: group_of[items[i][0]])        # stable: by group, then (b, q)
-        items = [items[i] for i in order]
-        src = frame_index[order] - torch.tensor([b * S for b, _, _ in items])[:, None]   # (B', S) frame of its sequence
+        group_of_hw = {hw: g for g, (hw, _) in enumerate(packed.groups)}
+        group_of = [group_of_hw[tuple(packed.frame_hw[c[0]].tolist())] for c in clip_ids]
+        items, pos, fine_index = clip_items(clip_ids, [[0] * n for n in counts] if qf is None else qf, group_of)
         item_counts = [len(ns) for _, _, ns in items]
         item_frames = None if all(f == S for f in frames) else [frames[b] for b, _, _ in items]
         group_items = [sum(1 for b, _, _ in items if group_of[b] == g) for g in range(len(packed.groups))]
-
-        fmaps = []
-        for g, (_, seqs) in enumerate(packed.groups):
-            fm = self._encode_flat(packed.group(g))                                       # (F_g, C, h, w)
-            if all(frames[b] == S for b in seqs):
-                fmaps.append(fm.reshape((len(seqs), S) + tuple(fm.shape[1:])))
-                continue
-            grp = fm.new_zeros((len(seqs), S) + tuple(fm.shape[1:]))
-            at = 0
-            for j, b in enumerate(seqs):
-                grp[j, :frames[b]] = fm[at:at + frames[b]]
-                at += frames[b]
-            fmaps.append(grp)
-        # coarse table (only with query frames): rows of group g index group g's (sequence, frame) maps
-        local = {b: j for _, seqs in packed.groups for j, b in enumerate(seqs)}
-        coarse_index = None
-        if any(q for _, q, _ in items):
-            coarse_index = src + torch.tensor([local[b] * S for b, _, _ in items])[:, None]
-        # fine table: packed frame of each (item, position); padded positions point at a real frame and are never read
-        fine_index = torch.stack([packed.seq_first[b] + src[i].clamp(max=frames[b] - 1) for i, (b, _, _) in enumerate(items)])
+        # coarse table: rows of group g index group g's packed frames, which are its source pool (1, F_g, C, h, w)
+        coarse_index = fine_index - torch.tensor([packed.group_first[group_of[b]] for b, _, _ in items])[:, None]
+        fmaps = [self._encode_flat(packed.group(g))[None] for g in range(len(packed.groups))]
 
         item_b = torch.tensor([b for b, _, ns in items for _ in ns], device=dev)
         item_i = torch.tensor([i for i, (_, _, ns) in enumerate(items) for _ in ns], device=dev)
@@ -404,8 +440,8 @@ class TrackerPredictor(nn.Module):
             out["refine_pred_track"] = coarse
             out["pred_score"] = torch.ones_like(vis) * real
 
-        # position s of item i shows frame src[i, s] of its sequence, and the swap is its own inverse
-        out = {k: _scatter_items(v, src.to(dev), (item_b, item_n, item_i, item_j), B, S, N) for k, v in out.items()}
+        # position s of item i shows clip position pos[i, s], and the swap is its own inverse
+        out = {k: _scatter_items(v, pos.to(dev), (item_b, item_n, item_i, item_j), B, S, N) for k, v in out.items()}
         out["num_tracks"] = torch.tensor(counts, dtype=torch.int64)
         out["num_frames"] = torch.tensor(frames, dtype=torch.int64)
         if qf is not None:
@@ -413,7 +449,6 @@ class TrackerPredictor(nn.Module):
             for b, q in enumerate(qf):
                 qf_pad[b, :len(q)] = torch.tensor(q, dtype=torch.int64)
             out["query_frames"] = qf_pad
-        out["image_sizes"] = torch.tensor(sizes, dtype=torch.int64)
         return out
 
 

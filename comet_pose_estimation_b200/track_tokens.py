@@ -91,13 +91,14 @@ class TrackTokenizer:
         padding, their token rows are zeros and cost no correlation work.  ``num_frames`` (likewise): sequence b has the
         first num_frames[b] of the S frames; the token rows of the others are zeros and read nothing.
 
-        ``frame_index`` (B', S) integer tensor: the pyramid holds B_src * S source frames and the B' items of
-        ``coords0`` read them in their own order -- item i sees source frame ``frame_index[i, s]`` (flat index) at
-        position s.  The pyramid is prepared once; counts, coordinates and tokens are per item.
+        ``frame_index`` (B', S) integer tensor: the pyramid holds B_src * S_src source frames (any S_src) and the B'
+        items of ``coords0`` read them in their own order -- item i sees source frame ``frame_index[i, s]`` (flat index)
+        at position s; any source frame may appear any number of times, in one row or in several.  The items have S
+        positions.  The pyramid is prepared once; counts, coordinates and tokens are per item.
 
         Size groups: ``corr`` a list of G per-group correlation blocks or maps (B_g, S, C, H_g, W_g), maps of different
         sizes.  The items of ``coords0`` are ordered group by group: group g has ``group_items[g]`` items (default
-        B_g; required with ``frame_index``, whose rows of group g index group g's B_g * S frames).  Each group gets its
+        B_g; required with ``frame_index``, whose rows of group g index group g's source frames).  Each group gets its
         own pyramid and position embedding, and ``tokens`` issues one launch per group into that group's rows of one
         token buffer: the rows are what the call on that group alone computes."""
         self._groups = None
@@ -136,13 +137,14 @@ class TrackTokenizer:
         self.pos = sampled_pos_emb(coords0, tdim, p.H, p.W)
         self.frame_index = None
         self.B = p.B
+        self.S = p.S
         if frame_index is not None:
-            assert frame_index.shape == (coords0.shape[0], p.S), \
-                f"frame_index must be (B', S) = ({coords0.shape[0]}, {p.S}), got {tuple(frame_index.shape)}"
+            assert frame_index.dim() == 2 and frame_index.shape[0] == coords0.shape[0], \
+                f"frame_index must be (B', S) with B' = {coords0.shape[0]}, got {tuple(frame_index.shape)}"
             fi = frame_index.to(device=coords0.device, dtype=torch.int32).contiguous()
             assert bool(((fi >= 0) & (fi < p.B * p.S)).all()), f"frame_index outside [0, {p.B * p.S})"
             self.frame_index = fi
-            self.B = coords0.shape[0]
+            self.B, self.S = coords0.shape[0], int(fi.shape[1])
         self.num_tracks = None
         if num_tracks is not None:
             from .utils import check_num_tracks
@@ -153,7 +155,7 @@ class TrackTokenizer:
         if num_frames is not None:
             from .utils import check_num_tracks
 
-            frames = check_num_tracks(num_frames, self.B, p.S)
+            frames = check_num_tracks(num_frames, self.B, self.S)
             self.num_frames = torch.tensor(frames, dtype=torch.int32).to(coords0.device)
 
     def tokens(self, coords: torch.Tensor, track_feats: torch.Tensor, out: Optional[torch.Tensor] = None):
@@ -170,7 +172,7 @@ class TrackTokenizer:
         B, S, N, D = coords.shape
         assert D == 2
         assert track_feats.shape == (B, S, N, p.C), "track_feats must be (B,S,N,latent) with latent == C"
-        assert S == p.S and B == self.B
+        assert S == self.S and B == self.B
         require_cuda(coords, "coords")
         require_cuda(track_feats, "track_feats")
         require_no_grad(coords, track_feats)

@@ -271,3 +271,39 @@ def query_frame_items(query_frames, frames, S_max: int):
         order[0], order[q] = q, 0
         frame_index[i] = torch.tensor(order) + b * S_max
     return items, frame_index
+
+
+def check_clip_frames(clip_frames, num_source_frames: int) -> list:
+    """Frame numbers of B clips (a list of B 1-D integer tensors or sequences) -> list of B non-empty lists of Python
+    ints, each in [0, num_source_frames).  Anything else raises AssertionError."""
+    assert isinstance(clip_frames, (list, tuple)) and len(clip_frames) >= 1, "clip_frames must be a non-empty list of clips"
+    vals = []
+    for b, c in enumerate(clip_frames):
+        t = c if isinstance(c, torch.Tensor) else torch.as_tensor(c)
+        assert t.dim() == 1, f"clip {b}: frame numbers must be 1-D, got shape {tuple(t.shape)}"
+        assert t.numel() >= 1, f"clip {b} is empty"
+        assert not t.is_floating_point() and not t.is_complex() and t.dtype != torch.bool, \
+            f"clip {b}: frame numbers must be integers"
+        v = [int(x) for x in t.tolist()]
+        assert all(0 <= x < num_source_frames for x in v), f"clip {b}: frame numbers outside [0, {num_source_frames})"
+        vals.append(v)
+    return vals
+
+
+def clip_items(clip_frames, query_frames, group_of):
+    """Items of a batch of clips over a buffer of source frames: clip b is made of source frames ``clip_frames[b]``
+    (validated lists, any order, repeats allowed), and the tracks of clip b with query position q form item (b, q)
+    (``query_frames``: validated lists, see ``check_query_frames``).  Items are ordered by (``group_of[b]``, b, q), tracks
+    inside an item keep their order.  -> (items, pos, table), both tables (B', S_max) int64 on the CPU: ``pos[i, s]`` the
+    clip position that item i shows at position s (positions 0 and q swapped; padded positions s >= S_b keep s), and
+    ``table[i, s]`` the source frame there, ``clip_frames[b][pos[i, s]]`` (padded positions: the clip's last frame, whose
+    maps are never read)."""
+    frames = [len(c) for c in clip_frames]
+    S = max(frames)
+    items, swapped = query_frame_items(query_frames, frames, S)
+    order = sorted(range(len(items)), key=lambda i: group_of[items[i][0]])        # stable: by group, then (b, q)
+    items = [items[i] for i in order]
+    pos = swapped[order] - torch.tensor([b * S for b, _, _ in items], dtype=torch.int64)[:, None]
+    table = torch.tensor([[clip_frames[b][min(p, frames[b] - 1)] for p in row] for (b, _, _), row in zip(items, pos.tolist())],
+                         dtype=torch.int64)
+    return items, pos, table

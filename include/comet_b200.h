@@ -167,7 +167,8 @@ int comet_track_tokens_varlen_f32(const float* fmaps, const float* pyr, const fl
                                   int prec_mode, int pyr_layout, int D_tok, comet_stream_t stream);
 /* The same for B items that read the BS_src frames of fmaps / pyr (pyramid of all BS_src frames, as comet_pyramid_f32 lays it
  * out for BS = BS_src) in their own order: frame_index (B,S) int32 in device memory gives the frame that item b reads at
- * position s (entries outside [0, BS_src) are clamped).  Coordinates, track features, position embedding and tokens stay
+ * position s (entries outside [0, BS_src) are clamped).  BS_src need not be a multiple of S, and a table may reference any
+ * source frame any number of times, within a row or across rows.  Coordinates, track features, position embedding and tokens stay
  * per (item, position); num_tracks / num_frames keep their meaning.  Every row equals comet_track_tokens_varlen_f32 on
  * fmaps gathered as fmaps.reshape(BS_src, ...)[frame_index].  frame_index NULL is comet_track_tokens_varlen_f32.  The
  * C == 32 layouts serve a frame table without counts; COMET_PYR_UP2_SOURCE serves none. */
@@ -262,7 +263,8 @@ int comet_shallow_encoder_from_images_varlen_f32(const float* images, const int*
                                                  int H, int W, float eps, comet_stream_t stream);
 /* The same where frame s of sequence b reads image frame frame_index[b * S + s] of the BS_src frames of `images`
  * ((BS_src, 3, H, W) viewed flat; frame_index (B,S) int32 in device memory, entries clamped to [0, BS_src)) instead of
- * frame b * S + s.  frame_index NULL is the call above. */
+ * frame b * S + s.  BS_src need not be a multiple of S, and a table may reference any source frame any number of times.
+ * frame_index NULL is the call above. */
 int comet_shallow_encoder_from_images_indexed_f32(const float* images, const int* topleft, const int* seq_of_track,
                                                   const int* num_frames, const int* frame_index, int BS_src,
                                                   const float* packed, float* out, int P, int B, int S, int H, int W,
@@ -270,8 +272,9 @@ int comet_shallow_encoder_from_images_indexed_f32(const float* images, const int
 /* The same reading a packed frame buffer of frames with different sizes: frame f starts at element frame_offset[f] of
  * `frames` (int64) and is frame_hw[2f] x frame_hw[2f+1] pixels (H, W; int32), stored (3, H, W) contiguous; both tables
  * in device memory, num_packed_frames entries.  Frame ids (b * S + s, or frame_index[b * S + s]) index the packed frames
- * and are clamped to [0, num_packed_frames).  Each corner is clamped to its own frame, [0, W_f - 31] x [0, H_f - 31], so
- * no read leaves the frame; a frame smaller than 31x31 is not read.  Each map is bit-identical to
+ * and are clamped to [0, num_packed_frames); a table may reference any packed frame any number of times.  Each corner
+ * is clamped to its own frame, [0, W_f - 31] x [0, H_f - 31], so no read leaves the frame; a frame smaller than 31x31 is
+ * not read.  Each map is bit-identical to
  * comet_shallow_encoder_from_images_indexed_f32 on a buffer holding that frame. */
 int comet_shallow_encoder_from_images_packed_f32(const float* frames, const long long* frame_offset, const int* frame_hw,
                                                  long long num_packed_frames, const int* topleft, const int* seq_of_track,
@@ -325,7 +328,8 @@ int comet_tc_track_tokens_varlen_f32(const void* split, const float* track_feats
                                      int B, int S, int N, int C, int H, int W, int L, int r, int pad_mode, int prec_mode,
                                      int D_tok, void* workspace, comet_stream_t stream);
 /* The same for B items that read the BS_src frames of `split` (comet_tc_prepare_f32 with BS = BS_src) in their own order:
- * frame_index (B,S) int32 in device memory, entries clamped to [0, BS_src).  The plan kernel reads each frame's entry once
+ * frame_index (B,S) int32 in device memory, entries clamped to [0, BS_src); BS_src need not be a multiple of S, and a
+ * table may reference any source frame any number of times.  The plan kernel reads each frame's entry once
  * and stores it in that frame's job records, from which the operand producer addresses its tiles.  Everything else stays
  * per (item, position), including `workspace` (comet_tc_workspace_bytes(B*S, N)).  Rows are bit-identical to
  * comet_tc_track_tokens_varlen_f32 on a split prepared from the gathered frames.  frame_index NULL is that call. */
