@@ -68,8 +68,11 @@ class BaseTrackerPredictor(nn.Module):
         group alone computes (up to the rounding of the iterated loop; tokens and the first transformer pass are the
         same bits): every group has its own pyramid, position embedding and token launch, and the update transformer
         runs once over all items.  Elsewhere than on the GPU each group runs alone and the results are concatenated."""
-        if isinstance(fmaps, (list, tuple)):
-            assert not TRACKorPOSE, "size groups are served with TRACKorPOSE=False only"
+        if frame_index is not None and not isinstance(fmaps, (list, tuple)):
+            fmaps, group_items = [fmaps], [query_points.shape[0]]         # one source pool: a single size group
+        grouped = isinstance(fmaps, (list, tuple))
+        if grouped:
+            assert not TRACKorPOSE, "size groups and frame_index are served with TRACKorPOSE=False only"
             fmaps = list(fmaps)
             Bi = query_points.shape[0]
             sizes = [f.shape[0] for f in fmaps] if group_items is None else [int(n) for n in group_items]
@@ -82,18 +85,19 @@ class BaseTrackerPredictor(nn.Module):
             if frame_index is not None:
                 assert frame_index.dim() == 2 and frame_index.shape[0] == Bi, \
                     f"frame_index must be (B', S) with B' = {Bi}, got {tuple(frame_index.shape)}"
-            S_items = fmaps[0].shape[1] if frame_index is None else frame_index.shape[1]
+            B_items, S_maps = Bi, fmaps[0].shape[1] if frame_index is None else frame_index.shape[1]
             if not fmaps[0].is_cuda:
                 from .utils import check_num_tracks
 
                 counts = None if num_tracks is None else check_num_tracks(num_tracks, Bi, query_points.shape[1])
-                frames = None if num_frames is None else check_num_tracks(num_frames, Bi, S_items)
+                frames = None if num_frames is None else check_num_tracks(num_frames, Bi, S_maps)
                 outs, at = [], 0
                 for f, n in zip(fmaps, sizes):
+                    if frame_index is not None:
+                        f = f.flatten(0, 1)[frame_index[at:at + n].long()]           # the group's gathered maps
                     outs.append(self.forward(query_points[at:at + n], f, iters, True, down_ratio, is_train, track_feats,
                                              TRACKorPOSE, ind, None if counts is None else counts[at:at + n],
-                                             None if frames is None else frames[at:at + n],
-                                             None if frame_index is None else frame_index[at:at + n]))
+                                             None if frames is None else frames[at:at + n]))
                     at += n
                 cat = lambda vs: None if vs[0] is None else torch.cat(vs)  # noqa: E731
                 res = ([cat([o[0][i] for o in outs]) for i in range(len(outs[0][0]))],) + tuple(
@@ -102,23 +106,9 @@ class BaseTrackerPredictor(nn.Module):
             if frame_index is not None:
                 frame_index = frame_index.to(fmaps[0].device)
             group_items = sizes
-        elif frame_index is not None:
-            assert not TRACKorPOSE, "frame_index is served with TRACKorPOSE=False only"
-            assert isinstance(fmaps, torch.Tensor) and fmaps.dim() == 5, "frame_index needs fmaps (B_src, S, C, H, W)"
-            assert frame_index.dim() == 2 and frame_index.shape[0] == query_points.shape[0], \
-                f"frame_index must be (B', S) with B' = {query_points.shape[0]}, got {tuple(frame_index.shape)}"
-            if not fmaps.is_cuda:
-                gathered = fmaps.flatten(0, 1)[frame_index.long()]                     # (B', S, C, H, W)
-                return self.forward(query_points, gathered, iters, return_feat, down_ratio, is_train, track_feats,
-                                    TRACKorPOSE, ind, num_tracks, num_frames)
-            frame_index = frame_index.to(fmaps.device)
-        grouped = isinstance(fmaps, list)
-        counts = frames = None
-        B_items = query_points.shape[0] if frame_index is not None or grouped else fmaps.shape[0]
-        if frame_index is not None:
-            S_maps = frame_index.shape[1]                     # positions of the items, not source frames of the maps
         else:
-            S_maps = fmaps[0].shape[1] if grouped else fmaps.shape[1]
+            B_items, S_maps = fmaps.shape[:2]
+        counts = frames = None
         if num_frames is not None:
             assert not TRACKorPOSE, "num_frames is served with TRACKorPOSE=False only"
             from .utils import check_num_tracks
@@ -139,7 +129,7 @@ class BaseTrackerPredictor(nn.Module):
         else:
             B, N, D = query_points.shape
         S = S_maps
-        if frame_index is None and not grouped:
+        if not grouped:
             B = fmaps.shape[0]
         assert D == 2
         if down_ratio > 1:  # guards BOTH divisions (SURVEY A.6 i)
@@ -157,9 +147,6 @@ class BaseTrackerPredictor(nn.Module):
             query_track_feat = torch.cat([sample_features4d(
                 f[:, 0] if frame_index is None else f.flatten(0, 1)[frame_index[r0:r1, 0].long()], coords[r0:r1, 0])
                 for f, r0, r1 in zip(fmaps, bounds[:-1], bounds[1:])])
-        elif frame_index is not None:
-            # each item's position-0 map: a gather of B' maps (the same values the gathered copy would hold)
-            query_track_feat = sample_features4d(fmaps.flatten(0, 1)[frame_index[:, 0].long()], coords[:, 0])
         elif isinstance(fmaps, Upsampled2x):
             # bilinear sample (border) of the 2x-1 up-sampling at p == bilinear sample of its source at p / 2
             query_track_feat = sample_features4d(fmaps.src[:, 0], coords[:, 0] * 0.5)

@@ -21,9 +21,9 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .base_track_predictor import BaseTrackerPredictor
-from .packed_frames import PackedFrames, pack_referenced_frames
+from .packed_frames import pack_referenced_frames
 from .refine_track import ShallowEncoder, _inorm, _ResidualBlock, _resize, inverted_score, refine_track
-from .utils import check_clip_frames, check_image_sizes, check_num_tracks, check_query_frames, clip_items, query_frame_items
+from .utils import check_clip_frames, check_image_sizes, check_num_tracks, check_query_frames, clip_items
 
 
 class BasicEncoder(nn.Module):
@@ -94,19 +94,9 @@ class TrackerPredictor(nn.Module):
             assert B == 1, "now we only support processing one scene during inference"
         return self._encode_frames(images)
 
-    def _encode_frames(self, images, frames=None):
-        """(B,S,3,H,W) -> (B,S,128,h,w): one encoder call over all B*S frames.  ``frames`` (B ints): only the first
-        frames[b] frames of sequence b are read and encoded (in one call: the instance norms are per frame); the maps of
-        the others are zeros."""
+    def _encode_frames(self, images):
+        """(B,S,3,H,W) -> (B,S,128,h,w): one encoder call over all B*S frames."""
         B, S, C, H, W = images.shape
-        if frames is not None:
-            fm = self._encode_frames(torch.cat([images[b, :n] for b, n in enumerate(frames)])[None])[0]
-            out = fm.new_zeros((B, S) + tuple(fm.shape[1:]))
-            at = 0
-            for b, n in enumerate(frames):
-                out[b, :n] = fm[at:at + n]
-                at += n
-            return out
         fmaps = self._encode_flat(images.reshape(B * S, C, H, W))
         return fmaps.reshape(B, S, -1, fmaps.shape[-2], fmaps.shape[-1])
 
@@ -201,213 +191,107 @@ class TrackerPredictor(nn.Module):
         the same keys and padding, ``num_frames`` included, and ``image_sizes`` when the sizes differ.  ``num_frames``
         and ``image_sizes``, if given, must agree with the clips.  Each referenced frame is copied once, encoded once and
         prepared into the coarse pyramid once; frames no clip references are never read."""
-        if clip_frames is not None:
-            return self._track_batch_clips(images, clip_frames, query_points, num_tracks, coarse_iters, fine_tracking,
-                                           num_frames, query_frames, image_sizes)
-        if image_sizes is not None or (isinstance(images, (list, tuple)) and len({tuple(x.shape[-2:]) for x in images}) > 1):
-            clips, sizes = self._sized_clips(images, num_frames, image_sizes, fine_tracking)
-            if len(set(sizes)) > 1:
-                return self._track_batch_sizes(clips, sizes, query_points, num_tracks, coarse_iters, fine_tracking,
-                                               query_frames)
-            if not isinstance(images, (list, tuple)):
-                images = images[..., :sizes[0][0], :sizes[0][1]]
-            out = self.track_batch(images, query_points, num_tracks, coarse_iters, fine_tracking, num_frames, query_frames)
-            out["image_sizes"] = torch.tensor(sizes, dtype=torch.int64)
-            return out
-        if isinstance(images, (list, tuple)):
-            slens = [int(x.shape[0]) for x in images]
-            assert num_frames is None or check_num_tracks(num_frames, len(images), max(slens)) == slens, \
-                "num_frames disagrees with the image lists"
-            padded = images[0].new_zeros((len(images), max(slens)) + tuple(images[0].shape[1:]))
-            for b, x in enumerate(images):
-                padded[b, :x.shape[0]] = x
-            images, num_frames = padded, slens
-        B, S = images.shape[:2]
-        frames = None if num_frames is None else check_num_tracks(num_frames, B, S)
+        videos, clips, sizes, S = self._batch_clips(images, num_frames, image_sizes, clip_frames, fine_tracking)
+        B = len(clips)
+        frames = [len(c) for c in clips]
+        mixed = len(set(sizes)) > 1
+        listed = not isinstance(images, torch.Tensor)
         query_points, counts = _padded_queries(query_points, num_tracks, B)
         N = query_points.shape[1]
-        if query_frames is not None:
-            qf = check_query_frames(query_frames, counts, [S] * B if frames is None else frames)
-            if any(t for q in qf for t in q):
-                return self._track_batch_query_frames(images, query_points, counts, frames, qf, coarse_iters, fine_tracking)
-            out = self.track_batch(images, query_points, counts, coarse_iters, fine_tracking, frames)
-            out["query_frames"] = torch.zeros((B, N), dtype=torch.int64)
-            return out
-        if frames is not None:
-            return self._track_batch_frames(images, query_points, counts, frames, coarse_iters, fine_tracking)
-        fmaps = self._encode_frames(images)
-        coarse_list, vis, track_feats, query_feat, conf = self.coarse_predictor(
-            query_points=query_points, fmaps=fmaps, iters=coarse_iters, down_ratio=self.coarse_down_ratio, is_train=False,
-            return_feat=True, TRACKorPOSE=False, num_tracks=counts)
-        coarse = coarse_list[-1]
-        out = {"coarse_pred_track_list": coarse_list, "coarse_pred_track": coarse, "vis": vis, "conf": conf}
-        if fine_tracking:
-            refined, score = refine_track(images, self.fine_fnet, self.fine_predictor, coarse, compute_score=True,
-                                          num_tracks=counts)
+        qf = [[0] * n for n in counts] if query_frames is None else check_query_frames(query_frames, counts, frames)
+        if clip_frames is not None or mixed or any(f != S for f in frames) or any(t for q in qf for t in q):
+            packed, clip_ids = pack_referenced_frames(videos, clips)
+            out = self._track_clips(packed, clip_ids, query_points, counts, qf, S, coarse_iters, fine_tracking)
+        else:
+            # a plain batch: one size, every frame real, every query on frame 0
+            images = torch.stack(videos) if listed else images[..., :sizes[0][0], :sizes[0][1]]
+            fmaps = self._encode_frames(images)
+            coarse_list, vis, track_feats, query_feat, conf = self.coarse_predictor(
+                query_points=query_points, fmaps=fmaps, iters=coarse_iters, down_ratio=self.coarse_down_ratio,
+                is_train=False, return_feat=True, TRACKorPOSE=False, num_tracks=counts)
+            coarse = coarse_list[-1]
+            out = {"coarse_pred_track_list": coarse_list, "coarse_pred_track": coarse, "vis": vis, "conf": conf}
             real = (torch.arange(N, device=coarse.device)[None, :] < torch.tensor(counts, device=coarse.device)[:, None])
-            out["refine_pred_track"] = refined
-            out["track_score"] = score
-            out["pred_score"] = inverted_score(score) * real[:, None, :]
-        else:
-            out["refine_pred_track"] = coarse
-            real = (torch.arange(N, device=coarse.device)[None, :] < torch.tensor(counts, device=coarse.device)[:, None])
-            out["pred_score"] = torch.ones_like(vis) * real[:, None, :]
+            if fine_tracking:
+                refined, score = refine_track(images, self.fine_fnet, self.fine_predictor, coarse, compute_score=True,
+                                              num_tracks=counts)
+                out["refine_pred_track"] = refined
+                out["track_score"] = score
+                out["pred_score"] = inverted_score(score) * real[:, None, :]
+            else:
+                out["refine_pred_track"] = coarse
+                out["pred_score"] = torch.ones_like(vis) * real[:, None, :]
         out["num_tracks"] = torch.tensor(counts, dtype=torch.int64)
-        return out
-
-    def _track_batch_frames(self, images, query_points, counts, frames, coarse_iters, fine_tracking):
-        """``track_batch`` with per-sequence frame counts (validated lists)."""
-        B, S = images.shape[:2]
-        N = query_points.shape[1]
-        fmaps = self._encode_frames(images, frames)
-        coarse_list, vis, track_feats, query_feat, conf = self.coarse_predictor(
-            query_points=query_points, fmaps=fmaps, iters=coarse_iters, down_ratio=self.coarse_down_ratio, is_train=False,
-            return_feat=True, TRACKorPOSE=False, num_tracks=counts, num_frames=frames)
-        coarse = coarse_list[-1]
-        out = {"coarse_pred_track_list": coarse_list, "coarse_pred_track": coarse, "vis": vis, "conf": conf}
-        real = padded_mask(counts, frames, S, N, coarse.device)
-        if fine_tracking:
-            refined, score = refine_track(images, self.fine_fnet, self.fine_predictor, coarse, compute_score=True,
-                                          num_tracks=counts, num_frames=frames)
-            out["refine_pred_track"] = refined
-            out["track_score"] = score
-            out["pred_score"] = inverted_score_padded(score, real)
-        else:
-            out["refine_pred_track"] = coarse
-            out["pred_score"] = torch.ones_like(vis) * real
-        out["num_tracks"] = torch.tensor(counts, dtype=torch.int64)
-        out["num_frames"] = torch.tensor(frames, dtype=torch.int64)
-        return out
-
-
-    def _track_batch_query_frames(self, images, query_points, counts, frames, qf, coarse_iters, fine_tracking):
-        """``track_batch`` with per-track query frames (validated lists): one item per (sequence, query frame), one
-        encoder pass over the source frames, one predictor and one ``refine_track`` call over the items, results
-        scattered back to (sequence, frame, track) order."""
-        B, S = images.shape[:2]
-        N = query_points.shape[1]
-        dev = query_points.device
-        items, frame_index = query_frame_items(qf, [S] * B if frames is None else frames, S)
-        item_counts = [len(ns) for _, _, ns in items]
-        item_frames = None if frames is None else [frames[b] for b, _, _ in items]
-        item_b = torch.tensor([b for b, _, ns in items for _ in ns], device=dev)        # (M,) per real track
-        item_i = torch.tensor([i for i, (_, _, ns) in enumerate(items) for _ in ns], device=dev)
-        item_j = torch.tensor([j for _, _, ns in items for j in range(len(ns))], device=dev)
-        item_n = torch.tensor([n for _, _, ns in items for n in ns], device=dev)
-        q_items = query_points.new_zeros((len(items), max(item_counts), 2))
-        q_items[item_i, item_j] = query_points[item_b, item_n]
-        # position s of item i shows frame swap(s) of its sequence, and the swap is its own inverse
-        pos_of_frame = (frame_index - torch.tensor([b * S for b, _, _ in items])[:, None]).to(dev)   # (B', S)
-
-        fmaps = self._encode_frames(images, frames)
-        coarse_list, vis, track_feats, query_feat, conf = self.coarse_predictor(
-            query_points=q_items, fmaps=fmaps, iters=coarse_iters, down_ratio=self.coarse_down_ratio, is_train=False,
-            return_feat=True, TRACKorPOSE=False, num_tracks=item_counts, num_frames=item_frames, frame_index=frame_index)
-        coarse = coarse_list[-1]
-        Si, Ni = coarse.shape[1], coarse.shape[2]
-        out = {"coarse_pred_track_list": coarse_list, "coarse_pred_track": coarse, "vis": vis, "conf": conf}
-        real = padded_mask(item_counts, [Si] * len(items) if item_frames is None else item_frames, Si, Ni, coarse.device)
-        if fine_tracking:
-            refined, score = refine_track(images, self.fine_fnet, self.fine_predictor, coarse, compute_score=True,
-                                          num_tracks=item_counts, num_frames=item_frames, frame_index=frame_index)
-            out["refine_pred_track"] = refined
-            out["track_score"] = score
-            out["pred_score"] = inverted_score(score) * real if item_frames is None else inverted_score_padded(score, real)
-        else:
-            out["refine_pred_track"] = coarse
-            out["pred_score"] = torch.ones_like(vis) * real
-
-        out = {k: _scatter_items(v, pos_of_frame, (item_b, item_n, item_i, item_j), B, S, N) for k, v in out.items()}
-        out["num_tracks"] = torch.tensor(counts, dtype=torch.int64)
-        if frames is not None:
+        if num_frames is not None or listed or clip_frames is not None or mixed:
             out["num_frames"] = torch.tensor(frames, dtype=torch.int64)
-        qf_pad = torch.zeros((B, N), dtype=torch.int64)
-        for b, q in enumerate(qf):
-            qf_pad[b, :len(q)] = torch.tensor(q, dtype=torch.int64)
-        out["query_frames"] = qf_pad
+        if query_frames is not None:
+            out["query_frames"] = torch.zeros((B, N), dtype=torch.int64)
+            for b, q in enumerate(qf):
+                out["query_frames"][b, :len(q)] = torch.tensor(q, dtype=torch.int64)
+        if mixed or (image_sizes is not None and clip_frames is None):
+            out["image_sizes"] = torch.tensor(sizes, dtype=torch.int64)
         return out
 
-    def _sized_clips(self, images, num_frames, image_sizes, fine_tracking):
-        """Validated inputs of a batch with image sizes -> (B clips (S_b,3,H_b,W_b) (views, nothing copied), sizes as a
-        list of (H_b, W_b))."""
-        if isinstance(images, (list, tuple)):
-            clips = list(images)
-            assert all(x.dim() == 4 and x.shape[1] == 3 for x in clips), "each clip must be (S_b, 3, H_b, W_b)"
-            sizes = [(int(x.shape[2]), int(x.shape[3])) for x in clips]
-            assert image_sizes is None or check_image_sizes(image_sizes, len(clips)) == sizes, \
-                "image_sizes disagrees with the image lists"
-            slens = [int(x.shape[0]) for x in clips]
-            assert num_frames is None or check_num_tracks(num_frames, len(clips), max(slens)) == slens, \
-                "num_frames disagrees with the image lists"
+    def _batch_clips(self, images, num_frames, image_sizes, clip_frames, fine_tracking):
+        """``track_batch``'s images, validated -> (videos, clips, sizes, S): V source videos (T_v,3,H_v,W_v) whose frames
+        are numbered one after another (views, nothing copied), clip b's frame numbers, clip b's (H_b, W_b), and the
+        length of the output frame axis: a padded tensor of one size keeps its S_max, every other form gets max(S_b).
+        A list of clips is one video per clip; a padded tensor is the videos ``images[b, :S_b, :, :H_b, :W_b]``."""
+        if clip_frames is not None:
+            videos = [images] if isinstance(images, torch.Tensor) else list(images)
+            assert len(videos) >= 1 and all(isinstance(v, torch.Tensor) and v.dim() == 4 and v.shape[1] == 3 for v in videos), \
+                "with clip_frames, images must be a video (T, 3, H, W) or a list of videos (T_v, 3, H_v, W_v)"
+            assert len({v.device for v in videos}) == 1, "the videos must be on one device"
+            hw_of = [tuple(int(x) for x in v.shape[-2:]) for v in videos for _ in range(v.shape[0])]   # per source frame
+            clips = check_clip_frames(clip_frames, len(hw_of))
+            sizes = []
+            for b, c in enumerate(clips):
+                hws = sorted({hw_of[t] for t in c})
+                assert len(hws) == 1, f"clip {b} mixes frame sizes {hws}"
+                sizes.append(hws[0])
+        elif isinstance(images, (list, tuple)):
+            videos = list(images)
+            sizes = [(int(x.shape[-2]), int(x.shape[-1])) for x in videos]
         else:
-            assert images.dim() == 5 and images.shape[2] == 3, "images must be (B, S_max, 3, H_max, W_max)"
+            assert images.dim() == 5, "images must be (B, S_max, 3, H_max, W_max)"
             B, S, _, H, W = images.shape
-            sizes = check_image_sizes(image_sizes, B)
+            sizes = [(H, W)] * B if image_sizes is None else check_image_sizes(image_sizes, B)
             assert all(h <= H and w <= W for h, w in sizes), f"image_sizes {sizes} exceed the padded {H}x{W}"
             frames = [S] * B if num_frames is None else check_num_tracks(num_frames, B, S)
-            clips = [images[b, :frames[b], :, :h, :w] for b, (h, w) in enumerate(sizes)]
-        floor = self.min_image_size(fine_tracking)
-        assert all(min(h, w) >= floor for h, w in sizes), f"image_sizes {sizes}: this tracker needs at least {floor}x{floor}"
-        return clips, sizes
-
-    def _track_batch_sizes(self, clips, sizes, query_points, num_tracks, coarse_iters, fine_tracking, query_frames):
-        """``track_batch`` over sequences of several image sizes: the real frames packed into one buffer, and clip b made
-        of its own consecutive packed frames (see ``_track_clips``)."""
-        B = len(clips)
-        frames = [int(c.shape[0]) for c in clips]
-        query_points, counts = _padded_queries(query_points, num_tracks, B)
-        qf = None if query_frames is None else check_query_frames(query_frames, counts, frames)
-        packed = PackedFrames(clips)
-        clip_ids = [list(range(packed.seq_first[b], packed.seq_first[b] + frames[b])) for b in range(B)]
-        out = self._track_clips(packed, clip_ids, query_points, counts, qf, coarse_iters, fine_tracking)
-        out["image_sizes"] = torch.tensor(sizes, dtype=torch.int64)
-        return out
-
-    def _track_batch_clips(self, images, clip_frames, query_points, num_tracks, coarse_iters, fine_tracking, num_frames,
-                           query_frames, image_sizes):
-        """``track_batch(clip_frames=...)``: validated inputs -> the distinct referenced frames packed once, then
-        ``_track_clips``."""
-        videos = [images] if isinstance(images, torch.Tensor) else list(images)
-        assert len(videos) >= 1 and all(isinstance(v, torch.Tensor) and v.dim() == 4 and v.shape[1] == 3 for v in videos), \
-            "with clip_frames, images must be a video (T, 3, H, W) or a list of videos (T_v, 3, H_v, W_v)"
-        assert len({v.device for v in videos}) == 1, "the videos must be on one device"
-        hw_of = [tuple(int(x) for x in v.shape[-2:]) for v in videos for _ in range(v.shape[0])]   # per source frame
-        clips = check_clip_frames(clip_frames, len(hw_of))
-        B = len(clips)
-        sizes = []
-        for b, c in enumerate(clips):
-            hws = sorted({hw_of[t] for t in c})
-            assert len(hws) == 1, f"clip {b} mixes frame sizes {hws}"
-            sizes.append(hws[0])
+            videos = [images[b, :n, :, :h, :w] for b, (n, (h, w)) in enumerate(zip(frames, sizes))]
+        if clip_frames is None:
+            first = [sum(int(v.shape[0]) for v in videos[:b]) for b in range(len(videos))]
+            clips = [list(range(f, f + int(v.shape[0]))) for f, v in zip(first, videos)]
         frames = [len(c) for c in clips]
-        assert num_frames is None or check_num_tracks(num_frames, B, max(frames)) == frames, \
-            "num_frames disagrees with the clips"
-        assert image_sizes is None or check_image_sizes(image_sizes, B) == sizes, "image_sizes disagrees with the clips"
-        floor = self.min_image_size(fine_tracking)
-        assert all(min(h, w) >= floor for h, w in sizes), f"image_sizes {sizes}: this tracker needs at least {floor}x{floor}"
-        query_points, counts = _padded_queries(query_points, num_tracks, B)
-        qf = None if query_frames is None else check_query_frames(query_frames, counts, frames)
-        packed, clip_ids = pack_referenced_frames(videos, clips)
-        out = self._track_clips(packed, clip_ids, query_points, counts, qf, coarse_iters, fine_tracking)
-        if len(set(sizes)) > 1:
-            out["image_sizes"] = torch.tensor(sizes, dtype=torch.int64)
-        return out
+        sized = clip_frames is not None or image_sizes is not None or len(set(sizes)) > 1
+        if not isinstance(images, torch.Tensor) or clip_frames is not None:         # the sizes and lengths are the clips'
+            what = "the image lists" if clip_frames is None else "the clips"
+            assert num_frames is None or check_num_tracks(num_frames, len(clips), max(frames)) == frames, \
+                f"num_frames disagrees with {what}"
+            assert image_sizes is None or check_image_sizes(image_sizes, len(clips)) == sizes, \
+                f"image_sizes disagrees with {what}"
+        if sized:
+            assert all(v.dim() == 4 and v.shape[1] == 3 for v in videos), "each clip must be (S_b, 3, H_b, W_b)"
+            floor = self.min_image_size(fine_tracking)
+            assert all(min(h, w) >= floor for h, w in sizes), \
+                f"image_sizes {sizes}: this tracker needs at least {floor}x{floor}"
+        one_size = isinstance(images, torch.Tensor) and clip_frames is None and len(set(sizes)) == 1
+        return videos, clips, sizes, images.shape[1] if one_size else max(frames)
 
-    def _track_clips(self, packed, clip_ids, query_points, counts, qf, coarse_iters, fine_tracking):
+    def _track_clips(self, packed, clip_ids, query_points, counts, qf, S, coarse_iters, fine_tracking):
         """The batch of clips over a packed source buffer: clip b is made of the packed frames ``clip_ids[b]``, all of one
-        size, in any order, with repeats and frames shared between clips.  One item per clip (per (clip, query position)
-        with query frames ``qf``, validated lists), items ordered by size group; each item reads its frames through a
-        row of the item table (``clip_items``).  Each group's packed frames are encoded by one call on their zero-copy
-        slice, and the coarse predictor gets them as one source pool per group; the fine side reads the packed buffer;
-        results are scattered back to (clip, position, track) order."""
+        size, in any order, with repeats and frames shared between clips.  One item per (clip, query position) of the
+        query frames ``qf`` (validated lists), items ordered by size group; each item reads its frames through a row of
+        the item table (``clip_items``).  Each group's packed frames are encoded by one call on their zero-copy slice,
+        and the coarse predictor gets them as one source pool per group; the fine side reads the packed buffer; results
+        are scattered back to (clip, position, track) order, S positions (S >= every clip's length)."""
         B = len(clip_ids)
         frames = [len(c) for c in clip_ids]
-        S = max(frames)
         N = query_points.shape[1]
         dev = query_points.device
         group_of_hw = {hw: g for g, (hw, _) in enumerate(packed.groups)}
         group_of = [group_of_hw[tuple(packed.frame_hw[c[0]].tolist())] for c in clip_ids]
-        items, pos, fine_index = clip_items(clip_ids, [[0] * n for n in counts] if qf is None else qf, group_of)
+        items, pos, fine_index = clip_items(clip_ids, qf, group_of, S)
         item_counts = [len(ns) for _, _, ns in items]
         item_frames = None if all(f == S for f in frames) else [frames[b] for b, _, _ in items]
         group_items = [sum(1 for b, _, _ in items if group_of[b] == g) for g in range(len(packed.groups))]
@@ -422,10 +306,11 @@ class TrackerPredictor(nn.Module):
         q_items = query_points.new_zeros((len(items), max(item_counts), 2))
         q_items[item_i, item_j] = query_points[item_b, item_n]
 
+        # one size: a single source pool with its table, the call a coarse predictor without size groups also serves
+        pools = dict(fmaps=fmaps[0]) if len(fmaps) == 1 else dict(fmaps=fmaps, group_items=group_items)
         coarse_list, vis, track_feats, query_feat, conf = self.coarse_predictor(
-            query_points=q_items, fmaps=fmaps, iters=coarse_iters, down_ratio=self.coarse_down_ratio, is_train=False,
-            return_feat=True, TRACKorPOSE=False, num_tracks=item_counts, num_frames=item_frames, frame_index=coarse_index,
-            group_items=group_items)
+            query_points=q_items, iters=coarse_iters, down_ratio=self.coarse_down_ratio, is_train=False, return_feat=True,
+            TRACKorPOSE=False, num_tracks=item_counts, num_frames=item_frames, frame_index=coarse_index, **pools)
         coarse = coarse_list[-1]
         Ni = coarse.shape[2]
         out = {"coarse_pred_track_list": coarse_list, "coarse_pred_track": coarse, "vis": vis, "conf": conf}
@@ -440,16 +325,10 @@ class TrackerPredictor(nn.Module):
             out["refine_pred_track"] = coarse
             out["pred_score"] = torch.ones_like(vis) * real
 
+        if Ni == N and [(b, q) for b, q, _ in items] == [(b, 0) for b in range(B)]:
+            return out          # the items are the clips in batch order with no position swapped: nothing to scatter
         # position s of item i shows clip position pos[i, s], and the swap is its own inverse
-        out = {k: _scatter_items(v, pos.to(dev), (item_b, item_n, item_i, item_j), B, S, N) for k, v in out.items()}
-        out["num_tracks"] = torch.tensor(counts, dtype=torch.int64)
-        out["num_frames"] = torch.tensor(frames, dtype=torch.int64)
-        if qf is not None:
-            qf_pad = torch.zeros((B, N), dtype=torch.int64)
-            for b, q in enumerate(qf):
-                qf_pad[b, :len(q)] = torch.tensor(q, dtype=torch.int64)
-            out["query_frames"] = qf_pad
-        return out
+        return {k: _scatter_items(v, pos.to(dev), (item_b, item_n, item_i, item_j), B, S, N) for k, v in out.items()}
 
 
 def _padded_queries(query_points, num_tracks, B: int):

@@ -290,16 +290,16 @@ def check_clip_frames(clip_frames, num_source_frames: int) -> list:
     return vals
 
 
-def clip_items(clip_frames, query_frames, group_of):
+def clip_items(clip_frames, query_frames, group_of, S=None):
     """Items of a batch of clips over a buffer of source frames: clip b is made of source frames ``clip_frames[b]``
     (validated lists, any order, repeats allowed), and the tracks of clip b with query position q form item (b, q)
     (``query_frames``: validated lists, see ``check_query_frames``).  Items are ordered by (``group_of[b]``, b, q), tracks
-    inside an item keep their order.  -> (items, pos, table), both tables (B', S_max) int64 on the CPU: ``pos[i, s]`` the
-    clip position that item i shows at position s (positions 0 and q swapped; padded positions s >= S_b keep s), and
-    ``table[i, s]`` the source frame there, ``clip_frames[b][pos[i, s]]`` (padded positions: the clip's last frame, whose
-    maps are never read)."""
+    inside an item keep their order; items have S positions (S >= every clip's length; None: the longest clip's).
+    -> (items, pos, table), both tables (B', S) int64 on the CPU: ``pos[i, s]`` the clip position that item i shows at
+    position s (positions 0 and q swapped; padded positions s >= S_b keep s), and ``table[i, s]`` the source frame
+    there, ``clip_frames[b][pos[i, s]]`` (padded positions: the clip's last frame, whose maps are never read)."""
     frames = [len(c) for c in clip_frames]
-    S = max(frames)
+    S = max(frames) if S is None else S
     items, swapped = query_frame_items(query_frames, frames, S)
     order = sorted(range(len(items)), key=lambda i: group_of[items[i][0]])        # stable: by group, then (b, q)
     items = [items[i] for i in order]

@@ -198,6 +198,47 @@ def test_cpu_equal_sizes_run_the_one_size_path():
                 assert torch.equal(v, got[k]), k
 
 
+def _input_forms():
+    """(images, keywords, extra keys, frame axis) of every input form of ``track_batch``: a one-size tensor keeps its
+    S_max whatever ``num_frames`` says; lists, mixed sizes and ``clip_frames`` give max(S_b)."""
+    g = torch.Generator().manual_seed(5)
+    c = lambda s, h=64, w=80: torch.rand(s, 3, h, w, generator=g)  # noqa: E731
+    T = torch.rand(3, 8, 3, 64, 80, generator=g)
+    zero = [torch.zeros(n, dtype=torch.int64) for n in (5, 2, 4)]
+    qf = [torch.tensor([0, 1, 1, 0, 2]), torch.tensor([0, 0]), torch.tensor([3, 0, 0, 0])]
+    equal, cropped, mixed = [[64, 80]] * 3, [[64, 72]] * 3, [[64, 80], [64, 72], [64, 80]]
+    nt, nf, nfq, ns = {"num_tracks"}, {"num_frames", "num_tracks"}, {"num_tracks", "query_frames"}, {"image_sizes", "num_tracks"}
+    nsf = ns | {"num_frames"}
+    return {"tensor": (T, {}, nt, 8),
+            "tensor_full_frames": (T, dict(num_frames=[8, 8, 8]), nf, 8),
+            "tensor_ragged_frames": (T, dict(num_frames=[6, 3, 5]), nf, 8),
+            "tensor_zero_query_frames": (T, dict(query_frames=zero), nfq, 8),
+            "tensor_query_frames": (T, dict(query_frames=qf), nfq, 8),
+            "tensor_query_frames_ragged_frames": (T, dict(query_frames=qf, num_frames=[6, 3, 5]), nfq | nf, 8),
+            "tensor_equal_sizes": (T, dict(image_sizes=equal), ns, 8),
+            "tensor_equal_sizes_cropped": (T, dict(image_sizes=cropped), ns, 8),
+            "tensor_mixed_sizes": (T, dict(image_sizes=mixed), nsf, 8),
+            "tensor_mixed_sizes_ragged_frames": (T, dict(image_sizes=mixed, num_frames=[6, 3, 5]), nsf, 6),
+            "list_equal": ([c(4), c(4), c(4)], {}, nf, 4),
+            "list_equal_sizes": ([c(4), c(4), c(4)], dict(image_sizes=equal), nsf, 4),
+            "list_ragged_frames": ([c(6), c(3), c(5)], {}, nf, 6),
+            "list_mixed_sizes": ([c(4), c(3, 72, 64), c(4)], {}, nsf, 4),
+            "clip_frames_one_size": (c(10), dict(clip_frames=[[0, 1, 2], [2, 3], [5, 5, 1, 0]]), nf, 4),
+            "clip_frames_two_sizes": ([c(5), c(4, 72, 64)], dict(clip_frames=[[0, 1, 2], [5, 6], [8, 7, 6, 5]]), nsf, 4)}
+
+
+@pytest.mark.parametrize("form", list(_input_forms()))
+def test_cpu_keys_and_frame_axis_of_every_input_form(form):
+    tp = _stub_tracker()
+    images, kw, extra, S = _input_forms()[form]
+    qs = [torch.rand(n, 2, generator=torch.Generator().manual_seed(n)) * 60 for n in (5, 2, 4)]
+    with torch.no_grad():
+        out = tp.track_batch(images, qs, fine_tracking=False, **kw)
+    assert set(out) == {"coarse_pred_track_list", "coarse_pred_track", "vis", "conf", "refine_pred_track",
+                        "pred_score"} | extra
+    assert out["coarse_pred_track"].shape == (3, S, 5, 2)
+
+
 def test_packed_frames_builder():
     import comet_pose_estimation_b200 as cb
 
